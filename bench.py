@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the depletion hot path (BASELINE.json: reads/s & FASTQ GB/s depleted at 1/2/4/8 B200).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c4|c2] [--pairs P] [--split]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[3] (C4, the configuration the metric is quoted on; it fits one GPU):
 100 M 2x150 pairs (2 x 33.1 GB of FASTQ) against a 50 M-id depletion set delivered as a one-column id list.
@@ -38,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it
 
 METRIC = "reads_per_s_depleted"
 UNIT = "reads/s"
@@ -325,6 +327,41 @@ def gen_txt_full(pairs: int, device, chunk: int = 25_000_000):
     return torch.cat(parts) if len(parts) > 1 else parts[0]
 
 
+DUMP_WINDOWS, DUMP_WINDOW_BYTES, DUMP_BLOCK_BYTES, DUMP_SEED = 1024, 2048, 1 << 24, 0x5C2B
+
+
+def dump_outputs(out_dir: str, torch, res, d_out, d_oth):
+    """Writes what the last timed step handed its caller to `out_dir`, so that two builds can be compared output for
+    output (the inputs depend only on the arguments):
+      counts.npy                   float64 [file, (reads_in, reads_out, bytes kept, bytes removed)]
+      kept_r{1,2}.npy              float32 [DUMP_WINDOWS, DUMP_WINDOW_BYTES]: the kept FASTQ bytes of windows at fixed,
+                                   seeded offsets (the whole output is ~16.5 GB per file at the default size)
+      kept_r{1,2}_block_sums.npy   float64: the byte sum of every DUMP_BLOCK_BYTES block of the kept output, so that every
+                                   byte takes part in the comparison
+      removed_r{1,2}*.npy          the same for the removed records (--split)
+    At most four 8 MiB sample arrays plus the block sums: well below 64 MB."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+    save("counts", np.array([[r.reads_in, r.reads_out, r.n_written, r.n_other] for r in res], dtype=np.float64))
+    for i, r in enumerate(res):
+        for j, (kind, buf, n) in enumerate((("kept", d_out[i], r.n_written), ("removed", d_oth[i], r.n_other))):
+            if buf is None:
+                continue
+            x = buf[:n]
+            w = min(DUMP_WINDOW_BYTES, n)
+            g = torch.Generator().manual_seed(DUMP_SEED + 2 * i + j)
+            starts = torch.randint(0, n - w + 1, (DUMP_WINDOWS,), generator=g).sort().values
+            save(f"{kind}_r{i + 1}", x[(starts[:, None] + torch.arange(w)).to(x.device)].float().cpu().numpy())
+            # block by block: a sum with an int64 accumulator copies its input to int64 first
+            sums = [x[a: a + DUMP_BLOCK_BYTES].sum(dtype=torch.int64) for a in range(0, n, DUMP_BLOCK_BYTES)]
+            save(f"{kind}_r{i + 1}_block_sums", torch.stack(sums).double().cpu().numpy() if sums else np.zeros(0))
+
+
 class Phases:
     """CUDA events on the launching stream at the phase boundaries of every timed step"""
 
@@ -488,7 +525,7 @@ def run_ours(args):
     ph = Phases(torch, names)
 
     def step_dev(timed=False):
-        """-> (reads_in, reads_out, bytes written) of the WHOLE job"""
+        """-> ((reads_in, reads_out, bytes written) of the WHOLE job, paths, one_pass, this rank's result per file)"""
         if timed:
             ph.begin()
         if c4:
@@ -515,7 +552,7 @@ def run_ours(args):
                 one_pass = True
             else:
                 jobs = [(d_r[i], shards[i], d_out[i], d_oth[i]) for i in range(2)]
-                rs = sdist.clean_files_sharded_dev(api, ctx, ids, jobs, D)
+                r = rs = sdist.clean_files_sharded_dev(api, ctx, ids, jobs, D)
                 if timed:
                     ph.mark()
                 # report counters: NCCL all-reduce (the all-gather above already carries them; this is the
@@ -540,12 +577,12 @@ def run_ours(args):
         ids.free()
         if timed:
             ph.end()
-        return tot, paths, one_pass
+        return tot, paths, one_pass, r
 
     # ---- device-resident arm
     ctx.set_profiling(False)
     for _ in range(args.warmup):
-        tot, paths, one_pass = step_dev()
+        tot, paths, one_pass, _ = step_dev()
     assert all(p == 1 for p in paths), "the fused kernel must be the path that runs"
     assert one_pass, "the one-pass (speculated line phase) protocol must hold on canonical input"
     ctx.set_profiling(True)
@@ -560,7 +597,7 @@ def run_ours(args):
     torch.cuda.profiler.start()  # `ncu --profile-from-start off` lists exactly the timed launches
     e0.record()
     for _ in range(args.steps):
-        tot, paths, one_pass = step_dev(True)
+        tot, paths, one_pass, res = step_dev(True)
     e1.record()
     barrier()
     torch.cuda.profiler.stop()
@@ -569,6 +606,8 @@ def run_ours(args):
     launches = (ctx.launches - l0)
     f_ms, f_n, f_bytes = ctx.fused_stats()
     ctx.set_profiling(False)
+    if args.dump_outputs:  # before the end-to-end arm, which frees the output buffers
+        dump_outputs(args.dump_outputs, torch, res, d_out, d_oth)
     phases = ph.mean_ms()
     sys.stderr.write(f"[bench] rank {rank}: phases of every timed step (ms; {', '.join(names)}) {ph.each_ms()}\n")
     if c4:
@@ -822,7 +861,7 @@ def run_e2e(args, torch, dist, D, api, sdist, ctx, dev, world, rank, c4, pairs, 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c4", choices=["c4", "c2"],
@@ -842,7 +881,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--split", action="store_true", help="also write the removed records (kept + removed)")
     ap.add_argument("--no-bind", action="store_true", help="do not bind the rank to its GPU's NUMA-local CPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one process only: write the outputs of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
