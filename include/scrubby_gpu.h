@@ -51,7 +51,7 @@ typedef enum {
     SGPU_ERR_KRAKEN_REPORT_READS = 12,  /* KrakenReportReadFieldConversion (error.rs:142) */
     SGPU_ERR_KRAKEN_REPORT_DIRECT = 13, /* KrakenReportDirectReadFieldConversion (error.rs:144) */
     SGPU_ERR_KRAKEN_REPORT_PARENT = 14, /* KrakenReportTaxonParent (error.rs:140) */
-    SGPU_ERR_FASTA_UNSUPPORTED = 15,    /* a SHARD of '>' input (sgpu_*_shard_dev): FASTA is handled on whole files only (SURVEY 8f.4) */
+    SGPU_ERR_FASTA_UNSUPPORTED = 15,    /* a shard of '>' input given to sgpu_fastq_ids_shard_dev: FASTA shards go to sgpu_*fasta*_shard* */
     SGPU_ERR_CUDA = 16,                 /* CUDA runtime failure / no device; sgpu_last_cuda_error() has the text */
     SGPU_ERR_NOMEM = 17,
     SGPU_ERR_INVALID_ARG = 18,
@@ -184,9 +184,10 @@ void sgpu_free(void *);
 
 /* ---- FASTQ filter ---------------------------------------------------------------- */
 /* FASTA input.  When the first byte is '>' needletail switches to its FASTA reader (utils.rs:377-383) and the same
- * clean_reads / get_difference loops run on those records; sgpu_clean_fastq{,_dev} and sgpu_diff{,_dev} follow (whole
- * files; the shard entry points return SGPU_ERR_FASTA_UNSUPPORTED).  needletail 0.5.1 fasta::Reader restated (parity
- * unpinned): a record runs from its '>' to the newline in front of the next "\n>" or to the end of the input; its
+ * clean_reads / get_difference loops run on those records; sgpu_clean_fastq{,_dev} and sgpu_diff{,_dev} follow on whole
+ * files, and sgpu_clean_fasta_shard{,_dev} / sgpu_fasta_ids_shard_dev below on shards (the FASTQ shard entry points do
+ * not take '>' input: the caller picks the entry point from byte 0).  needletail 0.5.1 fasta::Reader restated (parity unpinned): a
+ * record runs from its '>' to the newline in front of the next "\n>" or to the end of the input; its
  * positions are its newlines, except that a newline on the input's LAST byte is only counted after another one, and
  * that without a trailing newline the end of the input closes the last line; id = trim_cr(start+1 .. first position),
  * raw_seq = trim_cr(first position + 1 .. last position) when there are >= 2 positions, else empty -- the inner line
@@ -243,6 +244,41 @@ sgpu_status sgpu_clean_fastq_shard(sgpu_ctx *, const sgpu_idset *, const uint8_t
                                    uint64_t newlines_before, int is_first, int is_last, int crlf, int reverse,
                                    uint8_t *out_written, size_t cap_written, size_t *n_written,
                                    uint8_t *out_other, size_t cap_other, size_t *n_other, sgpu_counts *counts);
+/* One shard of a FASTA file cut at arbitrary byte offsets (the rules above, restated per shard).  The buffer holds the
+ * shard's own bytes [0, own_len) followed by a halo.
+ *   Ownership (as for FASTQ shards: no look-behind byte is needed): a record starts at byte 0 of the file or at any '>'
+ *     that follows a '\n'.  The first shard owns the starts in [0, own_len], any other shard the starts p in
+ *     [1, own_len] with buf[p-1] == '\n' (a start exactly at own_len belongs to this shard: the next one cannot see
+ *     the byte in front of its byte 0).  An owned record ends at the newline in front of the next record start, which
+ *     may lie in the halo.
+ *   Halo: a shard that is not last and does not hold the start of the record after its last owned one returns
+ *     SGPU_ERR_HALO.  Only the is_last shard applies the end-of-file rules (the last-byte newline, an unterminated last
+ *     line, UnexpectedEnd); the caller must never hand a buffer that reaches EOF to another shard (see FASTQ shards).
+ *   Line ending: the deciding record is the first record whose bytes before its last position hold a newline; it fixes
+ *     E, and records before it are written with LF.  le_before = -1: nothing decided before this shard, its own first
+ *     deciding record decides (always the case for the first shard); 0 / 1: an earlier shard decided LF / CRLF, and
+ *     every record of this shard uses it.  *le_own returns what this shard's own first deciding record (before an
+ *     error) says, -1 when it has none, whatever le_before was: shard k+1's le_before is le_before(k) when that was
+ *     decided, else le_own(k).  counts->crlf is the E this shard wrote with.
+ *   Errors: class and record index (counts->error_record) are local to the shard; the records before the error are
+ *     produced.  Records are counted as in the whole-file call.
+ *   Arguments: d_in 16-byte aligned; is_first requires le_before == -1 and a first byte '>' (else SGPU_ERR_INVALID_ARG:
+ *     the caller chose the wrong entry point); the fewer-than-5-bytes empty-input rule applies only to a shard that is
+ *     both first and last.
+ * A whole file is the shard (own_len = n_in, is_first = 1, is_last = 1, le_before = -1). */
+sgpu_status sgpu_clean_fasta_shard_dev(sgpu_ctx *, const sgpu_idset *, const uint8_t *d_in, size_t n_in, size_t own_len,
+                                       int is_first, int is_last, int le_before, int reverse,
+                                       uint8_t *d_out_written, size_t cap_written, size_t *n_written,
+                                       uint8_t *d_out_other, size_t cap_other, size_t *n_other,
+                                       sgpu_counts *counts, int *le_own);
+/* The same on HOST buffers: the shard goes through the device in chunks with the three-stream overlap of
+ * sgpu_clean_fastq_shard, each chunk starting from the line-ending state of the one before (exact, nothing is
+ * speculated).  sgpu_clean_fastq on a host FASTA file takes the same path. */
+sgpu_status sgpu_clean_fasta_shard(sgpu_ctx *, const sgpu_idset *, const uint8_t *in, size_t n_in, size_t own_len,
+                                   int is_first, int is_last, int le_before, int reverse,
+                                   uint8_t *out_written, size_t cap_written, size_t *n_written,
+                                   uint8_t *out_other, size_t cap_other, size_t *n_other,
+                                   sgpu_counts *counts, int *le_own);
 /* '\n' count of a device buffer (the per-shard figure that is allgathered) */
 sgpu_status sgpu_count_newlines_dev(sgpu_ctx *, const uint8_t *d_buf, size_t n, uint64_t *count);
 
@@ -255,6 +291,11 @@ sgpu_status sgpu_count_newlines_dev(sgpu_ctx *, const uint8_t *d_buf, size_t n, 
 sgpu_status sgpu_fastq_ids_shard_dev(sgpu_ctx *, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
                                      size_t own_len, uint64_t newlines_before, int is_first, int is_last,
                                      sgpu_idset *into, sgpu_counts *counts);
+/* sgpu_fastq_ids_shard_dev for FASTA shards (the ownership and halo rules of sgpu_clean_fasta_shard_dev; the line
+ * ending plays no part): ids of the owned records absent from `probe` (NULL: all) go into `into`;
+ * counts->reads_in += records, counts->difference += picked records. */
+sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
+                                     size_t own_len, int is_first, int is_last, sgpu_idset *into, sgpu_counts *counts);
 /* ReadDifference::get_difference, utils.rs:250-285, for ONE (input, output) file pair:
  * counts->{reads_in, reads_out, difference} are incremented (+=) and the ids absent from the
  * output are inserted into *diff_ids (created when *diff_ids == NULL), so calling it once

@@ -51,6 +51,7 @@ SYMBOLS = [
     "sgpu_clean_fastq", "sgpu_clean_fastq_dev", "sgpu_clean_fastq_shard_dev", "sgpu_clean_fastq_shard", "sgpu_count_newlines_dev",
     "sgpu_diff", "sgpu_diff_dev", "sgpu_fastq_ids_shard_dev", "sgpu_idset_export", "sgpu_idset_import",
     "sgpu_idset_keys_dev", "sgpu_idset_from_bam", "sgpu_idset_partition_txt_dev", "sgpu_idset_assemble_dev",
+    "sgpu_clean_fasta_shard_dev", "sgpu_clean_fasta_shard", "sgpu_fasta_ids_shard_dev",
 ]
 
 _lib = None
@@ -113,6 +114,10 @@ def load():
     L.sgpu_clean_fastq_shard.argtypes = L.sgpu_clean_fastq_shard_dev.argtypes
     L.sgpu_count_newlines_dev.argtypes = [vp, vp, sz, P(u64)]
     L.sgpu_fastq_ids_shard_dev.argtypes = [vp, vp, vp, sz, sz, u64, i32, i32, vp, P(Counts)]
+    L.sgpu_clean_fasta_shard_dev.argtypes = [vp, vp, vp, sz, sz, i32, i32, i32, i32, vp, sz, P(sz), vp, sz, P(sz),
+                                             P(Counts), P(i32)]
+    L.sgpu_clean_fasta_shard.argtypes = L.sgpu_clean_fasta_shard_dev.argtypes
+    L.sgpu_fasta_ids_shard_dev.argtypes = [vp, vp, vp, sz, sz, i32, i32, vp, P(Counts)]
     for name in ("sgpu_diff", "sgpu_diff_dev"):
         getattr(L, name).argtypes = [vp, vp, sz, vp, sz, P(Counts), P(vp)]
     L.sgpu_idset_export.argtypes = [vp, P(IdSetImage)]

@@ -342,6 +342,63 @@ def clean_fastq_shard_host(ctx: Context, ids: IdSet, h_in, n_in: int, own_len: i
                           bool(c.speculated), c.own_newlines, c.lead_newlines)
 
 
+@dataclass
+class FastaShardResult:
+    n_written: int
+    n_other: int
+    reads_in: int
+    reads_out: int
+    crlf: bool          # the line ending this shard wrote with
+    empty_input: bool
+    le_own: int         # the decision of the shard's own first deciding record: -1 none, 0 LF, 1 CRLF
+    path: int = 3
+    error: int = 0      # a parse error (raise_on_error=False): its class; the records before it were produced
+    error_record: int = 0
+
+
+def _fasta_shard(fn, what, ctx, ids, buf, n_in, own_len, is_first, is_last, le_before, out, other, reverse,
+                 raise_on_error):
+    n1, n2, c, le = C.c_size_t(), C.c_size_t(), _lib.Counts(), C.c_int()
+    rc = fn(ctx.h, ids.h, C.c_void_p(buf.data_ptr()), n_in, own_len, int(is_first), int(is_last), int(le_before),
+            int(reverse), C.c_void_p(out.data_ptr()), out.numel(), C.byref(n1),
+            C.c_void_p(other.data_ptr()) if other is not None else None, other.numel() if other is not None else 0,
+            C.byref(n2), C.byref(c), C.byref(le))
+    if rc and (raise_on_error or rc >= 16):
+        raise ScrubbyGpuError(rc, c.error_record, what)
+    return FastaShardResult(n1.value, n2.value, c.reads_in, c.reads_out, bool(c.crlf), bool(c.empty_input), le.value,
+                            c.path, rc, c.error_record)
+
+
+def clean_fasta_shard_dev(ctx: Context, ids: IdSet, d_in, n_in: int, own_len: int, is_first: bool, is_last: bool,
+                          le_before: int, d_out, d_other=None, reverse: bool = False,
+                          raise_on_error: bool = True) -> FastaShardResult:
+    """sgpu_clean_fasta_shard_dev: the FASTA records that start in the owned range of a device buffer (uint8, 16-byte
+    aligned).  le_before: -1 undecided, 0 / 1 LF / CRLF decided by an earlier shard."""
+    return _fasta_shard(ctx.L.sgpu_clean_fasta_shard_dev, "clean_fasta_shard_dev", ctx, ids, d_in, n_in, own_len,
+                        is_first, is_last, le_before, d_out, d_other, reverse, raise_on_error)
+
+
+def clean_fasta_shard_host(ctx: Context, ids: IdSet, h_in, n_in: int, own_len: int, is_first: bool, is_last: bool,
+                           le_before: int, h_out, h_other=None, reverse: bool = False,
+                           raise_on_error: bool = True) -> FastaShardResult:
+    """sgpu_clean_fasta_shard: the same contract on caller-owned HOST tensors (pinned for full PCIe rate); the chunked
+    H2D / kernel / D2H pipeline runs inside the call"""
+    return _fasta_shard(ctx.L.sgpu_clean_fasta_shard, "clean_fasta_shard", ctx, ids, h_in, n_in, own_len, is_first,
+                        is_last, le_before, h_out, h_other, reverse, raise_on_error)
+
+
+def fasta_ids_shard_dev(ctx: Context, probe, d_buf, n_buf: int, own_len: int, is_first: bool, is_last: bool,
+                        into: IdSet):
+    """one shard of ReadDifference::get_difference's loops over a FASTA file: ids of the owned records absent from
+    `probe` (None: all) go into `into`; returns (records, picked records)"""
+    c = _lib.Counts()
+    rc = ctx.L.sgpu_fasta_ids_shard_dev(ctx.h, probe.h if probe is not None else None, C.c_void_p(d_buf.data_ptr()),
+                                        n_buf, own_len, int(is_first), int(is_last), into.h if into is not None else None,
+                                        C.byref(c))
+    _check(rc, c.error_record, "fasta_ids_shard_dev")
+    return c.reads_in, c.difference
+
+
 def idset_partition_txt_dev(ctx: Context, d_buf, n: int, own_len: int, starts_line: bool, is_last: bool, log2_vpages: int,
                             d_recs, d_vstart):
     """sgpu_idset_partition_txt_dev (sharded set build, step 1): this rank's id-list shard -> slot images grouped by

@@ -74,7 +74,7 @@ static sgpu_status fastq_ids_into(sgpu_ctx *c, const uint8_t *d_buf, size_t n, s
         bool empty;
         const sgpu_status src = sniff(c, d_buf, n, &empty);
         if (src == SGPU_ERR_FASTA_UNSUPPORTED && is_last && own_len == n)  // a whole FASTA file
-            return fasta_ids_into(c, d_buf, n, probe, want_absent, into, n_records, n_picked, err_record);
+            return fasta_ids_shard(c, d_buf, n, n, 1, 1, probe, want_absent, into, n_records, n_picked, err_record);
         if (src != SGPU_OK) return src;
         if (empty) return SGPU_OK;
     } else if (n == 0 || own_len == 0) {
@@ -153,8 +153,11 @@ static sgpu_status clean_dev_locked(sgpu_ctx *c, const sgpu_idset *set, const ui
     bool empty;
     {
         const sgpu_status src = sniff(c, d_in, n_in, &empty);
-        if (src == SGPU_ERR_FASTA_UNSUPPORTED)  // '>': needletail's FASTA reader takes over (whole files only)
-            return clean_fasta(c, set, d_in, n_in, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o, counts);
+        if (src == SGPU_ERR_FASTA_UNSUPPORTED) {  // '>': needletail's FASTA reader takes over
+            int le_own;
+            return clean_fasta_shard(c, set, d_in, n_in, n_in, 1, 1, -1, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o,
+                                     counts, &le_own);
+        }
         if (src != SGPU_OK) return src;
     }
     if (empty) {
@@ -215,7 +218,7 @@ const char *sgpu_strerror(int s) {
     case SGPU_ERR_KRAKEN_REPORT_READS: return "failed to convert the read field in the report from `Kraken2`";
     case SGPU_ERR_KRAKEN_REPORT_DIRECT: return "failed to convert the direct read field in the report from `Kraken2`";
     case SGPU_ERR_KRAKEN_REPORT_PARENT: return "failed to provide a parent taxon while parsing report from `Kraken2`";
-    case SGPU_ERR_FASTA_UNSUPPORTED: return "FASTA input is not supported on this path (shards of a FASTA file)";
+    case SGPU_ERR_FASTA_UNSUPPORTED: return "FASTA input given to a FASTQ shard entry point (use the FASTA shard entry points)";
     case SGPU_ERR_CUDA: return "CUDA error (see sgpu_last_cuda_error)";
     case SGPU_ERR_NOMEM: return "out of memory";
     case SGPU_ERR_INVALID_ARG: return "invalid argument";
@@ -389,32 +392,27 @@ static sgpu_status clean_shard_locked(sgpu_ctx *c, const sgpu_idset *set, const 
                          reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o, counts);
 }
 
+}  // extern "C"
+
 // Host buffers, large input: the file (or one shard of it) goes through the GPU in chunks (shards of one device) so
 // that the host->device copy of chunk k+1.., the kernels of chunk k and the device->host copy of chunk k-1 overlap on
 // three streams -- the end-to-end time approaches the PCIe time of the larger direction instead of the sum.
-// Results are identical to the one-shot path (the same shard logic the multi-GPU driver uses: line phase
-// from the running newline count, the record that straddles a cut belongs to the chunk where it starts).
-// The buffer is a shard in the sense of sgpu_clean_fastq_shard_dev: own bytes [0, own_len) + halo; a whole file is the
-// shard (n_in, n_in, 0, first, last).  newlines_before == SGPU_NEWLINES_UNKNOWN: chunk 0 speculates the line phase, the
-// later chunks continue from it, counts->{own_newlines, lead_newlines} let the caller verify it.
+// Results are identical to the one-shot path (the same shard logic the multi-GPU driver uses; the record that
+// straddles a cut belongs to the chunk where it starts).  The staging, upload and download loop is shared by the
+// formats; `Fmt` holds what differs: the shard call of one chunk and the state the next chunk starts from
+// (FastqChunks: the running newline count; FastaChunks: the line-ending decision).
+// The buffer is a shard: own bytes [0, own_len) + halo; a whole file is the shard (n_in, n_in, first, last).
 // *done = 0: not applicable here (small input, halo too small for a record ...), take the one-shot path.
-static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
-                                        uint64_t newlines_before, int is_first, int is_last, int crlf_in, int reverse,
-                                        uint8_t *out_w, size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o,
-                                        size_t *n_o, sgpu_counts *counts, int *done) {
+template <class Fmt>
+static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, size_t own_len, int is_last, uint8_t *out_w,
+                                 size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o,
+                                 sgpu_counts *counts, int *done, Fmt &fmt) {
     *done = 0;
     // (environment knobs so that tests can drive the chunk logic with small inputs)
     const size_t CHUNK = getenv("SGPU_PIPE_CHUNK") ? (size_t)atoll(getenv("SGPU_PIPE_CHUNK")) & ~(size_t)15
                                                    : (size_t)128 << 20;
     const size_t HALO = getenv("SGPU_PIPE_HALO") ? (size_t)atoll(getenv("SGPU_PIPE_HALO")) : (size_t)8 << 20;
-    if (CHUNK < 4096 || own_len < 2 * CHUNK || c->mode != 0) return SGPU_OK;
-    if (is_first && in[0] != '@') return SGPU_OK;  // FASTA / unknown format: the one-shot path reports it
-    const bool spec = !is_first && newlines_before == SGPU_NEWLINES_UNKNOWN;
-    int crlf = crlf_in > 0;
-    if (is_first) {  // needletail decides the line ending on the first record's first line
-        const uint8_t *nl = (const uint8_t *)memchr(in, '\n', n_in);
-        crlf = nl && nl > in && nl[-1] == '\r';
-    }
+    if (CHUNK < 4096 || own_len < 2 * CHUNK) return SGPU_OK;
     if (!c->s_in) {
         SGPU_CUDA(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
         SGPU_CUDA(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
@@ -423,7 +421,7 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
     const size_t K = ceil_div(own_len, CHUNK);  // kernel chunks: the owned range
     const size_t U = ceil_div(n_in, CHUNK);     // upload pieces: the whole buffer (own range + halo)
     const size_t tail_halo = n_in - own_len;
-    const size_t obuf = CHUNK + std::max(HALO, tail_halo) + 64;
+    const size_t obuf = Fmt::OUT_FACTOR * (CHUNK + std::max(HALO, tail_halo)) + 64;
     // context-owned staging (the context is locked): 0 the file, 1-2 kept chunks, 3-4 removed chunks
     auto staging = [&](int i, size_t bytes, uint8_t **p) -> sgpu_status {
         if (c->pipe_cap[i] < bytes) {
@@ -466,8 +464,6 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
     };
     sgpu_status rc = SGPU_OK;
     size_t off_w = 0, off_o = 0;
-    uint64_t nb = spec ? 0 : newlines_before;  // running count: exact, or relative to the speculated phase
-    uint64_t own_nl_total = 0, lead_nl = 0;
     bool bail = false, unknown = false;
     sgpu_counts total;
     memset(&total, 0, sizeof(total));
@@ -477,8 +473,15 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
     for (; up_next < std::min<size_t>(U, 3) && ce == cudaSuccess; up_next++) ce = upload(up_next);
     for (size_t k = 0; k < K && ce == cudaSuccess && rc == SGPU_OK && !bail; k++) {
         const int r = (int)(k & 1);
-        const size_t a = k * CHUNK, own = std::min(CHUNK, own_len - a);
-        const bool last_chunk = k + 1 == K;
+        const size_t a = k * CHUNK;
+        size_t own = std::min(CHUNK, own_len - a);
+        bool last_chunk = k + 1 == K;
+        if (!last_chunk && is_last && a + own + HALO >= n_in) {
+            // the chunk's buffer reaches EOF: it owns the rest, as only the last chunk may apply the end-of-file rules
+            // (a record that runs to EOF would otherwise be a halo problem and send the whole call to the one-shot path)
+            own = own_len - a;
+            last_chunk = true;
+        }
         const size_t buf_len = last_chunk ? n_in - a : std::min(n_in - a, own + HALO);
         // keep the copy engine three pieces ahead, and at least as far as this chunk's halo reaches
         while (up_next < U && ce == cudaSuccess && (up_next < k + 4 || up_next * CHUNK < a + buf_len)) ce = upload(up_next++);
@@ -488,16 +491,9 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
         if (k >= 2) cudaStreamWaitEvent(st, ev_out[r], 0);
         size_t nw = 0, no = 0;
         sgpu_counts ck;
-        const bool spec0 = spec && k == 0;
-        rc = clean_shard_locked(c, set, d_in.p + a, buf_len, own, spec0 ? SGPU_NEWLINES_UNKNOWN : nb, is_first && k == 0,
-                                last_chunk && is_last, spec0 ? -1 : crlf, reverse, d_w[r].p, obuf, &nw,
-                                out_o ? d_o[r].p : nullptr, obuf, &no, &ck, true);
-        if (getenv("SGPU_DEBUG"))
-            fprintf(stderr, "[sgpu] pipe chunk %zu/%zu a=%zu own=%zu buf=%zu nlb=%llu -> rc=%d nw=%zu no=%zu in=%llu out=%llu path=%u own_nl=%llu lead_nl=%llu\n",
-                    k, K, a, own, buf_len, (unsigned long long)nb, (int)rc, nw, no,
-                    (unsigned long long)ck.reads_in, (unsigned long long)ck.reads_out, ck.path,
-                    (unsigned long long)ck.own_newlines, (unsigned long long)ck.lead_newlines);
-        if (rc == SGPU_ERR_PHASE_UNKNOWN || (spec && rc == SGPU_OK && ck.path != 1)) {
+        rc = fmt.run(c, k, a, d_in.p + a, buf_len, own, last_chunk && is_last, d_w[r].p, out_o ? d_o[r].p : nullptr, obuf,
+                     &nw, &no, &ck);
+        if (fmt.unknown(rc, ck)) {
             rc = SGPU_OK;  // speculation not applicable: the caller comes back with the exact phase
             unknown = true;
             break;
@@ -531,15 +527,8 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
             rc = parse_rc;
             break;
         }
-        // this chunk's newlines: a by-product of the single-pass kernel, else one counting pass
-        uint64_t cnt = ck.own_newlines;
-        if (ck.path != 1 && (!last_chunk || crlf_in < 0)) rc = count_newlines(c, d_in.p + a, own, &cnt);
-        if (spec0) {
-            lead_nl = ck.lead_newlines;
-            nb = (4 - (lead_nl & 3)) & 3;  // the phase the speculation stands for
-        }
-        nb += cnt;
-        own_nl_total += cnt;
+        rc = fmt.advance(c, k, d_in.p + a, own, last_chunk, ck);
+        if (last_chunk) break;
     }
     cudaStreamSynchronize(c->s_in);
     cudaStreamSynchronize(c->s_out);
@@ -563,13 +552,143 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
     if (bail) return SGPU_OK;  // *done stays 0
     *done = 1;
     *counts = total;
-    counts->own_newlines = own_nl_total;
-    counts->lead_newlines = lead_nl;
-    counts->speculated = spec ? 1 : 0;
+    fmt.finish(counts);
     *n_w = off_w;
     if (n_o) *n_o = out_o ? off_o : 0;
     return rc;
 }
+
+// FASTQ: the line phase of chunk k+1 comes from the running newline count.  newlines_before == SGPU_NEWLINES_UNKNOWN:
+// chunk 0 speculates the line phase, the later chunks continue from it, counts->{own_newlines, lead_newlines} let the
+// caller verify it.
+struct FastqChunks {
+    static constexpr size_t OUT_FACTOR = 1;
+    const sgpu_idset *set;
+    int is_first, crlf_in, reverse;
+    bool spec;
+    int crlf;
+    uint64_t nb;  // running count: exact, or relative to the speculated phase
+    uint64_t own_nl_total = 0, lead_nl = 0;
+
+    sgpu_status run(sgpu_ctx *c, size_t k, size_t a, const uint8_t *d, size_t buf_len, size_t own, bool last, uint8_t *dw,
+                    uint8_t *dov, size_t obuf, size_t *nw, size_t *no, sgpu_counts *ck) {
+        const bool spec0 = spec && k == 0;
+        const sgpu_status rc = clean_shard_locked(c, set, d, buf_len, own, spec0 ? SGPU_NEWLINES_UNKNOWN : nb,
+                                                  is_first && k == 0, last, spec0 ? -1 : crlf, reverse, dw, obuf, nw, dov,
+                                                  obuf, no, ck, true);
+        if (getenv("SGPU_DEBUG"))
+            fprintf(stderr, "[sgpu] pipe chunk %zu a=%zu own=%zu buf=%zu nlb=%llu -> rc=%d nw=%zu no=%zu in=%llu out=%llu path=%u own_nl=%llu lead_nl=%llu\n",
+                    k, a, own, buf_len, (unsigned long long)nb, (int)rc, *nw, *no,
+                    (unsigned long long)ck->reads_in, (unsigned long long)ck->reads_out, ck->path,
+                    (unsigned long long)ck->own_newlines, (unsigned long long)ck->lead_newlines);
+        return rc;
+    }
+    bool unknown(sgpu_status rc, const sgpu_counts &ck) const {
+        return rc == SGPU_ERR_PHASE_UNKNOWN || (spec && rc == SGPU_OK && ck.path != 1);
+    }
+    sgpu_status advance(sgpu_ctx *c, size_t k, const uint8_t *d, size_t own, bool last_chunk, const sgpu_counts &ck) {
+        // this chunk's newlines: a by-product of the single-pass kernel, else one counting pass
+        sgpu_status rc = SGPU_OK;
+        uint64_t cnt = ck.own_newlines;
+        if (ck.path != 1 && (!last_chunk || crlf_in < 0)) rc = count_newlines(c, d, own, &cnt);
+        if (spec && k == 0) {
+            lead_nl = ck.lead_newlines;
+            nb = (4 - (lead_nl & 3)) & 3;  // the phase the speculation stands for
+        }
+        nb += cnt;
+        own_nl_total += cnt;
+        return rc;
+    }
+    void finish(sgpu_counts *counts) const {
+        counts->own_newlines = own_nl_total;
+        counts->lead_newlines = lead_nl;
+        counts->speculated = spec ? 1 : 0;
+    }
+};
+
+static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
+                                        uint64_t newlines_before, int is_first, int is_last, int crlf_in, int reverse,
+                                        uint8_t *out_w, size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o,
+                                        size_t *n_o, sgpu_counts *counts, int *done) {
+    *done = 0;
+    if (c->mode != 0) return SGPU_OK;
+    if (is_first && n_in && in[0] != '@') return SGPU_OK;  // FASTA / unknown format: not this format's pipeline
+    const bool spec = !is_first && newlines_before == SGPU_NEWLINES_UNKNOWN;
+    int crlf = crlf_in > 0;
+    if (is_first) {  // needletail decides the line ending on the first record's first line
+        const uint8_t *nl = (const uint8_t *)memchr(in, '\n', n_in);
+        crlf = nl && nl > in && nl[-1] == '\r';
+    }
+    FastqChunks f{set, is_first, crlf_in, reverse, spec, crlf, spec ? 0 : newlines_before};
+    return pipeline_host(c, in, n_in, own_len, is_last, out_w, cap_w, n_w, out_o, cap_o, n_o, counts, done, f);
+}
+
+// FASTA: chunk k+1 starts from chunk k's line-ending state, le_before(k) when that was decided, else le_own(k) -- exact,
+// nothing is speculated.  A chunk's output is at most twice its records' bytes (">a\n" -> ">a\r\n\r\n").
+struct FastaChunks {
+    static constexpr size_t OUT_FACTOR = 2;
+    const sgpu_idset *set;
+    int is_first, reverse;
+    int le;            // le_before of the next chunk
+    int le_own = -1;   // the shard's own decision: the first chunk's that has one
+    int le_chunk = -1;
+
+    sgpu_status run(sgpu_ctx *c, size_t k, size_t, const uint8_t *d, size_t buf_len, size_t own, bool last, uint8_t *dw,
+                    uint8_t *dov, size_t obuf, size_t *nw, size_t *no, sgpu_counts *ck) {
+        memset(ck, 0, sizeof(*ck));
+        *nw = *no = 0;
+        const sgpu_status rc = clean_fasta_shard(c, set, d, buf_len, own, is_first && k == 0, last, le, reverse, dw, obuf, nw,
+                                                 dov, obuf, no, ck, &le_chunk);
+        if (le_own < 0) le_own = le_chunk;  // (also from a chunk that stops on a parse error: decided before the error)
+        return rc;
+    }
+    bool unknown(sgpu_status, const sgpu_counts &) const { return false; }
+    sgpu_status advance(sgpu_ctx *, size_t, const uint8_t *, size_t, bool, const sgpu_counts &) {
+        if (le < 0) le = le_chunk;
+        return SGPU_OK;
+    }
+    void finish(sgpu_counts *) const {}
+};
+
+static sgpu_status fasta_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
+                                        int is_first, int is_last, int le_before, int reverse, uint8_t *out_w, size_t cap_w,
+                                        size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
+                                        int *le_own, int *done) {
+    FastaChunks f{set, is_first, reverse, le_before};
+    const sgpu_status rc =
+        pipeline_host(c, in, n_in, own_len, is_last, out_w, cap_w, n_w, out_o, cap_o, n_o, counts, done, f);
+    *le_own = f.le_own;
+    return rc;
+}
+
+// the one-shot host path: the whole buffer on the device, `call(d_in, d_w, cap_w, d_o, cap_o)` on it, outputs back.
+// write_fastq's output is the input re-serialised: larger only when line endings are rewritten (FASTQ: LF records
+// after a CRLF first record) or FASTA header-only records gain an empty sequence line.  Device buffers are sized for
+// the common case first.
+template <class Call>
+static sgpu_status oneshot_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, uint8_t *out_w, size_t cap_w, size_t *n_w,
+                                uint8_t *out_o, size_t cap_o, size_t *n_o, Call call) {
+    cudaStream_t st = c->stream;
+    DevBuf<uint8_t> d_in, d_w, d_o;
+    SGPU_TRY(d_in.alloc(n_in + 16, st));
+    if (n_in) SGPU_CUDA(cudaMemcpyAsync(d_in.p, in, n_in, cudaMemcpyHostToDevice, st));
+    sgpu_status rc = SGPU_OK;
+    for (int attempt = 0; attempt < 2; attempt++) {
+        const size_t want = attempt ? ~(size_t)0 : n_in + n_in / 16 + 4096;
+        const size_t dcap_w = std::min(cap_w, want), dcap_o = std::min(cap_o, want);
+        SGPU_TRY(d_w.alloc(dcap_w + 16, st));
+        if (out_o) SGPU_TRY(d_o.alloc(dcap_o + 16, st));
+        rc = call(d_in.p, d_w.p, dcap_w, out_o ? d_o.p : nullptr, dcap_o);
+        if (rc != SGPU_ERR_CAPACITY || (dcap_w == cap_w && (!out_o || dcap_o == cap_o))) break;
+    }
+    if (rc == SGPU_ERR_CAPACITY || rc == SGPU_ERR_CUDA || rc == SGPU_ERR_NOMEM || rc == SGPU_ERR_PHASE_UNKNOWN) return rc;
+    if (*n_w) SGPU_CUDA(cudaMemcpyAsync(out_w, d_w.p, *n_w, cudaMemcpyDeviceToHost, st));
+    if (out_o && n_o && *n_o) SGPU_CUDA(cudaMemcpyAsync(out_o, d_o.p, *n_o, cudaMemcpyDeviceToHost, st));
+    SGPU_CUDA(cudaStreamSynchronize(st));
+    return rc;
+}
+
+extern "C" {
 
 sgpu_status sgpu_clean_fastq(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, int reverse,
                              uint8_t *out_w, size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o,
@@ -577,33 +696,19 @@ sgpu_status sgpu_clean_fastq(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *
     if (!c || !set || !n_w || !counts || (n_in && !in) || (cap_w && !out_w)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = c->stream;
     {
-        int done = 0;
-        sgpu_status prc = clean_host_pipelined(c, set, in, n_in, n_in, 0, 1, 1, -1, reverse, out_w, cap_w, n_w, out_o,
-                                               cap_o, n_o, counts, &done);
+        int done = 0, le_own;
+        sgpu_status prc = n_in >= 5 && in[0] == '>'
+                              ? fasta_host_pipelined(c, set, in, n_in, n_in, 1, 1, -1, reverse, out_w, cap_w, n_w, out_o,
+                                                     cap_o, n_o, counts, &le_own, &done)
+                              : clean_host_pipelined(c, set, in, n_in, n_in, 0, 1, 1, -1, reverse, out_w, cap_w, n_w, out_o,
+                                                     cap_o, n_o, counts, &done);
         if (done || prc != SGPU_OK) return prc;
     }
-    DevBuf<uint8_t> d_in, d_w, d_o;
-    SGPU_TRY(d_in.alloc(n_in + 16, st));
-    if (n_in) SGPU_CUDA(cudaMemcpyAsync(d_in.p, in, n_in, cudaMemcpyHostToDevice, st));
-    // write_fastq's output is the input re-serialised: larger only when LF records follow a CRLF first record (every
-    // record is then written with CRLF, +4 bytes each).  Device buffers are sized for the common case first.
-    sgpu_status rc = SGPU_OK;
-    for (int attempt = 0; attempt < 2; attempt++) {
-        const size_t want = attempt ? ~(size_t)0 : n_in + n_in / 16 + 4096;
-        const size_t dcap_w = std::min(cap_w, want), dcap_o = std::min(cap_o, want);
-        SGPU_TRY(d_w.alloc(dcap_w + 16, st));
-        if (out_o) SGPU_TRY(d_o.alloc(dcap_o + 16, st));
-        rc = clean_dev_locked(c, set, d_in.p, n_in, reverse, d_w.p, dcap_w, n_w, out_o ? d_o.p : nullptr, dcap_o, n_o,
-                              counts);
-        if (rc != SGPU_ERR_CAPACITY || (dcap_w == cap_w && (!out_o || dcap_o == cap_o))) break;
-    }
-    if (rc == SGPU_ERR_CAPACITY || rc == SGPU_ERR_CUDA || rc == SGPU_ERR_NOMEM) return rc;
-    if (*n_w) SGPU_CUDA(cudaMemcpyAsync(out_w, d_w.p, *n_w, cudaMemcpyDeviceToHost, st));
-    if (out_o && n_o && *n_o) SGPU_CUDA(cudaMemcpyAsync(out_o, d_o.p, *n_o, cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(cudaStreamSynchronize(st));
-    return rc;
+    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
+                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
+                            return clean_dev_locked(c, set, d_in, n_in, reverse, d_w, dcap_w, n_w, d_o, dcap_o, n_o, counts);
+                        });
 }
 
 sgpu_status sgpu_clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
@@ -616,30 +721,115 @@ sgpu_status sgpu_clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const uin
         return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = c->stream;
     {
         int done = 0;
         sgpu_status prc = clean_host_pipelined(c, set, in, n_in, own_len, newlines_before, is_first, is_last, crlf, reverse,
                                                out_w, cap_w, n_w, out_o, cap_o, n_o, counts, &done);
         if (done || prc != SGPU_OK) return prc;
     }
-    DevBuf<uint8_t> d_in, d_w, d_o;
-    SGPU_TRY(d_in.alloc(n_in + 16, st));
-    if (n_in) SGPU_CUDA(cudaMemcpyAsync(d_in.p, in, n_in, cudaMemcpyHostToDevice, st));
-    sgpu_status rc = SGPU_OK;
-    for (int attempt = 0; attempt < 2; attempt++) {
-        const size_t want = attempt ? ~(size_t)0 : n_in + n_in / 16 + 4096;
-        const size_t dcap_w = std::min(cap_w, want), dcap_o = std::min(cap_o, want);
-        SGPU_TRY(d_w.alloc(dcap_w + 16, st));
-        if (out_o) SGPU_TRY(d_o.alloc(dcap_o + 16, st));
-        rc = clean_shard_locked(c, set, d_in.p, n_in, own_len, newlines_before, is_first, is_last, crlf, reverse, d_w.p,
-                                dcap_w, n_w, out_o ? d_o.p : nullptr, dcap_o, n_o, counts, crlf < 0);
-        if (rc != SGPU_ERR_CAPACITY || (dcap_w == cap_w && (!out_o || dcap_o == cap_o))) break;
+    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
+                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
+                            return clean_shard_locked(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, crlf,
+                                                      reverse, d_w, dcap_w, n_w, d_o, dcap_o, n_o, counts, crlf < 0);
+                        });
+}
+
+// argument checks shared by the FASTA shard entry points
+static bool fasta_shard_args_ok(size_t n_in, size_t own_len, int is_last, int le_before, int is_first) {
+    return own_len <= n_in && (!is_last || own_len == n_in) && le_before >= -1 && le_before <= 1 &&
+           (!is_first || le_before == -1);
+}
+
+// the FASTA shard's first byte and the empty-input rule (context locked).  *empty: a first-and-last shard of fewer
+// than 5 bytes (utils.rs:359-375); SGPU_ERR_INVALID_ARG: a first shard that does not start with '>'
+static sgpu_status fasta_shard_head(sgpu_ctx *c, const uint8_t *buf, bool on_device, size_t n_in, int is_first,
+                                    int is_last, bool *empty) {
+    *empty = is_first && is_last && n_in < 5;
+    if (*empty || !is_first) return SGPU_OK;
+    if (n_in == 0) return SGPU_ERR_INVALID_ARG;
+    if (!on_device) return buf[0] == '>' ? SGPU_OK : SGPU_ERR_INVALID_ARG;
+    SGPU_CUDA(cudaMemcpyAsync(c->h_pinned, buf, 1, cudaMemcpyDeviceToHost, c->stream));
+    SGPU_CUDA(cudaStreamSynchronize(c->stream));
+    return *(uint8_t *)c->h_pinned == '>' ? SGPU_OK : SGPU_ERR_INVALID_ARG;
+}
+
+sgpu_status sgpu_clean_fasta_shard_dev(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
+                                       size_t own_len, int is_first, int is_last, int le_before, int reverse,
+                                       uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o,
+                                       size_t *n_o, sgpu_counts *counts, int *le_own) {
+    if (!c || !set || !n_w || !counts || !le_own || (n_in && !d_in) || (cap_w && !d_out_w) ||
+        !fasta_shard_args_ok(n_in, own_len, is_last, le_before, is_first))
+        return SGPU_ERR_INVALID_ARG;
+    if (n_in && ((uintptr_t)d_in & 15)) return SGPU_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(c->mu);
+    SGPU_CUDA(cudaSetDevice(c->device));
+    memset(counts, 0, sizeof(*counts));
+    *n_w = 0;
+    if (n_o) *n_o = 0;
+    *le_own = -1;
+    bool empty;
+    SGPU_TRY(fasta_shard_head(c, d_in, true, n_in, is_first, is_last, &empty));
+    if (empty) {
+        counts->empty_input = 1;
+        return SGPU_OK;
     }
-    if (rc == SGPU_ERR_CAPACITY || rc == SGPU_ERR_CUDA || rc == SGPU_ERR_NOMEM || rc == SGPU_ERR_PHASE_UNKNOWN) return rc;
-    if (*n_w) SGPU_CUDA(cudaMemcpyAsync(out_w, d_w.p, *n_w, cudaMemcpyDeviceToHost, st));
-    if (out_o && n_o && *n_o) SGPU_CUDA(cudaMemcpyAsync(out_o, d_o.p, *n_o, cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(cudaStreamSynchronize(st));
+    return clean_fasta_shard(c, set, d_in, n_in, own_len, is_first, is_last, le_before, reverse, d_out_w, cap_w, n_w, d_out_o,
+                             cap_o, n_o, counts, le_own);
+}
+
+sgpu_status sgpu_clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
+                                   int is_first, int is_last, int le_before, int reverse, uint8_t *out_w, size_t cap_w,
+                                   size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
+                                   int *le_own) {
+    if (!c || !set || !n_w || !counts || !le_own || (n_in && !in) || (cap_w && !out_w) ||
+        !fasta_shard_args_ok(n_in, own_len, is_last, le_before, is_first))
+        return SGPU_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(c->mu);
+    SGPU_CUDA(cudaSetDevice(c->device));
+    memset(counts, 0, sizeof(*counts));
+    *n_w = 0;
+    if (n_o) *n_o = 0;
+    *le_own = -1;
+    bool empty;
+    SGPU_TRY(fasta_shard_head(c, in, false, n_in, is_first, is_last, &empty));
+    if (empty) {
+        counts->empty_input = 1;
+        return SGPU_OK;
+    }
+    {
+        int done = 0;
+        sgpu_status prc = fasta_host_pipelined(c, set, in, n_in, own_len, is_first, is_last, le_before, reverse, out_w, cap_w,
+                                               n_w, out_o, cap_o, n_o, counts, le_own, &done);
+        if (done || prc != SGPU_OK) return prc;
+    }
+    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
+                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
+                            memset(counts, 0, sizeof(*counts));
+                            return clean_fasta_shard(c, set, d_in, n_in, own_len, is_first, is_last, le_before, reverse, d_w,
+                                                     dcap_w, n_w, d_o, dcap_o, n_o, counts, le_own);
+                        });
+}
+
+sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
+                                     size_t own_len, int is_first, int is_last, sgpu_idset *into, sgpu_counts *counts) {
+    if (!c || !counts || (n_buf && !d_buf) || !fasta_shard_args_ok(n_buf, own_len, is_last, -1, is_first))
+        return SGPU_ERR_INVALID_ARG;
+    if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(c->mu);
+    SGPU_CUDA(cudaSetDevice(c->device));
+    bool empty;
+    SGPU_TRY(fasta_shard_head(c, d_buf, true, n_buf, is_first, is_last, &empty));
+    if (empty) return SGPU_OK;
+    uint64_t n_rec = 0, n_pick = 0, err = 0;
+    sgpu_status rc = fasta_ids_shard(c, d_buf, n_buf, own_len, is_first, is_last, probe, probe != nullptr, into, &n_rec,
+                                     &n_pick, &err);
+    if (rc == SGPU_OK) {
+        counts->reads_in += n_rec;
+        counts->difference += n_pick;
+    } else {
+        counts->error_record = err;
+    }
+    cudaStreamSynchronize(c->stream);
     return rc;
 }
 

@@ -13,9 +13,10 @@
 //   holds a newline, records written before that use LF;
 //   output  : '>' id E raw_seq E.
 //
-// Pipeline (whole file on one device; shards of a FASTA file are not built):
-//   newline index (scan.cu) -> mark the newlines followed by '>' -> scan -> record table -> thread per record
-//   (spans, get_id, probe) -> line-ending decision -> lengths -> scans -> warp per record copy.
+// Pipeline (a whole file, or one shard of it: the contract is written down in include/scrubby_gpu.h):
+//   newline index (scan.cu) -> mark the newlines followed by '>' (and count the owned ones) -> scan -> record table ->
+//   thread per owned record (spans, get_id, probe) -> line-ending decision -> lengths -> scans -> warp per record copy.
+// A whole file is the shard (own_len = n, is_first = 1, is_last = 1, le_before = -1).
 #include "fastq_records.cuh"
 
 namespace sgpu {
@@ -25,8 +26,10 @@ struct FaParams {
     uint64_t n_in;
     const uint64_t *nlpos;
     uint64_t n_nl;
-    const uint64_t *rec_nl;  // record k >= 1 starts right after newline rec_nl[k]; rec_nl[0] is unused
-    uint64_t n_rec;
+    const uint64_t *rec_nl;  // record k starts right after newline rec_nl[k] (record 0 of a first shard: at byte 0)
+    uint64_t n_rec;          // records the shard owns
+    uint64_t n_tab;          // entries of rec_nl: the owned records + the next record start, when the buffer holds it
+    int at0;                 // record 0 starts at byte 0 (first shard); rec_nl[0] is then unused
 };
 
 struct FaMeta {
@@ -36,11 +39,19 @@ struct FaMeta {
     uint32_t pad;
 };
 
-__global__ void fa_mark_kernel(const uint8_t *in, uint64_t n_in, const uint64_t *nlpos, uint64_t n_nl, uint32_t *mark) {
+// record starts: a '>' that follows a newline; the shard owns those with the newline before own_len
+__global__ void fa_mark_kernel(const uint8_t *in, uint64_t n_in, const uint64_t *nlpos, uint64_t n_nl, uint64_t own_len,
+                               uint32_t *mark, unsigned long long *n_owned) {
     const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_nl) return;
-    const uint64_t p = nlpos[j];
-    mark[j] = (p + 1 < n_in && in[p + 1] == '>') ? 1u : 0u;
+    uint32_t m = 0;
+    uint64_t p = 0;
+    if (j < n_nl) {
+        p = nlpos[j];
+        m = (p + 1 < n_in && in[p + 1] == '>') ? 1u : 0u;
+        mark[j] = m;
+    }
+    const int owned = __syncthreads_count(m && p < own_len);
+    if (threadIdx.x == 0 && owned) atomicAdd(n_owned, (unsigned long long)owned);
 }
 
 __global__ void fa_scatter_kernel(const uint32_t *mark, const uint64_t *rank, uint64_t n_nl, uint64_t *rec_nl) {
@@ -49,19 +60,24 @@ __global__ void fa_scatter_kernel(const uint32_t *mark, const uint64_t *rank, ui
     if (mark[j]) rec_nl[rank[j] + 1] = j;
 }
 
+__device__ __forceinline__ uint64_t fa_start(const FaParams &P, uint64_t k) {
+    return (k == 0 && P.at0) ? 0 : P.nlpos[P.rec_nl[k]] + 1;
+}
+
 // start byte, first / last position of record k; false when the record has no position (UnexpectedEnd)
 __device__ __forceinline__ bool fa_locate(const FaParams &P, uint64_t k, uint64_t *start, uint64_t *first, uint64_t *last,
                                           uint32_t *npos) {
-    const uint64_t f = k ? P.rec_nl[k] + 1 : 0;  // index of the first newline at or after the record's start
-    *start = k ? P.nlpos[P.rec_nl[k]] + 1 : 0;
-    if (k + 1 < P.n_rec) {  // the newline in front of the next '>' closes the record
+    const uint64_t f = (k == 0 && P.at0) ? 0 : P.rec_nl[k] + 1;  // index of the first newline at or after the start
+    *start = fa_start(P, k);
+    if (k + 1 < P.n_tab) {  // the newline in front of the next '>' closes the record
         const uint64_t l = P.rec_nl[k + 1];
         *first = P.nlpos[f];
         *last = P.nlpos[l];
         *npos = (uint32_t)(l - f + 1 > 2 ? 2 : l - f + 1);
         return true;
     }
-    // the last record: newlines f .. n_nl-1; one on the input's last byte only counts after another one
+    // the last record of the input (only the last shard gets here): newlines f .. n_nl-1; one on the input's last byte
+    // only counts after another one
     uint64_t cnt = P.n_nl > f ? P.n_nl - f : 0;
     const bool trailing = cnt && P.nlpos[P.n_nl - 1] + 1 == P.n_in;
     if (trailing && cnt == 1) cnt = 0;
@@ -162,7 +178,7 @@ __global__ void __launch_bounds__(256)
         if (!out_o) return;
         dst = out_o + off_o[k];
     }
-    const uint64_t start = k ? P.nlpos[P.rec_nl[k]] + 1 : 0;
+    const uint64_t start = fa_start(P, k);
     const uint32_t e = (crlf && k >= le_from) ? 2u : 1u;
     if (lane == 0) dst[0] = '>';
     warp_copy(dst + 1, P.in + start + 1, m.id_n, lane);
@@ -186,7 +202,7 @@ __global__ void fa_count_sel_kernel(const uint8_t *sel, uint64_t n, unsigned lon
     if (threadIdx.x == 0 && b) atomicAdd(counter, (unsigned long long)b);
 }
 
-// the record table of a FASTA buffer + the per-record pass; shared by clean and ids
+// the record table of a FASTA shard + the per-record pass; shared by clean and ids
 struct FaTables {
     DevBuf<uint64_t> nlpos, rank, rec_nl, key_off, scratch;
     DevBuf<uint32_t> mark, key_len;
@@ -196,57 +212,76 @@ struct FaTables {
     uint64_t err_word = ~0ull, le_from = ~0ull;
 };
 
-static sgpu_status fasta_records(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, const sgpu_idset *set, int reverse,
-                                 int want_absent, bool want_keys, FaTables &T) {
+// SGPU_ERR_HALO: a shard that is not the last one does not hold the start of the record after its last owned one.
+// T.P.n_rec == 0: the shard owns no record (nothing was launched after the table)
+static sgpu_status fasta_records(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, size_t own_len, int is_first, int is_last,
+                                 const sgpu_idset *set, int reverse, int want_absent, bool want_keys, FaTables &T) {
     cudaStream_t st = c->stream;
+    // [0] err word, [1] first record that decides the line ending, [2] starts, [3..4] counters, [5..6] totals, [7] owned starts
+    SGPU_TRY(T.scratch.alloc(8, st));
+    const uint64_t init[8] = {~0ull, ~0ull, 0, 0, 0, 0, 0, 0};
+    memcpy(c->h_pinned + 32, init, sizeof(init));
+    SGPU_CUDA(cudaMemcpyAsync(T.scratch.p, c->h_pinned + 32, sizeof(init), cudaMemcpyHostToDevice, st));
     uint64_t n_nl = 0;
     SGPU_TRY(index_newlines(c, d_in, n_in, T.nlpos, &n_nl));
-    uint64_t n_starts = 0;
-    SGPU_TRY(T.scratch.alloc(8, st));  // [0] err word, [1] first record that decides the line ending, [2] starts, [3..4] counters, [5..6] totals
+    uint64_t h[6] = {0, 0, 0, 0, 0, 0};  // scratch [2..7]
     if (n_nl) {
         SGPU_TRY(T.mark.alloc(n_nl, st));
         SGPU_TRY(T.rank.alloc(n_nl, st));
-        fa_mark_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(d_in, n_in, T.nlpos.p, n_nl, T.mark.p);
+        fa_mark_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(d_in, n_in, T.nlpos.p, n_nl, own_len,
+                                                                                T.mark.p,
+                                                                                (unsigned long long *)(T.scratch.p + 7));
         SGPU_LAUNCH(c);
         SGPU_TRY(exclusive_scan_u32_to_u64(c, T.mark.p, T.rank.p, n_nl, T.scratch.p + 2));
-        SGPU_TRY(read_u64s(c, T.scratch.p + 2, &n_starts, 1));
+        SGPU_TRY(read_u64s(c, T.scratch.p + 2, h, 6));
     }
-    const uint64_t n_rec = n_starts + 1;
-    SGPU_TRY(T.rec_nl.alloc(n_rec, st));
+    const uint64_t n_starts = h[0], n_owned = h[5];
+    const uint64_t n_rec = (is_first ? 1 : 0) + n_owned;
+    const uint64_t n_tab = (is_first ? 1 : 0) + n_starts;
+    T.P = FaParams{d_in, (uint64_t)n_in, T.nlpos.p, n_nl, nullptr, n_rec, n_tab, is_first ? 1 : 0};
+    if (n_rec == 0) return SGPU_OK;
+    if (!is_last && n_tab == n_rec) return SGPU_ERR_HALO;  // the end of the last owned record is not in the buffer
+    SGPU_TRY(T.rec_nl.alloc(n_starts + 1, st));
     if (n_starts) {
         fa_scatter_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(T.mark.p, T.rank.p, n_nl, T.rec_nl.p);
         SGPU_LAUNCH(c);
     }
-    T.P = FaParams{d_in, (uint64_t)n_in, T.nlpos.p, n_nl, T.rec_nl.p, n_rec};
+    T.P.rec_nl = T.rec_nl.p + (is_first ? 0 : 1);  // table entry 0 stands for byte 0
     SGPU_TRY(T.meta.alloc(n_rec, st));
     if (want_keys) {
         SGPU_TRY(T.key_off.alloc(n_rec, st));
         SGPU_TRY(T.key_len.alloc(n_rec, st));
         SGPU_TRY(T.sel.alloc(n_rec, st));
     }
-    const uint64_t init[8] = {~0ull, ~0ull, 0, 0, 0, 0, 0, 0};
-    memcpy(c->h_pinned + 32, init, sizeof(init));
-    SGPU_CUDA(cudaMemcpyAsync(T.scratch.p, c->h_pinned + 32, sizeof(init), cudaMemcpyHostToDevice, st));
     fa_record_kernel<<<(unsigned)ceil_div(n_rec, (uint64_t)128), 128, 0, st>>>(
         T.P, view_of(set), reverse, want_absent, T.meta.p, want_keys ? T.key_off.p : nullptr,
         want_keys ? T.key_len.p : nullptr, want_keys ? T.sel.p : nullptr, (unsigned long long *)T.scratch.p,
         (unsigned long long *)(T.scratch.p + 1));
     SGPU_LAUNCH(c);
-    uint64_t h[2];
-    SGPU_TRY(read_u64s(c, T.scratch.p, h, 2));
-    T.err_word = h[0];
-    T.le_from = h[1];
+    uint64_t e[2];
+    SGPU_TRY(read_u64s(c, T.scratch.p, e, 2));
+    T.err_word = e[0];
+    T.le_from = e[1];
     return SGPU_OK;
 }
 
-// FastqCleaner::clean_reads over FASTA records.  Device pointers in, device outputs filled, counts on the host.
-sgpu_status clean_fasta(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse, uint8_t *d_out_w,
-                        size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts) {
+// FastqCleaner::clean_reads over the FASTA records a shard owns.  Device pointers in, device outputs filled, counts on
+// the host.  le_before: -1 undecided, 0 / 1 LF / CRLF decided by an earlier shard; *le_own: what this shard's first
+// deciding record (before an error) says, -1 when it has none.
+sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
+                              int is_first, int is_last, int le_before, int reverse, uint8_t *d_out_w, size_t cap_w,
+                              size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
+                              int *le_own) {
     cudaStream_t st = c->stream;
     counts->path = 3;
+    *le_own = -1;
     FaTables T;
-    SGPU_TRY(fasta_records(c, d_in, n_in, set, reverse, 0, false, T));
+    SGPU_TRY(fasta_records(c, d_in, n_in, own_len, is_first, is_last, set, reverse, 0, false, T));
     const uint64_t n_rec = T.P.n_rec;
+    if (n_rec == 0) {
+        counts->crlf = le_before > 0;
+        return SGPU_OK;
+    }
     sgpu_status rc = SGPU_OK;
     uint64_t err_from = ~0ull;
     if (T.err_word != ~0ull) {
@@ -263,8 +298,13 @@ sgpu_status clean_fasta(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in,
         SGPU_CUDA(cudaStreamSynchronize(st));
         memcpy(&m, c->h_pinned + 32, sizeof(m));
         crlf = (m.flags & 8u) ? 1 : 0;
+        *le_own = crlf;
     } else {
         le_from = ~0ull;
+    }
+    if (le_before >= 0) {  // an earlier shard decided: every record of this one uses it
+        crlf = le_before;
+        le_from = 0;
     }
     counts->crlf = (uint32_t)crlf;
     DevBuf<uint32_t> len_w, len_o;
@@ -295,18 +335,21 @@ sgpu_status clean_fasta(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in,
     return rc;
 }
 
-// one loop of ReadDifference::get_difference (utils.rs:259-267 / 269-283) over a FASTA buffer
-sgpu_status fasta_ids_into(sgpu_ctx *c, const uint8_t *d_buf, size_t n, const sgpu_idset *probe, int want_absent,
-                           sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record) {
+// one loop of ReadDifference::get_difference (utils.rs:259-267 / 269-283) over the FASTA records a shard owns
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t own_len, int is_first, int is_last,
+                            const sgpu_idset *probe, int want_absent, sgpu_idset *into, uint64_t *n_records,
+                            uint64_t *n_picked, uint64_t *err_record) {
+    *n_records = *n_picked = 0;
     FaTables T;
-    SGPU_TRY(fasta_records(c, d_buf, n, want_absent ? probe : nullptr, 0, want_absent, true, T));
+    SGPU_TRY(fasta_records(c, d_buf, n, own_len, is_first, is_last, want_absent ? probe : nullptr, 0, want_absent, true, T));
+    const uint64_t n_rec = T.P.n_rec;
+    if (n_rec == 0) return SGPU_OK;
     if (T.err_word != ~0ull) {
         if (err_record) *err_record = T.err_word >> 8;
         return (sgpu_status)(T.err_word & 0xFF);
     }
     // every record is valid here; picked = the selected spans
     cudaStream_t st = c->stream;
-    const uint64_t n_rec = T.P.n_rec;
     fa_count_sel_kernel<<<(unsigned)ceil_div(n_rec, (uint64_t)256), 256, 0, st>>>(T.sel.p, n_rec,
                                                                                  (unsigned long long *)(T.scratch.p + 3));
     SGPU_LAUNCH(c);

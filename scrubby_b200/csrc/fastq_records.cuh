@@ -118,10 +118,14 @@ sgpu_status clean_general(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_i
                           uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
                           sgpu_counts *counts);
 
-// fasta_general.cu: the same two operations over FASTA records (needletail's FASTA reader; whole files only)
-sgpu_status clean_fasta(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse, uint8_t *d_out_w,
-                        size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts);
-sgpu_status fasta_ids_into(sgpu_ctx *c, const uint8_t *d_buf, size_t n, const sgpu_idset *probe, int want_absent,
-                           sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record);
+// fasta_general.cu: the same two operations over the FASTA records a shard owns (needletail's FASTA reader; a whole
+// file is the shard (n, n, first, last)); the shard contract is sgpu_clean_fasta_shard_dev's
+sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
+                              int is_first, int is_last, int le_before, int reverse, uint8_t *d_out_w, size_t cap_w,
+                              size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
+                              int *le_own);
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t own_len, int is_first, int is_last,
+                            const sgpu_idset *probe, int want_absent, sgpu_idset *into, uint64_t *n_records,
+                            uint64_t *n_picked, uint64_t *err_record);
 
 }  // namespace sgpu

@@ -105,6 +105,10 @@ class GpuOps:
         return self.api.fastq_ids_shard_dev(self.ctx, probe, d_buf, sh.buf_len, sh.own_len, newlines_before,
                                             sh.is_first, sh.is_last, into)
 
+    def fasta_ids_shard(self, probe, d_buf, sh: Shard, into):
+        """the same for a FASTA file (no line phase: a record starts at any '>' after a newline)"""
+        return self.api.fasta_ids_shard_dev(self.ctx, probe, d_buf, sh.buf_len, sh.own_len, sh.is_first, sh.is_last, into)
+
     def set_ids(self, ids):
         return ids.sorted_ids()
 
@@ -233,23 +237,26 @@ class ShardedDiff:
     diff_ids: list      # sorted unique ids of the input records missing from their output file (every rank)
 
 
-def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo):
+def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo, fasta=False):
     """one loop of ReadDifference::get_difference over one file, every rank on its own byte range; the set of the
     rank's ids goes to `collect`; returns the (records, picked) totals of this rank.  A record longer than the halo
-    makes all ranks retry with a larger one."""
+    makes all ranks retry with a larger one.  FASTA shards need no newline counts."""
     world = dist.get_world_size() if dist is not None else 1
     rank = dist.get_rank() if dist is not None else 0
     n = len(file_bytes)
     while True:
         sh = plan_shards(n, world, halo)[rank]
         d_buf = ops.upload(file_bytes[sh.start : sh.start + sh.buf_len])
-        own_nl = ops.count_newlines(d_buf, sh.own_len)
-        counts = _all_gather_ints(dist, [own_nl], world)
-        newlines_before = sum(c[0] for c in counts[:rank])
+        if not fasta:
+            own_nl = ops.count_newlines(d_buf, sh.own_len)
+            counts = _all_gather_ints(dist, [own_nl], world)
+            newlines_before = sum(c[0] for c in counts[:rank])
         halo_short, rec, picked, failed = 0, 0, 0, None
         scratch = ops.new_set()  # a retry must not leave ids of the failed attempt behind
         try:
-            if sh.own_len:
+            if sh.own_len and fasta:
+                rec, picked = ops.fasta_ids_shard(probe, d_buf, sh, scratch)
+            elif sh.own_len:
                 rec, picked = ops.ids_shard(probe, d_buf, sh, newlines_before, scratch)
         except Exception as e:  # SGPU_ERR_HALO == 21
             if getattr(e, "status", None) == 21:
@@ -267,12 +274,12 @@ def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo):
         return rec, picked
 
 
-def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 << 30) -> ShardedDiff:
+def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 << 30, fasta: bool = False) -> ShardedDiff:
     """ReadDifference::get_difference (utils.rs:250-285) across all ranks (SURVEY 8e, config 5).  For every
     (input, output) file pair: each rank lists the ids of its byte range of the OUTPUT file, the lists are
     all-gathered into the replicated set O_i, each rank probes its byte range of the INPUT file against it;
     counters are summed over ranks, the absent ids are united (the reference keeps one global diff set, so mates
-    with the same id appear once but count twice)."""
+    with the same id appear once but count twice).  fasta=True: the files are FASTA (the caller knows it from byte 0)."""
     world = dist.get_world_size() if dist is not None else 1
     reads_in = reads_out = difference = 0
     on_device = hasattr(ops, "unite_sets")  # the product: id lists never leave the GPUs until the final TSV
@@ -280,7 +287,7 @@ def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 <
     for fin, fout in pairs:
         out_local: list = []
         keep = out_local.append if on_device else (lambda s: out_local.extend(ops.set_ids(s)))
-        rec_out, _ = _ids_of_file_sharded(ops, fout, dist, None, keep, halo, max_halo)
+        rec_out, _ = _ids_of_file_sharded(ops, fout, dist, None, keep, halo, max_halo, fasta)
         if on_device:
             o_set = ops.unite_sets(out_local, dist)
         else:
@@ -290,7 +297,7 @@ def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 <
                 dist.all_gather_object(gathered, out_local)
             o_set = ops.set_from_ids(sorted(set(x for part in gathered for x in part)))
         keep = diff_local.append if on_device else (lambda s: diff_local.extend(ops.set_ids(s)))
-        rec_in, picked = _ids_of_file_sharded(ops, fin, dist, o_set, keep, halo, max_halo)
+        rec_in, picked = _ids_of_file_sharded(ops, fin, dist, o_set, keep, halo, max_halo, fasta)
         reads_out += rec_out
         reads_in += rec_in
         difference += picked
@@ -677,3 +684,92 @@ def clean_files_sharded_host(api, ctx, ids, jobs, dist=None, reverse: bool = Fal
         return _crlf_of_head(bytes(h_buf[: min(sh.buf_len, 1 << 16)].numpy()), lambda: bytes(h_buf[: sh.buf_len].numpy()))
 
     return _clean_files_sharded(call, count, crlf, [j[1] for j in jobs], dist, device, api.ScrubbyGpuError)
+
+
+def _clean_fasta_files_sharded(call, shards, dist, device, ShardFailure):
+    """the one-pass protocol of FASTA shards over several files.  `call(f, le_before)` runs file f's shard of this rank
+    and returns a result with n_written, n_other, reads_in, reads_out and le_own (api.FastaShardResult).
+
+    Every rank runs once, rank 0 with le_before = -1 and every other rank with 0 (LF); ONE all-gather carries status,
+    le_own, output sizes and counters.  Let d be the first le_own != -1 in rank order.  No d, or d == 0 (LF): every
+    shard is right.  d == 1 (CRLF) at rank q: the ranks before q wrote only records before the decision (LF, right);
+    rank q runs again with -1 (unless q == 0, which already did), every rank after q with 1."""
+    world = dist.get_world_size() if dist is not None else 1
+    rank = dist.get_rank() if dist is not None else 0
+    W = 7  # integers per file in the exchange
+    row, mine, failures = [], {}, {}
+    for f, sh in enumerate(shards):
+        st, r = 0, None
+        if sh.own_len:
+            try:
+                r = call(f, -1 if rank == 0 else 0)
+            except ShardFailure as e:
+                st, failures[f] = e.status, e
+        mine[f] = r
+        row += [st, r.le_own if r else -1, r.n_written if r else 0, r.n_other if r else 0, r.reads_in if r else 0,
+                r.reads_out if r else 0, int(r is not None)]
+    rows = _gather_rows(dist, row, world, device)
+    results = []
+    for f, sh in enumerate(shards):
+        col = [rw[f * W: (f + 1) * W] for rw in rows]
+        bad = [q for q, c in enumerate(col) if c[0]]
+        if bad:  # a parse error / halo / capacity problem in one shard ends the run on EVERY rank
+            q = bad[0]
+            if f in failures and q == rank:
+                e = failures[f]
+                if 3 <= e.status <= 9:  # a parse error (FASTQ_INVALID_START .. FASTQ_HEADER): the index in the whole file
+                    raise type(e)(e.status, e.index + sum(c[4] for c in col[:rank])) from e
+                raise e
+            raise ShardError(q, col[q][0])
+        d = next((q for q, c in enumerate(col) if c[6] and c[1] != -1), None)
+        crlf = d is not None and col[d][1] == 1
+        if not crlf:
+            results.append(DevShardResult(col[rank][2], col[rank][3], sum(c[2] for c in col[:rank]),
+                                          sum(c[3] for c in col[:rank]), sum(c[2] for c in col), sum(c[3] for c in col),
+                                          sum(c[4] for c in col), sum(c[5] for c in col), False, True, 3))
+            continue
+        # CRLF decided at rank d: rank d (unless it is rank 0) and every rank after it run again
+        st, r, exc = 0, mine[f], None
+        if col[rank][6] and rank >= d and rank > 0:
+            try:
+                r = call(f, -1 if rank == d else 1)
+            except ShardFailure as e:
+                st, r, exc = e.status, None, e
+        fin = _gather_rows(dist, [st, r.n_written if r else 0, r.n_other if r else 0, r.reads_in if r else 0,
+                                  r.reads_out if r else 0], world, device)
+        _raise_collectively(fin, 0, exc, rank)
+        results.append(DevShardResult(fin[rank][1], fin[rank][2], sum(c[1] for c in fin[:rank]),
+                                      sum(c[2] for c in fin[:rank]), sum(c[1] for c in fin), sum(c[2] for c in fin),
+                                      sum(c[3] for c in fin), sum(c[4] for c in fin), True,
+                                      not any(c[6] for c in col[max(d, 1):]), 3))
+    return results
+
+
+def clean_fasta_files_sharded_dev(api, ctx, ids, jobs, dist=None, reverse: bool = False):
+    """FastqCleaner::clean_reads over FASTA files (the caller knows the format from byte 0), each cut into one byte range
+    per rank: jobs = [(d_buf, Shard, d_out, d_other_or_None), ...], all DEVICE tensors.  The one-pass protocol of
+    _clean_fasta_files_sharded: one shard call and one all-gather per file, a second call on the ranks from the one
+    that decides CRLF on."""
+    import torch
+
+    def call(f, le_before):
+        d_buf, sh, d_out, d_oth = jobs[f]
+        return api.clean_fasta_shard_dev(ctx, ids, d_buf, sh.buf_len, sh.own_len, sh.is_first, sh.is_last, le_before,
+                                         d_out, d_oth, reverse)
+
+    return _clean_fasta_files_sharded(call, [j[1] for j in jobs], dist, torch.device("cuda", ctx.device),
+                                      api.ScrubbyGpuError)
+
+
+def clean_fasta_files_sharded_host(api, ctx, ids, jobs, dist=None, reverse: bool = False):
+    """the same on HOST buffers (pinned for full PCIe rate): jobs = [(h_buf, Shard, h_out, h_other_or_None)], torch CPU
+    uint8 tensors; every shard goes through sgpu_clean_fasta_shard (chunked H2D / kernels / D2H inside the call)"""
+    import torch
+
+    def call(f, le_before):
+        h_buf, sh, h_out, h_oth = jobs[f]
+        return api.clean_fasta_shard_host(ctx, ids, h_buf, sh.buf_len, sh.own_len, sh.is_first, sh.is_last, le_before,
+                                          h_out, h_oth, reverse)
+
+    return _clean_fasta_files_sharded(call, [j[1] for j in jobs], dist, torch.device("cuda", ctx.device),
+                                      api.ScrubbyGpuError)

@@ -673,7 +673,18 @@ size_t env_size(const char *name, size_t dflt) {
 
 }  // namespace
 
-bool clean_fastq_gz_stream(const std::string &input, const std::string &output, const ShardFn &shard, size_t chunk, size_t halo) {
+namespace {
+
+// one chunk of a stream through a format's shard entry point: (window, n, own_len, is_first, is_last, out, cap, &n_out,
+// &counts) -> status.  `next` is told about every chunk that produced its records and is not the last one: the state
+// the following chunk starts from (FASTQ: running newline count, line ending; FASTA: line-ending decision)
+using ChunkFn = std::function<int(const uint8_t *, size_t, size_t, int, int, uint8_t *, size_t, size_t *, sgpu_counts *)>;
+using NextFn = std::function<void(const uint8_t *own_bytes, size_t own, const sgpu_counts &)>;
+
+// the inflate thread -> chunked shard calls -> deflate / write behind them pipeline shared by the formats.  false: not
+// gzip, or the decoded input does not start with `lead` (or is shorter than `min_len`): nothing was done
+bool gz_stream(const std::string &input, const std::string &output, uint8_t lead, size_t min_len, size_t chunk, size_t halo,
+               const ChunkFn &run, const NextFn &next) {
     bool bgzf = false;
     {   // gzip only (by magic bytes, as niffler sniffs): plain members are inflated serially, BGZF members in parallel
         FILE *f = fopen(input.c_str(), "rb");
@@ -704,8 +715,8 @@ bool clean_fastq_gz_stream(const std::string &input, const std::string &output, 
         }
     };
     fill(chunk + halo);
-    // nothing inside, FASTA, or not a sequence file: the whole-file path reports those exactly as before
-    if (win.empty() || win[0] != '@') return false;
+    // nothing inside, another format, or not a sequence file: the whole-file path reports those exactly as before
+    if (win.empty() || win[0] != lead || (src_end && win.size() < min_len)) return false;
 
     OutSink sink(output, 6);  // niffler::compression::Level::Six
     std::vector<uint8_t> out[2];
@@ -713,8 +724,7 @@ bool clean_fastq_gz_stream(const std::string &input, const std::string &output, 
     auto settle = [&] {
         if (writing.valid()) writing.get();
     };
-    uint64_t nlb = 0, reads_before = 0;
-    int crlf = -1;
+    uint64_t reads_before = 0;
     bool first = true;
     for (unsigned turn = 0;; turn ^= 1) {
         fill(chunk + halo);
@@ -728,7 +738,7 @@ bool clean_fastq_gz_stream(const std::string &input, const std::string &output, 
         while (true) {
             if (o.size() < cap) o.resize(cap);
             memset(&counts, 0, sizeof(counts));
-            st = shard(win.data(), win.size(), own, nlb, first ? 1 : 0, last ? 1 : 0, crlf, o.data(), o.size(), &n_out, &counts);
+            st = run(win.data(), win.size(), own, first ? 1 : 0, last ? 1 : 0, o.data(), o.size(), &n_out, &counts);
             if (st != SGPU_ERR_CAPACITY || cap >= 2 * win.size() + 64) break;
             cap = 2 * win.size() + 64;
         }
@@ -748,16 +758,45 @@ bool clean_fastq_gz_stream(const std::string &input, const std::string &output, 
             if (parse_error) sink.close();
             check(st, reads_before + counts.error_record, "clean_reads");
         }
-        if (first) crlf = counts.crlf ? 1 : 0;
         first = false;
         if (last) break;
-        nlb += (uint64_t)std::count(win.begin(), win.begin() + (ptrdiff_t)own, (uint8_t)'\n');
+        next(win.data(), own, counts);
         reads_before += counts.reads_in;
         win.erase(win.begin(), win.begin() + (ptrdiff_t)own);
     }
     settle();
     sink.close();
     return true;
+}
+
+}  // namespace
+
+bool clean_fastq_gz_stream(const std::string &input, const std::string &output, const ShardFn &shard, size_t chunk, size_t halo) {
+    uint64_t nlb = 0;  // running newline count: the line phase of the next chunk
+    int crlf = -1;     // the first chunk decides the line ending
+    return gz_stream(
+        input, output, '@', 0, chunk, halo,
+        [&](const uint8_t *in, size_t n, size_t own, int is_first, int is_last, uint8_t *out, size_t cap, size_t *n_out,
+            sgpu_counts *counts) { return shard(in, n, own, nlb, is_first, is_last, crlf, out, cap, n_out, counts); },
+        [&](const uint8_t *own_bytes, size_t own, const sgpu_counts &counts) {
+            if (crlf < 0) crlf = counts.crlf ? 1 : 0;
+            nlb += (uint64_t)std::count(own_bytes, own_bytes + own, (uint8_t)'\n');
+        });
+}
+
+bool clean_fasta_gz_stream(const std::string &input, const std::string &output, const FastaShardFn &shard, size_t chunk,
+                           size_t halo) {
+    int le = -1, le_chunk = -1;  // the next chunk's le_before: this chunk's, once decided, else its own decision
+    return gz_stream(
+        input, output, '>', 5, chunk, halo,
+        [&](const uint8_t *in, size_t n, size_t own, int is_first, int is_last, uint8_t *out, size_t cap, size_t *n_out,
+            sgpu_counts *counts) {
+            le_chunk = -1;
+            return shard(in, n, own, is_first, is_last, le, out, cap, n_out, counts, &le_chunk);
+        },
+        [&](const uint8_t *, size_t, const sgpu_counts &) {
+            if (le < 0) le = le_chunk;
+        });
 }
 
 static bool file_exists(const std::string &p) {
@@ -1027,15 +1066,20 @@ ReadIdSet get_taxid_reads_metabuli(const GpuContext &g, const std::vector<std::s
 
 // ------------------------------------------------------------------------------------------ cleaner.rs
 void FastqCleaner::clean_reads(const GpuContext &g, const ReadIdSet &read_ids, bool reverse) const {
-    if (!getenv("SCRUBBY_NO_GZ_STREAM")) {  // plain gzip FASTQ: inflate, filter and deflate as one pipeline
+    if (!getenv("SCRUBBY_NO_GZ_STREAM")) {  // gzip / BGZF FASTQ or FASTA: inflate, filter and deflate as one pipeline
         ShardFn shard = [&](const uint8_t *in, size_t n_in, size_t own_len, uint64_t newlines_before, int is_first, int is_last,
                             int crlf, uint8_t *out, size_t cap, size_t *n_out, sgpu_counts *counts) {
             return (int)sgpu_clean_fastq_shard(g.get(), read_ids.get(), in, n_in, own_len, newlines_before, is_first, is_last, crlf,
                                                reverse ? 1 : 0, out, cap, n_out, nullptr, 0, nullptr, counts);
         };
-        if (clean_fastq_gz_stream(input, output, shard, env_size("SCRUBBY_STREAM_CHUNK", (size_t)64 << 20),
-                                  env_size("SCRUBBY_STREAM_HALO", (size_t)8 << 20)))
-            return;
+        const size_t chunk = env_size("SCRUBBY_STREAM_CHUNK", (size_t)64 << 20), halo = env_size("SCRUBBY_STREAM_HALO", (size_t)8 << 20);
+        if (clean_fastq_gz_stream(input, output, shard, chunk, halo)) return;
+        FastaShardFn fasta = [&](const uint8_t *in, size_t n_in, size_t own_len, int is_first, int is_last, int le_before,
+                                 uint8_t *out, size_t cap, size_t *n_out, sgpu_counts *counts, int *le_own) {
+            return (int)sgpu_clean_fasta_shard(g.get(), read_ids.get(), in, n_in, own_len, is_first, is_last, le_before,
+                                               reverse ? 1 : 0, out, cap, n_out, nullptr, 0, nullptr, counts, le_own);
+        };
+        if (clean_fasta_gz_stream(input, output, fasta, chunk, halo)) return;
     }
     bool empty = false;
     std::vector<uint8_t> in = read_file(input, &empty);
@@ -1666,6 +1710,23 @@ int scrubby_host_stream_clean(const char *input, const char *output, size_t chun
     try {
         scrubby::ShardFn fn = cb;
         *handled = scrubby::clean_fastq_gz_stream(input, output, fn, chunk, halo) ? 1 : 0;
+        return 0;
+    } catch (const scrubby::ScrubbyError &e) {
+        if (err_index) *err_index = e.index;
+        return 100 + (int)e.kind;
+    }
+}
+
+// the same for FASTA (clean_fasta_gz_stream) with a sgpu_clean_fasta_shard-shaped callback.  *handled = 0: the input is
+// not a gzip FASTA
+typedef int (*scrubby_fasta_shard_cb)(const uint8_t *in, size_t n_in, size_t own_len, int is_first, int is_last,
+                                      int le_before, uint8_t *out, size_t cap, size_t *n_out, sgpu_counts *counts,
+                                      int *le_own);
+int scrubby_host_stream_clean_fasta(const char *input, const char *output, size_t chunk, size_t halo,
+                                    scrubby_fasta_shard_cb cb, int *handled, uint64_t *err_index) {
+    try {
+        scrubby::FastaShardFn fn = cb;
+        *handled = scrubby::clean_fasta_gz_stream(input, output, fn, chunk, halo) ? 1 : 0;
         return 0;
     } catch (const scrubby::ScrubbyError &e) {
         if (err_index) *err_index = e.index;

@@ -159,6 +159,13 @@ class OutSink {
 using ShardFn = std::function<int(const uint8_t *in, size_t n_in, size_t own_len, uint64_t newlines_before, int is_first,
                                   int is_last, int crlf, uint8_t *out, size_t cap, size_t *n_out, sgpu_counts *counts)>;
 bool clean_fastq_gz_stream(const std::string &input, const std::string &output, const ShardFn &shard, size_t chunk, size_t halo);
+// the same pipeline for a gzip / BGZF FASTA: `shard` has sgpu_clean_fasta_shard's contract (same omissions); chunk k+1
+// starts from chunk k's line-ending state.  false: not a gzip FASTA (or fewer than 5 decoded bytes), nothing was done.
+using FastaShardFn = std::function<int(const uint8_t *in, size_t n_in, size_t own_len, int is_first, int is_last,
+                                       int le_before, uint8_t *out, size_t cap, size_t *n_out, sgpu_counts *counts,
+                                       int *le_own)>;
+bool clean_fasta_gz_stream(const std::string &input, const std::string &output, const FastaShardFn &shard, size_t chunk,
+                           size_t halo);
 
 // ---------------------------------------------------------------- alignment.rs
 struct ReadAlignment {

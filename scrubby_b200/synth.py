@@ -104,6 +104,39 @@ def gen_fastq(n: int, mate: int = 1, seed: int = SEED, device="cpu", start: int 
     return out[:total]
 
 
+def gen_fasta(n: int, mate: int = 1, wrap: int | None = None, crlf: bool = False, seed: int = SEED, device="cpu",
+              start: int = 0, read_len: int = 150) -> torch.Tensor:
+    """the gen_fastq records as FASTA (same ids and sequences, so the id lists and PAF generators apply):
+    '>' header E sequence E, the sequence in lines of `wrap` bases (None: one line), E = CRLF when `crlf`.
+    read_len=30_000 gives ONT-like long records (shard halo tests)."""
+    fq = gen_fastq(n, mate, seed, device, start, read_len=read_len)
+    e = _bytes("\r\n" if crlf else "\n", device)
+    E = e.numel()
+    w = read_len if not wrap else wrap
+    n_lines = -(-read_len // w)
+    parts, pos, lo = [], 0, start
+    while lo < start + n:
+        d = _digits(lo)
+        hi = min(start + n, 10 ** d)
+        m, L = hi - lo, 23 + 2 * read_len + d
+        rows = fq[pos: pos + m * L].view(m, L)
+        pos += m * L
+        H = 17 + d  # header without '@' and '\n'
+        out = torch.empty((m, 1 + H + E + read_len + n_lines * E), dtype=torch.uint8, device=device)
+        out[:, 0] = 62  # '>'
+        out[:, 1: 1 + H] = rows[:, 1: 1 + H]
+        out[:, 1 + H: 1 + H + E] = e
+        o, s0 = 1 + H + E, 19 + d
+        for k in range(n_lines):
+            a, b = k * w, min(read_len, (k + 1) * w)
+            out[:, o: o + b - a] = rows[:, s0 + a: s0 + b]
+            out[:, o + b - a: o + b - a + E] = e
+            o += b - a + E
+        parts.append(out.view(-1))
+        lo = hi
+    return torch.cat(parts) if parts else torch.empty(0, dtype=torch.uint8, device=device)
+
+
 def _num_field(v: torch.Tensor, width: int):
     """left-aligned decimal rendering of non-negative int64 values: (chars [n,width], mask [n,width])"""
     dev = v.device
