@@ -1,177 +1,65 @@
-// capi.cu -- extern "C" entry points of libscrubby_gpu.so (see include/scrubby_gpu.h).
+// capi.cu -- extern "C" entry points of libscrubby_gpu.so (see include/scrubby_gpu.h): argument checks, the format
+// decision, the chunked and one-shot host-buffer paths.  The work itself is done by the shard cores declared in
+// fastq_records.cuh; a whole file is the shard (n, n, first = 1, last = 1) of either format.
 #include <vector>
 
 #include "fastq_records.cuh"
 
 namespace sgpu {
 const char *last_cuda_error_text();
-// fastq_fused.cu: single-pass kernel; returns SGPU_OK with *used = 0 when the input is not canonical
-sgpu_status clean_fused(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse,
-                        uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                        sgpu_counts *counts, int *used);
-sgpu_status ids_fused(sgpu_ctx *c, const sgpu_idset *probe, const uint8_t *d_in, size_t n_in, size_t own_len,
-                      uint64_t newlines_before, int is_first, int is_last, uint64_t *span_off, uint32_t *span_len,
-                      uint64_t cap, uint64_t *n_spans, uint64_t *span_base, uint64_t *n_records, int *used,
-                      sgpu_counts *spec_out);
-sgpu_status clean_fused_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                              uint64_t newlines_before, int is_first, int is_last, int reverse, uint8_t *d_out_w,
-                              size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                              sgpu_counts *counts, int *used, bool want_nl);
 
-// ids of every record of a FASTQ buffer (diff): span + validity
-__global__ void __launch_bounds__(128)
-    fastq_ids_kernel(RecParams P, IdSetView probe, int want_absent, uint64_t *key_off, uint32_t *key_len, uint8_t *sel,
-                     unsigned long long *err_word, unsigned long long *counters) {
-    uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    bool rec = false, pick = false;
-    if (k <= P.k_full) {
-        RecMeta m = {0, 0, 0, 0};
-        uint64_t start, p1, p3;
-        size_t id_off = 0, id_len = 0;
-        uint64_t off = 0;
-        uint32_t len = 0;
-        if (locate_record(P, k, &start, &p1, &p3, &m, &id_off, &id_len, err_word)) {
-            rec = true;
-            off = start + 1 + id_off;
-            len = (uint32_t)id_len;
-            if (want_absent)
-                pick = !(id_len <= IDSET_MAX_KEY && idset_contains(probe, P.in + off, len));
-            else
-                pick = true;
-        }
-        key_off[k] = off;
-        key_len[k] = len;
-        sel[k] = pick ? 1 : 0;
-    }
-    unsigned br = __ballot_sync(0xffffffffu, rec), bp = __ballot_sync(0xffffffffu, pick);
-    if ((threadIdx.x & 31) == 0) {
-        if (br) atomicAdd(&counters[0], (unsigned long long)__popc(br));
-        if (bp) atomicAdd(&counters[1], (unsigned long long)__popc(bp));
-    }
-}
+enum class Fmt { fastq, fasta, empty, unknown };
 
-// needletail picks the parser from the first byte; niffler needs 5 bytes (utils.rs:359-383)
-static sgpu_status sniff(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, bool *empty) {
-    *empty = n_in < 5;
-    if (*empty) return SGPU_OK;
-    SGPU_CUDA(cudaMemcpyAsync(c->h_pinned, d_in, 1, cudaMemcpyDeviceToHost, c->stream));
-    SGPU_CUDA(cudaStreamSynchronize(c->stream));
-    uint8_t b = *(uint8_t *)c->h_pinned;
-    if (b == '>') return SGPU_ERR_FASTA_UNSUPPORTED;
-    if (b != '@') return SGPU_ERR_FASTQ_UNKNOWN_FORMAT;
+// needletail picks the parser from the first byte; niffler needs 5 bytes (utils.rs:359-383).  `whole`: the 5-byte rule
+// applies to the buffer (a file, or a shard the caller treats as one).  Byte 0 is read only when the decision needs
+// it; a device buffer's comes back with a one-byte copy (the stream is synchronised).
+static sgpu_status input_format(sgpu_ctx *c, const uint8_t *buf, bool on_device, size_t n, bool whole, Fmt *f) {
+    *f = Fmt::empty;
+    if (n == 0 || (whole && n < 5)) return SGPU_OK;
+    const uint8_t *b0 = buf;
+    if (on_device) {
+        SGPU_CUDA(cudaMemcpyAsync(c->h_pinned, buf, 1, cudaMemcpyDeviceToHost, c->stream));
+        SGPU_CUDA(cudaStreamSynchronize(c->stream));
+        b0 = (const uint8_t *)c->h_pinned;
+    }
+    const uint8_t b = *b0;
+    *f = b == '>' ? Fmt::fasta : b == '@' ? Fmt::fastq : Fmt::unknown;
     return SGPU_OK;
 }
 
-// one FASTQ buffer (or one shard of it: the records that start in [0, own_len], see sgpu_clean_fastq_shard_dev)
-// -> ids (all, or only those absent from `probe`) inserted into `into`
-static sgpu_status fastq_ids_into(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t own_len, uint64_t newlines_before,
-                                  int is_first, int is_last, const sgpu_idset *probe, int want_absent, sgpu_idset *into,
-                                  uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record,
-                                  sgpu_counts *spec_out = nullptr) {
+// a whole file whose format is known: '>' hands it to needletail's FASTA reader, FASTQ is the shard (n, n, 0, 1, 1,
+// crlf -1)
+static sgpu_status clean_file(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, Fmt f, int reverse, const Outs &out,
+                              sgpu_counts *counts) {
+    clear_outputs(out, counts);
+    switch (f) {
+    case Fmt::fasta: {
+        int le_own;
+        return clean_fasta_shard(c, set, s, -1, reverse, out, counts, &le_own);
+    }
+    case Fmt::empty: counts->empty_input = 1; return SGPU_OK;
+    case Fmt::unknown: return SGPU_ERR_FASTQ_UNKNOWN_FORMAT;
+    default: return clean_fastq_shard(c, set, s, 0, -1, reverse, out, counts, false);
+    }
+}
+
+// the ids of a FASTQ shard, or of a whole FASTA file (sgpu_diff_dev, sgpu_fastq_ids_shard_dev); a first shard that
+// starts with '>' but is not the whole file is refused with SGPU_ERR_FASTA_UNSUPPORTED
+static sgpu_status ids_locked(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
+                              int want_absent, sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked,
+                              uint64_t *err_record, sgpu_counts *spec_out = nullptr) {
     *n_records = *n_picked = 0;
-    const bool spec = !is_first && newlines_before == SGPU_NEWLINES_UNKNOWN;
-    if (is_first) {
-        bool empty;
-        const sgpu_status src = sniff(c, d_buf, n, &empty);
-        if (src == SGPU_ERR_FASTA_UNSUPPORTED && is_last && own_len == n)  // a whole FASTA file
-            return fasta_ids_shard(c, d_buf, n, n, 1, 1, probe, want_absent, into, n_records, n_picked, err_record);
-        if (src != SGPU_OK) return src;
-        if (empty) return SGPU_OK;
-    } else if (n == 0 || own_len == 0) {
-        return SGPU_OK;
+    if (s.is_first) {
+        Fmt f;
+        SGPU_TRY(input_format(c, s.p, true, s.n, true, &f));
+        if (f == Fmt::empty) return SGPU_OK;
+        if (f == Fmt::unknown) return SGPU_ERR_FASTQ_UNKNOWN_FORMAT;
+        if (f == Fmt::fasta)
+            return s.is_last && s.own_len == s.n
+                       ? fasta_ids_shard(c, s, probe, want_absent, into, n_records, n_picked, err_record)
+                       : SGPU_ERR_FASTA_UNSUPPORTED;
     }
-    cudaStream_t st = c->stream;
-    if (c->mode == 0 && ((uintptr_t)d_buf & 15) == 0) {
-        // canonical input: one pass of the fused kernel in ids mode -> (offset, length) spans of the wanted ids
-        DevBuf<uint64_t> s_off;
-        DevBuf<uint32_t> s_len;
-        const uint64_t cap = n / 100 + 4096;  // the fused kernel handles >= ~102 bytes per record
-        SGPU_TRY(s_off.alloc(cap, st));
-        SGPU_TRY(s_len.alloc(cap, st));
-        uint64_t n_spans = 0, n_rec = 0, base = 0;
-        int used = 0;
-        SGPU_TRY(ids_fused(c, want_absent ? probe : nullptr, d_buf, n, own_len, newlines_before, is_first, is_last,
-                           s_off.p, s_len.p, cap, &n_spans, &base, &n_rec, &used, spec_out));
-        if (used) {
-            *n_records = n_rec;
-            *n_picked = n_spans;
-            if (into && n_spans)
-                SGPU_TRY(idset_insert_spans(c, into, d_buf + base, s_off.p, s_len.p, nullptr, (size_t)n_spans));
-            return SGPU_OK;
-        }
-    }
-    if (spec) return SGPU_ERR_PHASE_UNKNOWN;
-    DevBuf<uint64_t> nlpos, key_off, scratch;
-    DevBuf<uint32_t> key_len;
-    DevBuf<uint8_t> sel;
-    uint64_t n_nl;
-    SGPU_TRY(index_newlines(c, d_buf, n, nlpos, &n_nl));
-    RecParams P;
-    P.in = d_buf;
-    P.n_in = n;
-    P.own_len = own_len;
-    P.nlpos = nlpos.p;
-    P.is_last = is_last;
-    P.reverse = 0;
-    P.crlf = 0;
-    P.set = view_of(nullptr);
-    if (!setup_records(P, n_nl, newlines_before, is_first)) {
-        // no record boundary in the whole buffer: a record longer than the halo (or a truncated file)
-        return is_last ? SGPU_ERR_FASTQ_UNEXPECTED_END : SGPU_ERR_HALO;
-    }
-    uint64_t n_thr = P.k_full + 1;
-    SGPU_TRY(key_off.alloc(n_thr, st));
-    SGPU_TRY(key_len.alloc(n_thr, st));
-    SGPU_TRY(sel.alloc(n_thr, st));
-    SGPU_TRY(scratch.alloc(4, st));
-    uint64_t init[4] = {~0ull, 0, 0, 0};
-    memcpy(c->h_pinned + 32, init, sizeof(init));
-    SGPU_CUDA(cudaMemcpyAsync(scratch.p, c->h_pinned + 32, sizeof(init), cudaMemcpyHostToDevice, st));
-    fastq_ids_kernel<<<(unsigned)ceil_div(n_thr, 128), 128, 0, st>>>(P, view_of(probe), want_absent, key_off.p,
-                                                                      key_len.p, sel.p, (unsigned long long *)scratch.p,
-                                                                      (unsigned long long *)(scratch.p + 1));
-    SGPU_LAUNCH(c);
-    uint64_t h[3];
-    SGPU_TRY(read_u64s(c, scratch.p, h, 3));
-    if (h[0] != ~0ull) {
-        if (err_record) *err_record = h[0] >> 8;
-        return (sgpu_status)(h[0] & 0xFF);
-    }
-    *n_records = h[1];
-    *n_picked = h[2];
-    if (into) SGPU_TRY(idset_insert_spans(c, into, d_buf, key_off.p, key_len.p, sel.p, n_thr));
-    return SGPU_OK;
-}
-
-static sgpu_status clean_dev_locked(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse,
-                                    uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o,
-                                    size_t *n_o, sgpu_counts *counts) {
-    memset(counts, 0, sizeof(*counts));
-    *n_w = 0;
-    if (n_o) *n_o = 0;
-    if (n_in && ((uintptr_t)d_in & 15)) return SGPU_ERR_INVALID_ARG;
-    bool empty;
-    {
-        const sgpu_status src = sniff(c, d_in, n_in, &empty);
-        if (src == SGPU_ERR_FASTA_UNSUPPORTED) {  // '>': needletail's FASTA reader takes over
-            int le_own;
-            return clean_fasta_shard(c, set, d_in, n_in, n_in, 1, 1, -1, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o,
-                                     counts, &le_own);
-        }
-        if (src != SGPU_OK) return src;
-    }
-    if (empty) {
-        counts->empty_input = 1;
-        return SGPU_OK;
-    }
-    if (c->mode == 0) {
-        int used = 0;
-        SGPU_TRY(clean_fused(c, set, d_in, n_in, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o, counts, &used));
-        if (used) return SGPU_OK;
-        memset(counts, 0, sizeof(*counts));
-    }
-    return clean_general(c, set, d_in, n_in, n_in, 0, 1, 1, -1, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o,
-                         counts);
+    return fastq_ids_shard(c, s, newlines_before, probe, want_absent, into, n_records, n_picked, err_record, spec_out);
 }
 
 void ctx_release(sgpu_ctx *c) {
@@ -337,59 +225,39 @@ sgpu_status sgpu_count_newlines_dev(sgpu_ctx *c, const uint8_t *d_buf, size_t n,
     return count_newlines(c, d_buf, n, count);
 }
 
+// argument checks shared by the FASTQ shard entry points
+static bool fastq_shard_args_ok(size_t n_in, size_t own_len, uint64_t newlines_before, int is_first, int is_last,
+                                int crlf) {
+    return own_len <= n_in && (!is_last || own_len == n_in) && (!is_first || newlines_before == 0) && crlf >= -1 &&
+           crlf <= 1 && (is_first || crlf >= 0 || newlines_before == SGPU_NEWLINES_UNKNOWN);
+}
+
 sgpu_status sgpu_clean_fastq_dev(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse,
                                  uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o,
                                  size_t *n_o, sgpu_counts *counts) {
     if (!c || !set || !n_w || !counts || (n_in && !d_in) || (cap_w && !d_out_w)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    return clean_dev_locked(c, set, d_in, n_in, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o, counts);
+    const Outs out{d_out_w, cap_w, n_w, d_out_o, cap_o, n_o};
+    clear_outputs(out, counts);
+    if (n_in && ((uintptr_t)d_in & 15)) return SGPU_ERR_INVALID_ARG;
+    Fmt f;
+    SGPU_TRY(input_format(c, d_in, true, n_in, true, &f));
+    return clean_file(c, set, Shard{d_in, n_in, n_in, 1, 1}, f, reverse, out, counts);
 }
-
-static sgpu_status clean_shard_locked(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
-                                      size_t own_len, uint64_t newlines_before, int is_first, int is_last, int crlf,
-                                      int reverse, uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o,
-                                      size_t cap_o, size_t *n_o, sgpu_counts *counts, bool want_nl);
 
 sgpu_status sgpu_clean_fastq_shard_dev(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
                                        size_t own_len, uint64_t newlines_before, int is_first, int is_last, int crlf,
                                        int reverse, uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o,
                                        size_t cap_o, size_t *n_o, sgpu_counts *counts) {
-    if (!c || !set || !n_w || !counts || (n_in && !d_in) || own_len > n_in || (is_last && own_len != n_in) ||
-        (is_first && newlines_before != 0) || crlf < -1 || crlf > 1 || (!is_first && crlf < 0 && newlines_before != SGPU_NEWLINES_UNKNOWN))
+    if (!c || !set || !n_w || !counts || (n_in && !d_in) ||
+        !fastq_shard_args_ok(n_in, own_len, newlines_before, is_first, is_last, crlf))
         return SGPU_ERR_INVALID_ARG;
     if (n_in && ((uintptr_t)d_in & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    return clean_shard_locked(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, crlf, reverse, d_out_w,
-                              cap_w, n_w, d_out_o, cap_o, n_o, counts, crlf < 0);
-}
-
-// shard body shared by sgpu_clean_fastq_shard_dev and the pipelined host path (context locked, device set).
-// want_nl: when the single-pass kernel produces the result, counts->own_newlines is filled from its per-tile counts
-static sgpu_status clean_shard_locked(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
-                                      size_t own_len, uint64_t newlines_before, int is_first, int is_last, int crlf,
-                                      int reverse, uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o,
-                                      size_t cap_o, size_t *n_o, sgpu_counts *counts, bool want_nl) {
-    memset(counts, 0, sizeof(*counts));
-    *n_w = 0;
-    if (n_o) *n_o = 0;
-    // crlf == -1: not exchanged yet.  The single-pass kernel only takes LF input, so whatever it produces is right for a
-    // file whose first record is LF (the caller checks shard 0's counts->crlf); the first shard decides it itself.
-    const bool spec = !is_first && (newlines_before == SGPU_NEWLINES_UNKNOWN || crlf < 0);
-    if (spec && newlines_before != SGPU_NEWLINES_UNKNOWN) return SGPU_ERR_INVALID_ARG;
-    if (c->mode == 0 && crlf <= 0 && n_in >= 5) {
-        int used = 0;
-        SGPU_TRY(clean_fused_shard(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, reverse, d_out_w,
-                                   cap_w, n_w, d_out_o, cap_o, n_o, counts, &used, want_nl));
-        if (used) return SGPU_OK;
-        memset(counts, 0, sizeof(*counts));
-        *n_w = 0;
-        if (n_o) *n_o = 0;
-    }
-    if (spec) return SGPU_ERR_PHASE_UNKNOWN;  // the exact protocol (newline counts exchanged first) takes over
-    return clean_general(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, is_first && crlf < 0 ? -1 : (crlf ? 1 : 0),
-                         reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o, counts);
+    return clean_fastq_shard(c, set, Shard{d_in, n_in, own_len, is_first, is_last}, newlines_before, crlf, reverse,
+                             Outs{d_out_w, cap_w, n_w, d_out_o, cap_o, n_o}, counts, crlf < 0);
 }
 
 }  // extern "C"
@@ -403,11 +271,12 @@ static sgpu_status clean_shard_locked(sgpu_ctx *c, const sgpu_idset *set, const 
 // (FastqChunks: the running newline count; FastaChunks: the line-ending decision).
 // The buffer is a shard: own bytes [0, own_len) + halo; a whole file is the shard (n_in, n_in, first, last).
 // *done = 0: not applicable here (small input, halo too small for a record ...), take the one-shot path.
-template <class Fmt>
-static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, size_t own_len, int is_last, uint8_t *out_w,
-                                 size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o,
-                                 sgpu_counts *counts, int *done, Fmt &fmt) {
+template <class Chunks>
+static sgpu_status pipeline_host(sgpu_ctx *c, const Shard &s, const Outs &out, sgpu_counts *counts, int *done,
+                                 Chunks &fmt) {
     *done = 0;
+    const size_t n_in = s.n, own_len = s.own_len;
+    uint8_t *out_o = out.o;
     // (environment knobs so that tests can drive the chunk logic with small inputs)
     const size_t CHUNK = getenv("SGPU_PIPE_CHUNK") ? (size_t)atoll(getenv("SGPU_PIPE_CHUNK")) & ~(size_t)15
                                                    : (size_t)128 << 20;
@@ -421,7 +290,7 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
     const size_t K = ceil_div(own_len, CHUNK);  // kernel chunks: the owned range
     const size_t U = ceil_div(n_in, CHUNK);     // upload pieces: the whole buffer (own range + halo)
     const size_t tail_halo = n_in - own_len;
-    const size_t obuf = Fmt::OUT_FACTOR * (CHUNK + std::max(HALO, tail_halo)) + 64;
+    const size_t obuf = Chunks::OUT_FACTOR * (CHUNK + std::max(HALO, tail_halo)) + 64;
     // context-owned staging (the context is locked): 0 the file, 1-2 kept chunks, 3-4 removed chunks
     auto staging = [&](int i, size_t bytes, uint8_t **p) -> sgpu_status {
         if (c->pipe_cap[i] < bytes) {
@@ -458,7 +327,7 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
     }
     auto upload = [&](size_t k) -> cudaError_t {
         const size_t a = k * CHUNK, len = std::min(CHUNK, n_in - a);
-        cudaError_t e = cudaMemcpyAsync(d_in.p + a, in + a, len, cudaMemcpyHostToDevice, c->s_in);
+        cudaError_t e = cudaMemcpyAsync(d_in.p + a, s.p + a, len, cudaMemcpyHostToDevice, c->s_in);
         if (e != cudaSuccess) return e;
         return cudaEventRecord(ev_in[k], c->s_in);
     };
@@ -476,7 +345,7 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
         const size_t a = k * CHUNK;
         size_t own = std::min(CHUNK, own_len - a);
         bool last_chunk = k + 1 == K;
-        if (!last_chunk && is_last && a + own + HALO >= n_in) {
+        if (!last_chunk && s.is_last && a + own + HALO >= n_in) {
             // the chunk's buffer reaches EOF: it owns the rest, as only the last chunk may apply the end-of-file rules
             // (a record that runs to EOF would otherwise be a halo problem and send the whole call to the one-shot path)
             own = own_len - a;
@@ -491,8 +360,8 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
         if (k >= 2) cudaStreamWaitEvent(st, ev_out[r], 0);
         size_t nw = 0, no = 0;
         sgpu_counts ck;
-        rc = fmt.run(c, k, a, d_in.p + a, buf_len, own, last_chunk && is_last, d_w[r].p, out_o ? d_o[r].p : nullptr, obuf,
-                     &nw, &no, &ck);
+        rc = fmt.run(c, k, a, Shard{d_in.p + a, buf_len, own, s.is_first && k == 0, last_chunk && s.is_last},
+                     Outs{d_w[r].p, obuf, &nw, out_o ? d_o[r].p : nullptr, obuf, &no}, &ck);
         if (fmt.unknown(rc, ck)) {
             rc = SGPU_OK;  // speculation not applicable: the caller comes back with the exact phase
             unknown = true;
@@ -507,13 +376,13 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
         const sgpu_status parse_rc = rc;  // a parse error: like the one-shot path (and the reference, which
         rc = SGPU_OK;                     // leaves the records before the error on disk) the output so far stays
         if (parse_rc != SGPU_OK) total.error_record = ck.error_record + total.reads_in;  // earlier chunks come first
-        if (off_w + nw > cap_w || (out_o && off_o + no > cap_o)) {
+        if (off_w + nw > out.cap_w || (out_o && off_o + no > out.cap_o)) {
             rc = SGPU_ERR_CAPACITY;
             break;
         }
         cudaEventRecord(ev_k[r], st);
         cudaStreamWaitEvent(c->s_out, ev_k[r], 0);
-        if (nw) ce = cudaMemcpyAsync(out_w + off_w, d_w[r].p, nw, cudaMemcpyDeviceToHost, c->s_out);
+        if (nw) ce = cudaMemcpyAsync(out.w + off_w, d_w[r].p, nw, cudaMemcpyDeviceToHost, c->s_out);
         if (out_o && no && ce == cudaSuccess)
             ce = cudaMemcpyAsync(out_o + off_o, d_o[r].p, no, cudaMemcpyDeviceToHost, c->s_out);
         cudaEventRecord(ev_out[r], c->s_out);
@@ -544,17 +413,15 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
     }
     if (unknown) {
         *done = 1;
-        memset(counts, 0, sizeof(*counts));
-        *n_w = 0;
-        if (n_o) *n_o = 0;
+        clear_outputs(out, counts);
         return SGPU_ERR_PHASE_UNKNOWN;
     }
     if (bail) return SGPU_OK;  // *done stays 0
     *done = 1;
     *counts = total;
     fmt.finish(counts);
-    *n_w = off_w;
-    if (n_o) *n_o = out_o ? off_o : 0;
+    *out.n_w = off_w;
+    if (out.n_o) *out.n_o = out_o ? off_o : 0;
     return rc;
 }
 
@@ -564,21 +431,19 @@ static sgpu_status pipeline_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, si
 struct FastqChunks {
     static constexpr size_t OUT_FACTOR = 1;
     const sgpu_idset *set;
-    int is_first, crlf_in, reverse;
+    int crlf_in, reverse;
     bool spec;
     int crlf;
     uint64_t nb;  // running count: exact, or relative to the speculated phase
     uint64_t own_nl_total = 0, lead_nl = 0;
 
-    sgpu_status run(sgpu_ctx *c, size_t k, size_t a, const uint8_t *d, size_t buf_len, size_t own, bool last, uint8_t *dw,
-                    uint8_t *dov, size_t obuf, size_t *nw, size_t *no, sgpu_counts *ck) {
+    sgpu_status run(sgpu_ctx *c, size_t k, size_t a, const Shard &d, const Outs &o, sgpu_counts *ck) {
         const bool spec0 = spec && k == 0;
-        const sgpu_status rc = clean_shard_locked(c, set, d, buf_len, own, spec0 ? SGPU_NEWLINES_UNKNOWN : nb,
-                                                  is_first && k == 0, last, spec0 ? -1 : crlf, reverse, dw, obuf, nw, dov,
-                                                  obuf, no, ck, true);
+        const sgpu_status rc = clean_fastq_shard(c, set, d, spec0 ? SGPU_NEWLINES_UNKNOWN : nb, spec0 ? -1 : crlf, reverse,
+                                                 o, ck, true);
         if (getenv("SGPU_DEBUG"))
             fprintf(stderr, "[sgpu] pipe chunk %zu a=%zu own=%zu buf=%zu nlb=%llu -> rc=%d nw=%zu no=%zu in=%llu out=%llu path=%u own_nl=%llu lead_nl=%llu\n",
-                    k, a, own, buf_len, (unsigned long long)nb, (int)rc, *nw, *no,
+                    k, a, d.own_len, d.n, (unsigned long long)nb, (int)rc, *o.n_w, *o.n_o,
                     (unsigned long long)ck->reads_in, (unsigned long long)ck->reads_out, ck->path,
                     (unsigned long long)ck->own_newlines, (unsigned long long)ck->lead_newlines);
         return rc;
@@ -606,21 +471,23 @@ struct FastqChunks {
     }
 };
 
-static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
-                                        uint64_t newlines_before, int is_first, int is_last, int crlf_in, int reverse,
-                                        uint8_t *out_w, size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o,
-                                        size_t *n_o, sgpu_counts *counts, int *done) {
+static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint64_t newlines_before,
+                                        int crlf_in, int reverse, const Outs &out, sgpu_counts *counts, int *done) {
     *done = 0;
     if (c->mode != 0) return SGPU_OK;
-    if (is_first && n_in && in[0] != '@') return SGPU_OK;  // FASTA / unknown format: not this format's pipeline
-    const bool spec = !is_first && newlines_before == SGPU_NEWLINES_UNKNOWN;
-    int crlf = crlf_in > 0;
-    if (is_first) {  // needletail decides the line ending on the first record's first line
-        const uint8_t *nl = (const uint8_t *)memchr(in, '\n', n_in);
-        crlf = nl && nl > in && nl[-1] == '\r';
+    if (s.is_first) {
+        Fmt f;
+        SGPU_TRY(input_format(c, s.p, false, s.n, true, &f));
+        if (f != Fmt::fastq) return SGPU_OK;  // FASTA / unknown format / too small: not this format's pipeline
     }
-    FastqChunks f{set, is_first, crlf_in, reverse, spec, crlf, spec ? 0 : newlines_before};
-    return pipeline_host(c, in, n_in, own_len, is_last, out_w, cap_w, n_w, out_o, cap_o, n_o, counts, done, f);
+    const bool spec = !s.is_first && newlines_before == SGPU_NEWLINES_UNKNOWN;
+    int crlf = crlf_in > 0;
+    if (s.is_first) {  // needletail decides the line ending on the first record's first line
+        const uint8_t *nl = (const uint8_t *)memchr(s.p, '\n', s.n);
+        crlf = nl && nl > s.p && nl[-1] == '\r';
+    }
+    FastqChunks f{set, crlf_in, reverse, spec, crlf, spec ? 0 : newlines_before};
+    return pipeline_host(c, s, out, counts, done, f);
 }
 
 // FASTA: chunk k+1 starts from chunk k's line-ending state, le_before(k) when that was decided, else le_own(k) -- exact,
@@ -628,17 +495,13 @@ static sgpu_status clean_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, cons
 struct FastaChunks {
     static constexpr size_t OUT_FACTOR = 2;
     const sgpu_idset *set;
-    int is_first, reverse;
+    int reverse;
     int le;            // le_before of the next chunk
     int le_own = -1;   // the shard's own decision: the first chunk's that has one
     int le_chunk = -1;
 
-    sgpu_status run(sgpu_ctx *c, size_t k, size_t, const uint8_t *d, size_t buf_len, size_t own, bool last, uint8_t *dw,
-                    uint8_t *dov, size_t obuf, size_t *nw, size_t *no, sgpu_counts *ck) {
-        memset(ck, 0, sizeof(*ck));
-        *nw = *no = 0;
-        const sgpu_status rc = clean_fasta_shard(c, set, d, buf_len, own, is_first && k == 0, last, le, reverse, dw, obuf, nw,
-                                                 dov, obuf, no, ck, &le_chunk);
+    sgpu_status run(sgpu_ctx *c, size_t, size_t, const Shard &d, const Outs &o, sgpu_counts *ck) {
+        const sgpu_status rc = clean_fasta_shard(c, set, d, le, reverse, o, ck, &le_chunk);
         if (le_own < 0) le_own = le_chunk;  // (also from a chunk that stops on a parse error: decided before the error)
         return rc;
     }
@@ -650,40 +513,38 @@ struct FastaChunks {
     void finish(sgpu_counts *) const {}
 };
 
-static sgpu_status fasta_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
-                                        int is_first, int is_last, int le_before, int reverse, uint8_t *out_w, size_t cap_w,
-                                        size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
-                                        int *le_own, int *done) {
-    FastaChunks f{set, is_first, reverse, le_before};
-    const sgpu_status rc =
-        pipeline_host(c, in, n_in, own_len, is_last, out_w, cap_w, n_w, out_o, cap_o, n_o, counts, done, f);
+static sgpu_status fasta_host_pipelined(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, int le_before, int reverse,
+                                        const Outs &out, sgpu_counts *counts, int *le_own, int *done) {
+    FastaChunks f{set, reverse, le_before};
+    const sgpu_status rc = pipeline_host(c, s, out, counts, done, f);
     *le_own = f.le_own;
     return rc;
 }
 
-// the one-shot host path: the whole buffer on the device, `call(d_in, d_w, cap_w, d_o, cap_o)` on it, outputs back.
+// the one-shot host path: the whole buffer on the device, `call(d, d_out)` on it -- d is the shard `s` with its bytes
+// on the device, d_out the device outputs --, outputs back.
 // write_fastq's output is the input re-serialised: larger only when line endings are rewritten (FASTQ: LF records
 // after a CRLF first record) or FASTA header-only records gain an empty sequence line.  Device buffers are sized for
 // the common case first.
 template <class Call>
-static sgpu_status oneshot_host(sgpu_ctx *c, const uint8_t *in, size_t n_in, uint8_t *out_w, size_t cap_w, size_t *n_w,
-                                uint8_t *out_o, size_t cap_o, size_t *n_o, Call call) {
+static sgpu_status oneshot_host(sgpu_ctx *c, const Shard &s, const Outs &out, Call call) {
     cudaStream_t st = c->stream;
     DevBuf<uint8_t> d_in, d_w, d_o;
-    SGPU_TRY(d_in.alloc(n_in + 16, st));
-    if (n_in) SGPU_CUDA(cudaMemcpyAsync(d_in.p, in, n_in, cudaMemcpyHostToDevice, st));
+    SGPU_TRY(d_in.alloc(s.n + 16, st));
+    if (s.n) SGPU_CUDA(cudaMemcpyAsync(d_in.p, s.p, s.n, cudaMemcpyHostToDevice, st));
     sgpu_status rc = SGPU_OK;
     for (int attempt = 0; attempt < 2; attempt++) {
-        const size_t want = attempt ? ~(size_t)0 : n_in + n_in / 16 + 4096;
-        const size_t dcap_w = std::min(cap_w, want), dcap_o = std::min(cap_o, want);
+        const size_t want = attempt ? ~(size_t)0 : s.n + s.n / 16 + 4096;
+        const size_t dcap_w = std::min(out.cap_w, want), dcap_o = std::min(out.cap_o, want);
         SGPU_TRY(d_w.alloc(dcap_w + 16, st));
-        if (out_o) SGPU_TRY(d_o.alloc(dcap_o + 16, st));
-        rc = call(d_in.p, d_w.p, dcap_w, out_o ? d_o.p : nullptr, dcap_o);
-        if (rc != SGPU_ERR_CAPACITY || (dcap_w == cap_w && (!out_o || dcap_o == cap_o))) break;
+        if (out.o) SGPU_TRY(d_o.alloc(dcap_o + 16, st));
+        rc = call(Shard{d_in.p, s.n, s.own_len, s.is_first, s.is_last},
+                  Outs{d_w.p, dcap_w, out.n_w, out.o ? d_o.p : nullptr, dcap_o, out.n_o});
+        if (rc != SGPU_ERR_CAPACITY || (dcap_w == out.cap_w && (!out.o || dcap_o == out.cap_o))) break;
     }
     if (rc == SGPU_ERR_CAPACITY || rc == SGPU_ERR_CUDA || rc == SGPU_ERR_NOMEM || rc == SGPU_ERR_PHASE_UNKNOWN) return rc;
-    if (*n_w) SGPU_CUDA(cudaMemcpyAsync(out_w, d_w.p, *n_w, cudaMemcpyDeviceToHost, st));
-    if (out_o && n_o && *n_o) SGPU_CUDA(cudaMemcpyAsync(out_o, d_o.p, *n_o, cudaMemcpyDeviceToHost, st));
+    if (*out.n_w) SGPU_CUDA(cudaMemcpyAsync(out.w, d_w.p, *out.n_w, cudaMemcpyDeviceToHost, st));
+    if (out.o && out.n_o && *out.n_o) SGPU_CUDA(cudaMemcpyAsync(out.o, d_o.p, *out.n_o, cudaMemcpyDeviceToHost, st));
     SGPU_CUDA(cudaStreamSynchronize(st));
     return rc;
 }
@@ -696,42 +557,40 @@ sgpu_status sgpu_clean_fastq(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *
     if (!c || !set || !n_w || !counts || (n_in && !in) || (cap_w && !out_w)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
+    const Shard s{in, n_in, n_in, 1, 1};
+    const Outs out{out_w, cap_w, n_w, out_o, cap_o, n_o};
+    Fmt f;
+    SGPU_TRY(input_format(c, in, false, n_in, true, &f));
     {
         int done = 0, le_own;
-        sgpu_status prc = n_in >= 5 && in[0] == '>'
-                              ? fasta_host_pipelined(c, set, in, n_in, n_in, 1, 1, -1, reverse, out_w, cap_w, n_w, out_o,
-                                                     cap_o, n_o, counts, &le_own, &done)
-                              : clean_host_pipelined(c, set, in, n_in, n_in, 0, 1, 1, -1, reverse, out_w, cap_w, n_w, out_o,
-                                                     cap_o, n_o, counts, &done);
+        sgpu_status prc = f == Fmt::fasta ? fasta_host_pipelined(c, set, s, -1, reverse, out, counts, &le_own, &done)
+                                          : clean_host_pipelined(c, set, s, 0, -1, reverse, out, counts, &done);
         if (done || prc != SGPU_OK) return prc;
     }
-    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
-                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
-                            return clean_dev_locked(c, set, d_in, n_in, reverse, d_w, dcap_w, n_w, d_o, dcap_o, n_o, counts);
-                        });
+    return oneshot_host(c, s, out, [&](const Shard &d, const Outs &d_out) {
+        return clean_file(c, set, d, f, reverse, d_out, counts);
+    });
 }
 
 sgpu_status sgpu_clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
                                    uint64_t newlines_before, int is_first, int is_last, int crlf, int reverse,
                                    uint8_t *out_w, size_t cap_w, size_t *n_w, uint8_t *out_o, size_t cap_o, size_t *n_o,
                                    sgpu_counts *counts) {
-    if (!c || !set || !n_w || !counts || (n_in && !in) || (cap_w && !out_w) || own_len > n_in ||
-        (is_last && own_len != n_in) || (is_first && newlines_before != 0) || crlf < -1 || crlf > 1 ||
-        (!is_first && crlf < 0 && newlines_before != SGPU_NEWLINES_UNKNOWN))
+    if (!c || !set || !n_w || !counts || (n_in && !in) || (cap_w && !out_w) ||
+        !fastq_shard_args_ok(n_in, own_len, newlines_before, is_first, is_last, crlf))
         return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
+    const Shard s{in, n_in, own_len, is_first, is_last};
+    const Outs out{out_w, cap_w, n_w, out_o, cap_o, n_o};
     {
         int done = 0;
-        sgpu_status prc = clean_host_pipelined(c, set, in, n_in, own_len, newlines_before, is_first, is_last, crlf, reverse,
-                                               out_w, cap_w, n_w, out_o, cap_o, n_o, counts, &done);
+        sgpu_status prc = clean_host_pipelined(c, set, s, newlines_before, crlf, reverse, out, counts, &done);
         if (done || prc != SGPU_OK) return prc;
     }
-    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
-                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
-                            return clean_shard_locked(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, crlf,
-                                                      reverse, d_w, dcap_w, n_w, d_o, dcap_o, n_o, counts, crlf < 0);
-                        });
+    return oneshot_host(c, s, out, [&](const Shard &d, const Outs &d_out) {
+        return clean_fastq_shard(c, set, d, newlines_before, crlf, reverse, d_out, counts, crlf < 0);
+    });
 }
 
 // argument checks shared by the FASTA shard entry points
@@ -742,15 +601,13 @@ static bool fasta_shard_args_ok(size_t n_in, size_t own_len, int is_last, int le
 
 // the FASTA shard's first byte and the empty-input rule (context locked).  *empty: a first-and-last shard of fewer
 // than 5 bytes (utils.rs:359-375); SGPU_ERR_INVALID_ARG: a first shard that does not start with '>'
-static sgpu_status fasta_shard_head(sgpu_ctx *c, const uint8_t *buf, bool on_device, size_t n_in, int is_first,
-                                    int is_last, bool *empty) {
-    *empty = is_first && is_last && n_in < 5;
-    if (*empty || !is_first) return SGPU_OK;
-    if (n_in == 0) return SGPU_ERR_INVALID_ARG;
-    if (!on_device) return buf[0] == '>' ? SGPU_OK : SGPU_ERR_INVALID_ARG;
-    SGPU_CUDA(cudaMemcpyAsync(c->h_pinned, buf, 1, cudaMemcpyDeviceToHost, c->stream));
-    SGPU_CUDA(cudaStreamSynchronize(c->stream));
-    return *(uint8_t *)c->h_pinned == '>' ? SGPU_OK : SGPU_ERR_INVALID_ARG;
+static sgpu_status fasta_shard_head(sgpu_ctx *c, const Shard &s, bool on_device, bool *empty) {
+    *empty = false;
+    if (!s.is_first) return SGPU_OK;
+    Fmt f;
+    SGPU_TRY(input_format(c, s.p, on_device, s.n, s.is_last, &f));
+    *empty = f == Fmt::empty && s.is_last;
+    return *empty || f == Fmt::fasta ? SGPU_OK : SGPU_ERR_INVALID_ARG;
 }
 
 sgpu_status sgpu_clean_fasta_shard_dev(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
@@ -763,18 +620,17 @@ sgpu_status sgpu_clean_fasta_shard_dev(sgpu_ctx *c, const sgpu_idset *set, const
     if (n_in && ((uintptr_t)d_in & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    memset(counts, 0, sizeof(*counts));
-    *n_w = 0;
-    if (n_o) *n_o = 0;
+    const Shard s{d_in, n_in, own_len, is_first, is_last};
+    const Outs out{d_out_w, cap_w, n_w, d_out_o, cap_o, n_o};
+    clear_outputs(out, counts);
     *le_own = -1;
     bool empty;
-    SGPU_TRY(fasta_shard_head(c, d_in, true, n_in, is_first, is_last, &empty));
+    SGPU_TRY(fasta_shard_head(c, s, true, &empty));
     if (empty) {
         counts->empty_input = 1;
         return SGPU_OK;
     }
-    return clean_fasta_shard(c, set, d_in, n_in, own_len, is_first, is_last, le_before, reverse, d_out_w, cap_w, n_w, d_out_o,
-                             cap_o, n_o, counts, le_own);
+    return clean_fasta_shard(c, set, s, le_before, reverse, out, counts, le_own);
 }
 
 sgpu_status sgpu_clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *in, size_t n_in, size_t own_len,
@@ -786,28 +642,24 @@ sgpu_status sgpu_clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uin
         return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    memset(counts, 0, sizeof(*counts));
-    *n_w = 0;
-    if (n_o) *n_o = 0;
+    const Shard s{in, n_in, own_len, is_first, is_last};
+    const Outs out{out_w, cap_w, n_w, out_o, cap_o, n_o};
+    clear_outputs(out, counts);
     *le_own = -1;
     bool empty;
-    SGPU_TRY(fasta_shard_head(c, in, false, n_in, is_first, is_last, &empty));
+    SGPU_TRY(fasta_shard_head(c, s, false, &empty));
     if (empty) {
         counts->empty_input = 1;
         return SGPU_OK;
     }
     {
         int done = 0;
-        sgpu_status prc = fasta_host_pipelined(c, set, in, n_in, own_len, is_first, is_last, le_before, reverse, out_w, cap_w,
-                                               n_w, out_o, cap_o, n_o, counts, le_own, &done);
+        sgpu_status prc = fasta_host_pipelined(c, set, s, le_before, reverse, out, counts, le_own, &done);
         if (done || prc != SGPU_OK) return prc;
     }
-    return oneshot_host(c, in, n_in, out_w, cap_w, n_w, out_o, cap_o, n_o,
-                        [&](const uint8_t *d_in, uint8_t *d_w, size_t dcap_w, uint8_t *d_o, size_t dcap_o) {
-                            memset(counts, 0, sizeof(*counts));
-                            return clean_fasta_shard(c, set, d_in, n_in, own_len, is_first, is_last, le_before, reverse, d_w,
-                                                     dcap_w, n_w, d_o, dcap_o, n_o, counts, le_own);
-                        });
+    return oneshot_host(c, s, out, [&](const Shard &d, const Outs &d_out) {
+        return clean_fasta_shard(c, set, d, le_before, reverse, d_out, counts, le_own);
+    });
 }
 
 sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
@@ -817,12 +669,12 @@ sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const
     if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
+    const Shard s{d_buf, n_buf, own_len, is_first, is_last};
     bool empty;
-    SGPU_TRY(fasta_shard_head(c, d_buf, true, n_buf, is_first, is_last, &empty));
+    SGPU_TRY(fasta_shard_head(c, s, true, &empty));
     if (empty) return SGPU_OK;
     uint64_t n_rec = 0, n_pick = 0, err = 0;
-    sgpu_status rc = fasta_ids_shard(c, d_buf, n_buf, own_len, is_first, is_last, probe, probe != nullptr, into, &n_rec,
-                                     &n_pick, &err);
+    sgpu_status rc = fasta_ids_shard(c, s, probe, probe != nullptr, into, &n_rec, &n_pick, &err);
     if (rc == SGPU_OK) {
         counts->reads_in += n_rec;
         counts->difference += n_pick;
@@ -842,10 +694,10 @@ sgpu_status sgpu_diff_dev(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, const u
     sgpu_idset *o_ids = nullptr;  // utils.rs:257 reads2_ids
     SGPU_TRY(idset_create(c, &o_ids));
     uint64_t n_rec = 0, n_pick = 0, err = 0;
-    sgpu_status rc = fastq_ids_into(c, d_out, n_out, n_out, 0, 1, 1, nullptr, 0, o_ids, &n_rec, &n_pick, &err);  // :259-267
+    sgpu_status rc = ids_locked(c, Shard{d_out, n_out, n_out, 1, 1}, 0, nullptr, 0, o_ids, &n_rec, &n_pick, &err);  // :259-267
     if (rc == SGPU_OK) {
         counts->reads_out += n_rec;
-        rc = fastq_ids_into(c, d_in, n_in, n_in, 0, 1, 1, o_ids, 1, *diff_ids, &n_rec, &n_pick, &err);  // :269-283
+        rc = ids_locked(c, Shard{d_in, n_in, n_in, 1, 1}, 0, o_ids, 1, *diff_ids, &n_rec, &n_pick, &err);  // :269-283
         if (rc == SGPU_OK) {
             counts->reads_in += n_rec;
             counts->difference += n_pick;
@@ -860,8 +712,7 @@ sgpu_status sgpu_diff_dev(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, const u
 sgpu_status sgpu_fastq_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
                                      size_t own_len, uint64_t newlines_before, int is_first, int is_last,
                                      sgpu_idset *into, sgpu_counts *counts) {
-    if (!c || !counts || (n_buf && !d_buf) || own_len > n_buf || (is_last && own_len != n_buf) ||
-        (is_first && newlines_before != 0))
+    if (!c || !counts || (n_buf && !d_buf) || !fastq_shard_args_ok(n_buf, own_len, newlines_before, is_first, is_last, 0))
         return SGPU_ERR_INVALID_ARG;
     if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
@@ -869,8 +720,8 @@ sgpu_status sgpu_fastq_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const
     uint64_t n_rec = 0, n_pick = 0, err = 0;
     sgpu_counts spec;
     memset(&spec, 0, sizeof(spec));
-    sgpu_status rc = fastq_ids_into(c, d_buf, n_buf, own_len, newlines_before, is_first, is_last, probe, probe != nullptr,
-                                    into, &n_rec, &n_pick, &err, &spec);
+    sgpu_status rc = ids_locked(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, newlines_before, probe,
+                                probe != nullptr, into, &n_rec, &n_pick, &err, &spec);
     if (rc == SGPU_OK) {
         counts->reads_in += n_rec;
         counts->difference += n_pick;

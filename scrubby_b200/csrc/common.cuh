@@ -339,6 +339,8 @@ sgpu_status index_newlines(sgpu_ctx *c, const uint8_t *d_buf, size_t n, DevBuf<u
 sgpu_status count_newlines(sgpu_ctx *c, const uint8_t *d_buf, size_t n, uint64_t *count);
 // d2h of a few u64 through the pinned staging buffer, synchronises the stream
 sgpu_status read_u64s(sgpu_ctx *c, const void *d_src, uint64_t *h_dst, size_t count);
+// h2d of a few u64 (scratch initialisation) through the upper half of the pinned staging buffer, stream-ordered
+sgpu_status write_u64s(sgpu_ctx *c, void *d_dst, const uint64_t *h_src, size_t count);
 
 // capi.cu: drops one reference; the last one tears the context down
 void ctx_release(sgpu_ctx *c);

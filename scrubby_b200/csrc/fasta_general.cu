@@ -214,21 +214,20 @@ struct FaTables {
 
 // SGPU_ERR_HALO: a shard that is not the last one does not hold the start of the record after its last owned one.
 // T.P.n_rec == 0: the shard owns no record (nothing was launched after the table)
-static sgpu_status fasta_records(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, size_t own_len, int is_first, int is_last,
-                                 const sgpu_idset *set, int reverse, int want_absent, bool want_keys, FaTables &T) {
+static sgpu_status fasta_records(sgpu_ctx *c, const Shard &s, const sgpu_idset *set, int reverse, int want_absent,
+                                 bool want_keys, FaTables &T) {
     cudaStream_t st = c->stream;
     // [0] err word, [1] first record that decides the line ending, [2] starts, [3..4] counters, [5..6] totals, [7] owned starts
     SGPU_TRY(T.scratch.alloc(8, st));
     const uint64_t init[8] = {~0ull, ~0ull, 0, 0, 0, 0, 0, 0};
-    memcpy(c->h_pinned + 32, init, sizeof(init));
-    SGPU_CUDA(cudaMemcpyAsync(T.scratch.p, c->h_pinned + 32, sizeof(init), cudaMemcpyHostToDevice, st));
+    SGPU_TRY(write_u64s(c, T.scratch.p, init, 8));
     uint64_t n_nl = 0;
-    SGPU_TRY(index_newlines(c, d_in, n_in, T.nlpos, &n_nl));
+    SGPU_TRY(index_newlines(c, s.p, s.n, T.nlpos, &n_nl));
     uint64_t h[6] = {0, 0, 0, 0, 0, 0};  // scratch [2..7]
     if (n_nl) {
         SGPU_TRY(T.mark.alloc(n_nl, st));
         SGPU_TRY(T.rank.alloc(n_nl, st));
-        fa_mark_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(d_in, n_in, T.nlpos.p, n_nl, own_len,
+        fa_mark_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(s.p, s.n, T.nlpos.p, n_nl, s.own_len,
                                                                                 T.mark.p,
                                                                                 (unsigned long long *)(T.scratch.p + 7));
         SGPU_LAUNCH(c);
@@ -236,17 +235,17 @@ static sgpu_status fasta_records(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, 
         SGPU_TRY(read_u64s(c, T.scratch.p + 2, h, 6));
     }
     const uint64_t n_starts = h[0], n_owned = h[5];
-    const uint64_t n_rec = (is_first ? 1 : 0) + n_owned;
-    const uint64_t n_tab = (is_first ? 1 : 0) + n_starts;
-    T.P = FaParams{d_in, (uint64_t)n_in, T.nlpos.p, n_nl, nullptr, n_rec, n_tab, is_first ? 1 : 0};
+    const uint64_t n_rec = (s.is_first ? 1 : 0) + n_owned;
+    const uint64_t n_tab = (s.is_first ? 1 : 0) + n_starts;
+    T.P = FaParams{s.p, (uint64_t)s.n, T.nlpos.p, n_nl, nullptr, n_rec, n_tab, s.is_first ? 1 : 0};
     if (n_rec == 0) return SGPU_OK;
-    if (!is_last && n_tab == n_rec) return SGPU_ERR_HALO;  // the end of the last owned record is not in the buffer
+    if (!s.is_last && n_tab == n_rec) return SGPU_ERR_HALO;  // the end of the last owned record is not in the buffer
     SGPU_TRY(T.rec_nl.alloc(n_starts + 1, st));
     if (n_starts) {
         fa_scatter_kernel<<<(unsigned)ceil_div(n_nl, (uint64_t)256), 256, 0, st>>>(T.mark.p, T.rank.p, n_nl, T.rec_nl.p);
         SGPU_LAUNCH(c);
     }
-    T.P.rec_nl = T.rec_nl.p + (is_first ? 0 : 1);  // table entry 0 stands for byte 0
+    T.P.rec_nl = T.rec_nl.p + (s.is_first ? 0 : 1);  // table entry 0 stands for byte 0
     SGPU_TRY(T.meta.alloc(n_rec, st));
     if (want_keys) {
         SGPU_TRY(T.key_off.alloc(n_rec, st));
@@ -268,15 +267,14 @@ static sgpu_status fasta_records(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, 
 // FastqCleaner::clean_reads over the FASTA records a shard owns.  Device pointers in, device outputs filled, counts on
 // the host.  le_before: -1 undecided, 0 / 1 LF / CRLF decided by an earlier shard; *le_own: what this shard's first
 // deciding record (before an error) says, -1 when it has none.
-sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                              int is_first, int is_last, int le_before, int reverse, uint8_t *d_out_w, size_t cap_w,
-                              size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
-                              int *le_own) {
+sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, int le_before, int reverse,
+                              const Outs &out, sgpu_counts *counts, int *le_own) {
     cudaStream_t st = c->stream;
+    clear_outputs(out, counts);
     counts->path = 3;
     *le_own = -1;
     FaTables T;
-    SGPU_TRY(fasta_records(c, d_in, n_in, own_len, is_first, is_last, set, reverse, 0, false, T));
+    SGPU_TRY(fasta_records(c, s, set, reverse, 0, false, T));
     const uint64_t n_rec = T.P.n_rec;
     if (n_rec == 0) {
         counts->crlf = le_before > 0;
@@ -316,7 +314,7 @@ sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
                                                                              len_o.p, (unsigned long long *)(T.scratch.p + 3));
     SGPU_LAUNCH(c);
     SGPU_TRY(exclusive_scan_u32_to_u64(c, len_w.p, off_w.p, n_rec, T.scratch.p + 5));
-    if (d_out_o) {
+    if (out.o) {
         SGPU_TRY(off_o.alloc(n_rec, st));
         SGPU_TRY(exclusive_scan_u32_to_u64(c, len_o.p, off_o.p, n_rec, T.scratch.p + 6));
     }
@@ -324,11 +322,11 @@ sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
     SGPU_TRY(read_u64s(c, T.scratch.p + 3, h, 4));
     counts->reads_in = h[0];
     counts->reads_out = h[1];
-    *n_w = (size_t)h[2];
-    if (n_o) *n_o = d_out_o ? (size_t)h[3] : 0;
-    if (h[2] > cap_w || (d_out_o && h[3] > cap_o)) return SGPU_ERR_CAPACITY;
+    *out.n_w = (size_t)h[2];
+    if (out.n_o) *out.n_o = out.o ? (size_t)h[3] : 0;
+    if (h[2] > out.cap_w || (out.o && h[3] > out.cap_o)) return SGPU_ERR_CAPACITY;
     fa_copy_kernel<<<(unsigned)ceil_div(n_rec * 32, (uint64_t)256), 256, 0, st>>>(T.P, T.meta.p, off_w.p, off_o.p, le_from, crlf,
-                                                                                  d_out_w, d_out_o);
+                                                                                  out.w, out.o);
     SGPU_LAUNCH(c);
     SGPU_CUDA(cudaGetLastError());
     SGPU_CUDA(cudaStreamSynchronize(st));  // scratch buffers are released after this call returns
@@ -336,12 +334,11 @@ sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
 }
 
 // one loop of ReadDifference::get_difference (utils.rs:259-267 / 269-283) over the FASTA records a shard owns
-sgpu_status fasta_ids_shard(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t own_len, int is_first, int is_last,
-                            const sgpu_idset *probe, int want_absent, sgpu_idset *into, uint64_t *n_records,
-                            uint64_t *n_picked, uint64_t *err_record) {
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, sgpu_idset *into,
+                            uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record) {
     *n_records = *n_picked = 0;
     FaTables T;
-    SGPU_TRY(fasta_records(c, d_buf, n, own_len, is_first, is_last, want_absent ? probe : nullptr, 0, want_absent, true, T));
+    SGPU_TRY(fasta_records(c, s, want_absent ? probe : nullptr, 0, want_absent, true, T));
     const uint64_t n_rec = T.P.n_rec;
     if (n_rec == 0) return SGPU_OK;
     if (T.err_word != ~0ull) {
@@ -357,7 +354,7 @@ sgpu_status fasta_ids_shard(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t 
     SGPU_TRY(read_u64s(c, T.scratch.p + 3, &picked, 1));
     *n_records = n_rec;
     *n_picked = picked;
-    if (into && picked) SGPU_TRY(idset_insert_spans(c, into, d_buf, T.key_off.p, T.key_len.p, T.sel.p, (size_t)n_rec));
+    if (into && picked) SGPU_TRY(idset_insert_spans(c, into, s.p, T.key_off.p, T.key_len.p, T.sel.p, (size_t)n_rec));
     SGPU_CUDA(cudaStreamSynchronize(st));
     return SGPU_OK;
 }

@@ -1277,18 +1277,6 @@ __global__ void fused_verify_kernel(const uint64_t *sum_prefix, const long long 
     }
 }
 
-// Runs the fused kernel over d_in[0..n_in).  The first owned record starts at `lead` (< 16); records that
-// start after own_len (when !is_last) are left to the next shard.  *used = 0 when the input turned out
-// not to be canonical (the caller then takes the general path).
-// ids mode (IdsOut != nullptr): nothing is written; the id tokens of the records absent from `set` are listed
-struct IdsOut {
-    uint64_t *off;
-    uint32_t *len;
-    uint64_t cap;
-    uint64_t n_spans;  // out
-    uint64_t base;     // out: the spans' offsets are relative to d_in + base
-};
-
 // '\n' bytes in [lead, own_len) of the range the fused kernel ran over, from its per-tile counts (whole tiles below
 // own_len: the exclusive prefix) plus the bytes of the one tile own_len cuts.  One CTA.
 __global__ void fused_own_newlines_kernel(const uint8_t *in, uint32_t lead, uint64_t own_len, const uint64_t *nl_prefix,
@@ -1314,11 +1302,14 @@ __global__ void fused_own_newlines_kernel(const uint8_t *in, uint32_t lead, uint
     }
 }
 
+// Runs the fused kernel over d_in[0..n_in).  The first owned record starts at `lead` (< 16); records that
+// start after own_len (when !is_last) are left to the next shard.  *used = 0 when the input turned out
+// not to be canonical (the caller then takes the general path).
+// ids mode (IdsOut != nullptr): nothing is written; the id tokens of the records absent from `set` are listed
 // want_own_nl: also count the '\n' bytes of [lead, own_len) into counts->own_newlines (speculative shards)
-sgpu_status clean_fused_range(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, uint32_t lead,
-                              size_t own_len, int is_last, int reverse, uint8_t *d_out_w, size_t cap_w, size_t *n_w,
-                              uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts, int *used,
-                              IdsOut *ids = nullptr, bool want_own_nl = false) {
+static sgpu_status clean_fused_range(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, uint32_t lead,
+                                     size_t own_len, int is_last, int reverse, const Outs &out, sgpu_counts *counts,
+                                     int *used, IdsOut *ids, bool want_own_nl) {
     *used = 0;
     if (n_in == 0 || lead >= 16) return SGPU_OK;
     // (the outputs may be smaller than the input: the kernel never writes past cap_w / cap_o and reports it)
@@ -1351,9 +1342,8 @@ sgpu_status clean_fused_range(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
     FusedResult init;
     memset(&init, 0, sizeof(init));
     init.owned_end = ~0ull;
-    static_assert(sizeof(FusedResult) <= 64 * 8 - 32 * 8, "pinned staging too small");
-    memcpy(c->h_pinned + 32, &init, sizeof(init));
-    SGPU_CUDA(cudaMemcpyAsync(res.p, c->h_pinned + 32, sizeof(init), cudaMemcpyHostToDevice, st));
+    static_assert(sizeof(FusedResult) % 8 == 0 && sizeof(FusedResult) <= 32 * 8, "pinned staging too small");
+    SGPU_TRY(write_u64s(c, res.p, (const uint64_t *)&init, sizeof(FusedResult) / 8));
     FusedParams P;
     P.in = d_in;
     P.n_in = n_in;
@@ -1361,10 +1351,10 @@ sgpu_status clean_fused_range(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
     P.own_len = own_len;
     P.lead = lead;
     P.is_last = is_last;
-    P.out_w = d_out_w;
-    P.out_o = d_out_o;
-    P.cap_w = cap_w;
-    P.cap_o = d_out_o ? cap_o : 0;
+    P.out_w = out.w;
+    P.out_o = out.o;
+    P.cap_w = out.cap_w;
+    P.cap_o = out.o ? out.cap_o : 0;
     P.reverse = reverse;
     P.set = view_of(set);
     P.desc1 = desc.p;
@@ -1477,9 +1467,9 @@ sgpu_status clean_fused_range(sgpu_ctx *c, const sgpu_idset *set, const uint8_t 
     }
     const uint64_t owned_end = is_last ? n_in : h.owned_end;
     const uint64_t other_total = owned_end - lead - h.kept_total;
-    if (c->profiling) c->prof_alg_bytes += n_in + h.kept_total + (d_out_o ? other_total : 0);
-    *n_w = (size_t)h.kept_total;
-    if (n_o) *n_o = d_out_o ? (size_t)other_total : 0;
+    if (c->profiling) c->prof_alg_bytes += n_in + h.kept_total + (out.o ? other_total : 0);
+    *out.n_w = (size_t)h.kept_total;
+    if (out.n_o) *out.n_o = out.o ? (size_t)other_total : 0;
     counts->reads_in = h.reads_in;
     counts->reads_out = h.reads_out;
     counts->crlf = 0;
@@ -1518,23 +1508,21 @@ __global__ void first_newlines_kernel(const uint8_t *buf, uint64_t n, unsigned l
 }
 
 // one shard (see sgpu_clean_fastq_shard_dev): locate the first owned record start, then run the fused kernel
-// from the 16-byte aligned address below it.  *used = 0: take the general path.
+// from the 16-byte aligned address below it.  A whole file is the shard (n, n, 0, 1, 1): the range is the buffer.
 // newlines_before == SGPU_NEWLINES_UNKNOWN: the line phase is SPECULATED from the first "\n+\n" among the shard's first
 // four newlines (it ends a sequence line, so the newline two places before / behind it ends a record); the caller
 // verifies (true newlines_before + counts->lead_newlines) % 4 == 0 once the shards' own_newlines are exchanged.
-static sgpu_status fused_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                               uint64_t newlines_before, int is_first, int is_last, int reverse, uint8_t *d_out_w,
-                               size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                               sgpu_counts *counts, int *used, IdsOut *ids, bool want_nl = false) {
+sgpu_status fused_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint64_t newlines_before, int reverse,
+                        const Outs &out, IdsOut *ids, sgpu_counts *counts, int *used, bool want_nl) {
     *used = 0;
     const bool spec = newlines_before == SGPU_NEWLINES_UNKNOWN;
     want_nl = want_nl || spec;
     uint64_t s0 = 0, lead_nl = 0;
-    if (!is_first) {
+    if (!s.is_first) {
         DevBuf<unsigned long long> pos;
         SGPU_TRY(pos.alloc(8, c->stream));
         SGPU_CUDA(cudaMemsetAsync(pos.p, 0xFF, 64, c->stream));
-        first_newlines_kernel<<<1, 32, 0, c->stream>>>(d_in, n_in, pos.p);
+        first_newlines_kernel<<<1, 32, 0, c->stream>>>(s.p, s.n, pos.p);
         SGPU_LAUNCH(c);
         uint64_t h[8];
         SGPU_TRY(read_u64s(c, pos.p, h, 8));
@@ -1551,59 +1539,19 @@ static sgpu_status fused_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t
         if (h[k] == ~0ull) return SGPU_OK;  // no record boundary in the buffer: the general path sorts it out
         s0 = h[k] + 1;
         lead_nl = k + 1;
-        if (s0 >= n_in || s0 > own_len) return SGPU_OK;  // owns nothing (general path: zero records / errors)
+        if (s0 >= s.n || s0 > s.own_len) return SGPU_OK;  // owns nothing (general path: zero records / errors)
     }
     const uint32_t lead = (uint32_t)(s0 & 15);
     const uint64_t skip = s0 - lead;
-    sgpu_status rc;
-    if (ids) {  // span offsets are relative to the range the kernel sees: rebase them to d_in afterwards
-        rc = clean_fused_range(c, set, d_in + skip, n_in - skip, lead, own_len - skip, is_last, reverse, nullptr, 0,
-                               nullptr, nullptr, 0, nullptr, counts, used, ids, want_nl);
-        ids->base = skip;
-    } else {
-        rc = clean_fused_range(c, set, d_in + skip, n_in - skip, lead, own_len - skip, is_last, reverse, d_out_w, cap_w,
-                               n_w, d_out_o, cap_o, n_o, counts, used, nullptr, want_nl);
-    }
+    const sgpu_status rc = clean_fused_range(c, set, s.p + skip, s.n - skip, lead, s.own_len - skip, s.is_last, reverse,
+                                             out, counts, used, ids, want_nl);
+    if (ids) ids->base = skip;  // span offsets are relative to the range the kernel saw
     if (want_nl && *used) {
         counts->lead_newlines = lead_nl;
         counts->own_newlines += lead_nl;  // [0, s0) + [s0, own_len)
         counts->speculated = spec ? 1 : 0;
     }
     return rc;
-}
-
-sgpu_status clean_fused_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                              uint64_t newlines_before, int is_first, int is_last, int reverse, uint8_t *d_out_w,
-                              size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                              sgpu_counts *counts, int *used, bool want_nl) {
-    return fused_shard(c, set, d_in, n_in, own_len, newlines_before, is_first, is_last, reverse, d_out_w, cap_w, n_w,
-                       d_out_o, cap_o, n_o, counts, used, nullptr, want_nl);
-}
-
-// ReadDifference::get_difference's two loops (utils.rs:259-267, 269-283) over canonical FASTQ: the id tokens of
-// the records absent from `probe` (nullptr: every record) as (offset, length) spans; *used = 0: general path
-// (shards as in clean_fused_shard; *span_base: the offsets are relative to d_in + *span_base)
-sgpu_status ids_fused(sgpu_ctx *c, const sgpu_idset *probe, const uint8_t *d_in, size_t n_in, size_t own_len,
-                      uint64_t newlines_before, int is_first, int is_last, uint64_t *span_off, uint32_t *span_len,
-                      uint64_t cap, uint64_t *n_spans, uint64_t *span_base, uint64_t *n_records, int *used,
-                      sgpu_counts *spec_out) {
-    IdsOut ids{span_off, span_len, cap, 0, 0};
-    sgpu_counts counts;
-    memset(&counts, 0, sizeof(counts));
-    SGPU_TRY(fused_shard(c, probe, d_in, n_in, own_len, newlines_before, is_first, is_last, 0, nullptr, 0, nullptr,
-                         nullptr, 0, nullptr, &counts, used, &ids));
-    if (spec_out) *spec_out = counts;
-    *n_spans = ids.n_spans;
-    *span_base = ids.base;
-    *n_records = counts.reads_in;
-    return SGPU_OK;
-}
-
-sgpu_status clean_fused(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, int reverse,
-                        uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                        sgpu_counts *counts, int *used) {
-    return clean_fused_range(c, set, d_in, n_in, 0, n_in, 1, reverse, d_out_w, cap_w, n_w, d_out_o, cap_o, n_o,
-                             counts, used);
 }
 
 }  // namespace sgpu

@@ -1,4 +1,5 @@
-// fastq_records.cuh -- record location / validation shared by the general clean path and diff.
+// fastq_records.cuh -- record location / validation shared by the general clean path and diff, and the internal
+// interface of the FASTQ and FASTA shard cores.
 // Restates needletail 0.5.1 fastq Reader::next / find / validate / check_end over a '\n' index.
 #pragma once
 #include "idset.cuh"
@@ -112,20 +113,63 @@ static inline bool setup_records(RecParams &P, uint64_t n_nl, uint64_t newlines_
     return true;
 }
 
-// fastq_general.cu
-sgpu_status clean_general(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                          uint64_t newlines_before, int is_first, int is_last, int crlf_in, int reverse,
-                          uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o,
-                          sgpu_counts *counts);
+// one shard of a file: its own bytes [0, own_len) followed by a halo (the contracts are those of the shard entry points
+// in include/scrubby_gpu.h); a whole file is the shard {p, n, n, 1, 1}
+struct Shard {
+    const uint8_t *p;
+    size_t n, own_len;
+    int is_first, is_last;
+};
+
+// the two outputs of a clean call: the written records and the others (o == nullptr: not produced), their capacities,
+// and where the produced sizes go (n_o may be nullptr)
+struct Outs {
+    uint8_t *w;
+    size_t cap_w;
+    size_t *n_w;
+    uint8_t *o;
+    size_t cap_o;
+    size_t *n_o;
+};
+
+// nothing produced (yet): counts and produced sizes zeroed
+static inline void clear_outputs(const Outs &out, sgpu_counts *counts) {
+    memset(counts, 0, sizeof(*counts));
+    *out.n_w = 0;
+    if (out.n_o) *out.n_o = 0;
+}
+
+// fastq_general.cu: FastqCleaner::clean_reads and one loop of ReadDifference::get_difference over the FASTQ records a
+// shard owns (the contracts are sgpu_clean_fastq_shard_dev's and sgpu_fastq_ids_shard_dev's; a whole file is the shard
+// (n, n, newlines_before 0, first, last, crlf -1)).  The single-pass kernel runs when it takes the input, else the
+// general path.  want_nl: when the single-pass kernel produces the result, counts->own_newlines is filled from its
+// per-tile counts.  spec_out (may be nullptr): the single-pass kernel's counts (speculated, own / lead newlines); the
+// general path adds nothing to it.  A non-first shard without a record boundary: clean produces zero records, ids returns
+// SGPU_ERR_FASTQ_UNEXPECTED_END (last shard) or SGPU_ERR_HALO
+sgpu_status clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint64_t newlines_before, int crlf,
+                              int reverse, const Outs &out, sgpu_counts *counts, bool want_nl);
+sgpu_status fastq_ids_shard(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
+                            int want_absent, sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked,
+                            uint64_t *err_record, sgpu_counts *spec_out);
+
+// fastq_fused.cu: the single-pass kernel over one FASTQ shard; *used = 0 when the input is not canonical (the caller
+// then takes the general path).  ids mode (ids != nullptr, `out` unused): nothing is written; the id tokens of the
+// records absent from `set` (nullptr: every record) are listed as (offset, length) spans
+struct IdsOut {
+    uint64_t *off;
+    uint32_t *len;
+    uint64_t cap;
+    uint64_t n_spans;  // out
+    uint64_t base;     // out: the spans' offsets are relative to the shard's byte `base`
+};
+sgpu_status fused_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint64_t newlines_before, int reverse,
+                        const Outs &out, IdsOut *ids, sgpu_counts *counts, int *used, bool want_nl);
 
 // fasta_general.cu: the same two operations over the FASTA records a shard owns (needletail's FASTA reader; a whole
 // file is the shard (n, n, first, last)); the shard contract is sgpu_clean_fasta_shard_dev's
-sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in, size_t own_len,
-                              int is_first, int is_last, int le_before, int reverse, uint8_t *d_out_w, size_t cap_w,
-                              size_t *n_w, uint8_t *d_out_o, size_t cap_o, size_t *n_o, sgpu_counts *counts,
-                              int *le_own);
-sgpu_status fasta_ids_shard(sgpu_ctx *c, const uint8_t *d_buf, size_t n, size_t own_len, int is_first, int is_last,
-                            const sgpu_idset *probe, int want_absent, sgpu_idset *into, uint64_t *n_records,
-                            uint64_t *n_picked, uint64_t *err_record);
+sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, int le_before, int reverse,
+                              const Outs &out, sgpu_counts *counts, int *le_own);
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, sgpu_idset *into,
+                            uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record);
 
 }  // namespace sgpu

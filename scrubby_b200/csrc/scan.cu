@@ -139,6 +139,13 @@ sgpu_status read_u64s(sgpu_ctx *c, const void *d_src, uint64_t *h_dst, size_t co
     return SGPU_OK;
 }
 
+sgpu_status write_u64s(sgpu_ctx *c, void *d_dst, const uint64_t *h_src, size_t count) {
+    if (count > 32) return SGPU_ERR_INVALID_ARG;
+    memcpy(c->h_pinned + 32, h_src, count * 8);
+    SGPU_CUDA(cudaMemcpyAsync(d_dst, c->h_pinned + 32, count * 8, cudaMemcpyHostToDevice, c->stream));
+    return SGPU_OK;
+}
+
 // ------------------------------------------------------------------------------------
 // '\n' index: tile counts -> exclusive scan -> positions
 // ------------------------------------------------------------------------------------
