@@ -296,6 +296,33 @@ sgpu_status sgpu_fastq_ids_shard_dev(sgpu_ctx *, const sgpu_idset *probe, const 
  * counts->reads_in += records, counts->difference += picked records. */
 sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *, const sgpu_idset *probe, const uint8_t *d_buf, size_t n_buf,
                                      size_t own_len, int is_first, int is_last, sgpu_idset *into, sgpu_counts *counts);
+/* Hash-partitioned diff (scrubby_b200/dist.py diff_partitioned): every id has ONE owner rank, a pure function of its
+ * bytes, so the output-id set and the diff set are split across the ranks instead of being replicated on each.
+ *   Owner: route_owner(home, n_parts) = mulhi64(remix(home), n_parts), with home the 64-bit hash the id set uses for the
+ *     key (inline ids of 1..15 bytes: mix64 of the slot image; longer ids: mix64 of the fingerprint slot word) and remix
+ *     a fixed bijective 64-bit finaliser (x ^= 0x2545F4914F6CDD1D; x ^= x >> 30; x *= 0xBF58476D1CE4E5B9; x ^= x >> 27;
+ *     x *= 0x94D049BB133111EB; x ^= x >> 31).  The set an owner builds takes the page from home's high bits and the
+ *     bucket from its low 8 bits; the remix keeps a partition's keys spread over all pages.  Defined once, in
+ *     scrubby_b200/csrc/idset.cuh.
+ * The route entry points take the shard contract, statuses and counts of the ids entry points with probe NULL (counts->
+ * reads_in / difference += records, error_record, the speculation counts of sgpu_fastq_ids_shard_dev), and write the
+ * ids of the owned records as "id\n" lines grouped by owner partition: partition 0's lines first, then partition 1's,
+ * ...; inside a partition the lines keep file order.  part_bytes / part_lines: host arrays of n_parts (1..64) receiving
+ * each partition's bytes and lines; *n_lines: bytes written.  cap >= n_buf is always enough; a smaller cap may give
+ * SGPU_ERR_CAPACITY with *n_lines = bytes needed. */
+sgpu_status sgpu_fastq_ids_route_shard_dev(sgpu_ctx *, const uint8_t *d_buf, size_t n_buf, size_t own_len,
+                                           uint64_t newlines_before, int is_first, int is_last, int n_parts,
+                                           uint8_t *d_lines, size_t cap, size_t *n_lines,
+                                           uint64_t *part_bytes, uint64_t *part_lines, sgpu_counts *counts);
+/* the same for a FASTA shard (sgpu_fasta_ids_shard_dev's contract) */
+sgpu_status sgpu_fasta_ids_route_shard_dev(sgpu_ctx *, const uint8_t *d_buf, size_t n_buf, size_t own_len, int is_first,
+                                           int is_last, int n_parts, uint8_t *d_lines, size_t cap, size_t *n_lines,
+                                           uint64_t *part_bytes, uint64_t *part_lines, sgpu_counts *counts);
+/* "id\n" lines as routed (d_lines 16-byte aligned; a last line without '\n' counts too): counts->reads_in += lines,
+ * counts->difference += lines whose id is absent from `probe` (NULL: every line), and those ids are inserted into `into`
+ * (NULL: counted only).  Every line is one input record: a repeated id counts once per line (utils.rs:269-283). */
+sgpu_status sgpu_idset_probe_lines_dev(sgpu_ctx *, const sgpu_idset *probe, const uint8_t *d_lines, size_t n,
+                                       sgpu_idset *into, sgpu_counts *counts);
 /* ReadDifference::get_difference, utils.rs:250-285, for ONE (input, output) file pair:
  * counts->{reads_in, reads_out, difference} are incremented (+=) and the ids absent from the
  * output are inserted into *diff_ids (created when *diff_ids == NULL), so calling it once

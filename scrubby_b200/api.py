@@ -446,6 +446,59 @@ def fastq_ids_shard_dev(ctx: Context, probe, d_buf, n_buf: int, own_len: int, ne
     return c.reads_in, c.difference
 
 
+@dataclass
+class RouteResult:
+    lines: object           # device uint8 tensor: the "id\n" lines, partition 0's first, file order inside a partition
+    part_bytes: list        # bytes of each partition's lines
+    part_lines: list
+    reads_in: int           # records of the shard
+    speculated: bool = False  # FASTQ: the single-pass kernel's speculation counts (as fastq_ids_shard_dev's)
+    own_newlines: int = 0
+    lead_newlines: int = 0
+
+
+def _route(fn, what, ctx, d_buf, n_buf, n_parts, args):
+    import torch
+
+    cap = n_buf + 16  # the lines of a shard's records never exceed its buffer
+    out = torch.empty(cap, dtype=torch.uint8, device=d_buf.device)
+    n_lines, c = C.c_size_t(), _lib.Counts()
+    pb, pl = (C.c_uint64 * n_parts)(), (C.c_uint64 * n_parts)()
+    rc = fn(ctx.h, C.c_void_p(d_buf.data_ptr()), n_buf, *args, n_parts, C.c_void_p(out.data_ptr()), cap, C.byref(n_lines),
+            pb, pl, C.byref(c))
+    _check(rc, c.error_record, what)
+    return RouteResult(out[: n_lines.value], list(pb), list(pl), c.reads_in, bool(c.speculated), c.own_newlines,
+                       c.lead_newlines)
+
+
+def fastq_ids_route_shard_dev(ctx: Context, d_buf, n_buf: int, own_len: int, newlines_before, is_first: bool,
+                              is_last: bool, n_parts: int) -> RouteResult:
+    """sgpu_fastq_ids_route_shard_dev: the ids of the records a FASTQ shard owns as "id\\n" lines grouped by owner
+    partition (the hash-partitioned diff).  newlines_before=None: not exchanged yet (speculated, as in
+    fastq_ids_shard_dev with SGPU_NEWLINES_UNKNOWN)."""
+    nb = _lib.NEWLINES_UNKNOWN if (newlines_before is None and not is_first) else int(newlines_before or 0)
+    return _route(ctx.L.sgpu_fastq_ids_route_shard_dev, "fastq_ids_route_shard_dev", ctx, d_buf, n_buf, n_parts,
+                  (own_len, nb, int(is_first), int(is_last)))
+
+
+def fasta_ids_route_shard_dev(ctx: Context, d_buf, n_buf: int, own_len: int, is_first: bool, is_last: bool,
+                              n_parts: int) -> RouteResult:
+    """sgpu_fasta_ids_route_shard_dev: the same for a FASTA shard"""
+    return _route(ctx.L.sgpu_fasta_ids_route_shard_dev, "fasta_ids_route_shard_dev", ctx, d_buf, n_buf, n_parts,
+                  (own_len, int(is_first), int(is_last)))
+
+
+def idset_probe_lines_dev(ctx: Context, probe, d_lines, n: int, into):
+    """sgpu_idset_probe_lines_dev: "id\\n" lines (device uint8, 16-byte aligned) probed against `probe` (None: every line
+    is absent); the absent ids go into `into` (None: counted only).  Returns (lines, absent lines)."""
+    c = _lib.Counts()
+    rc = ctx.L.sgpu_idset_probe_lines_dev(ctx.h, probe.h if probe is not None else None,
+                                          C.c_void_p(d_lines.data_ptr()) if n else None, n,
+                                          into.h if into is not None else None, C.byref(c))
+    _check(rc, 0, "idset_probe_lines_dev")
+    return c.reads_in, c.difference
+
+
 def diff(ctx: Context, pairs, raise_on_error: bool = True):
     """ReadDifference::get_difference (utils.rs:250-285) over [(input, output), ...] host or device buffers
     -> (reads_in, reads_out, difference, IdSet of absent ids)"""

@@ -21,7 +21,7 @@ VARIANT = os.environ.get("SGPU_VARIANT", "")
 _SUFFIX = f"_{VARIANT}" if VARIANT else ""
 OBJDIR = os.path.join(HERE, "lib", "obj" + _SUFFIX)
 SO = os.path.join(LIBDIR, f"libscrubby_gpu{_SUFFIX}.so")
-SOURCES = ["scan.cu", "idset.cu", "idset_build.cu", "evidence.cu", "fastq_general.cu", "fasta_general.cu", "fastq_fused.cu", "capi.cu"]
+SOURCES = ["scan.cu", "idset.cu", "idset_build.cu", "evidence.cu", "fastq_general.cu", "fasta_general.cu", "fastq_fused.cu", "idset_route.cu", "capi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

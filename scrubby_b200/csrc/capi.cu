@@ -46,7 +46,7 @@ static sgpu_status clean_file(sgpu_ctx *c, const sgpu_idset *set, const Shard &s
 // the ids of a FASTQ shard, or of a whole FASTA file (sgpu_diff_dev, sgpu_fastq_ids_shard_dev); a first shard that
 // starts with '>' but is not the whole file is refused with SGPU_ERR_FASTA_UNSUPPORTED
 static sgpu_status ids_locked(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
-                              int want_absent, sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked,
+                              int want_absent, const SpanSink &sink, uint64_t *n_records, uint64_t *n_picked,
                               uint64_t *err_record, sgpu_counts *spec_out = nullptr) {
     *n_records = *n_picked = 0;
     if (s.is_first) {
@@ -56,10 +56,10 @@ static sgpu_status ids_locked(sgpu_ctx *c, const Shard &s, uint64_t newlines_bef
         if (f == Fmt::unknown) return SGPU_ERR_FASTQ_UNKNOWN_FORMAT;
         if (f == Fmt::fasta)
             return s.is_last && s.own_len == s.n
-                       ? fasta_ids_shard(c, s, probe, want_absent, into, n_records, n_picked, err_record)
+                       ? fasta_ids_shard(c, s, probe, want_absent, sink, n_records, n_picked, err_record)
                        : SGPU_ERR_FASTA_UNSUPPORTED;
     }
-    return fastq_ids_shard(c, s, newlines_before, probe, want_absent, into, n_records, n_picked, err_record, spec_out);
+    return fastq_ids_shard(c, s, newlines_before, probe, want_absent, sink, n_records, n_picked, err_record, spec_out);
 }
 
 void ctx_release(sgpu_ctx *c) {
@@ -610,6 +610,58 @@ static sgpu_status fasta_shard_head(sgpu_ctx *c, const Shard &s, bool on_device,
     return *empty || f == Fmt::fasta ? SGPU_OK : SGPU_ERR_INVALID_ARG;
 }
 
+}  // extern "C"
+
+// the ids entry points of both formats (context locked): the shard's ids go to `sink`; counts->reads_in += records,
+// counts->difference += picked records, error_record on a failure (FASTQ: the single-pass kernel's speculation counts)
+static sgpu_status fastq_ids_entry(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
+                                   const SpanSink &sink, sgpu_counts *counts) {
+    uint64_t n_rec = 0, n_pick = 0, err = 0;
+    sgpu_counts spec;
+    memset(&spec, 0, sizeof(spec));
+    sgpu_status rc = ids_locked(c, s, newlines_before, probe, probe != nullptr, sink, &n_rec, &n_pick, &err, &spec);
+    if (rc == SGPU_OK) {
+        counts->reads_in += n_rec;
+        counts->difference += n_pick;
+        counts->speculated = spec.speculated;
+        counts->own_newlines = spec.own_newlines;
+        counts->lead_newlines = spec.lead_newlines;
+    } else {
+        counts->error_record = err;
+    }
+    cudaStreamSynchronize(c->stream);
+    return rc;
+}
+
+static sgpu_status fasta_ids_entry(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, const SpanSink &sink,
+                                   sgpu_counts *counts) {
+    bool empty;
+    SGPU_TRY(fasta_shard_head(c, s, true, &empty));
+    if (empty) return SGPU_OK;
+    uint64_t n_rec = 0, n_pick = 0, err = 0;
+    sgpu_status rc = fasta_ids_shard(c, s, probe, probe != nullptr, sink, &n_rec, &n_pick, &err);
+    if (rc == SGPU_OK) {
+        counts->reads_in += n_rec;
+        counts->difference += n_pick;
+    } else {
+        counts->error_record = err;
+    }
+    cudaStreamSynchronize(c->stream);
+    return rc;
+}
+
+// the route sink of the route entry points: outputs zeroed before anything runs
+static bool route_args_ok(int n_parts, uint8_t *d_lines, size_t cap, size_t *n_lines, uint64_t *part_bytes,
+                          uint64_t *part_lines) {
+    if (!n_lines || !part_bytes || !part_lines || n_parts < 1 || n_parts > 64 || (cap && !d_lines)) return false;
+    *n_lines = 0;
+    memset(part_bytes, 0, (size_t)n_parts * sizeof(uint64_t));
+    memset(part_lines, 0, (size_t)n_parts * sizeof(uint64_t));
+    return true;
+}
+
+extern "C" {
+
 sgpu_status sgpu_clean_fasta_shard_dev(sgpu_ctx *c, const sgpu_idset *set, const uint8_t *d_in, size_t n_in,
                                        size_t own_len, int is_first, int is_last, int le_before, int reverse,
                                        uint8_t *d_out_w, size_t cap_w, size_t *n_w, uint8_t *d_out_o, size_t cap_o,
@@ -669,20 +721,7 @@ sgpu_status sgpu_fasta_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const
     if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    const Shard s{d_buf, n_buf, own_len, is_first, is_last};
-    bool empty;
-    SGPU_TRY(fasta_shard_head(c, s, true, &empty));
-    if (empty) return SGPU_OK;
-    uint64_t n_rec = 0, n_pick = 0, err = 0;
-    sgpu_status rc = fasta_ids_shard(c, s, probe, probe != nullptr, into, &n_rec, &n_pick, &err);
-    if (rc == SGPU_OK) {
-        counts->reads_in += n_rec;
-        counts->difference += n_pick;
-    } else {
-        counts->error_record = err;
-    }
-    cudaStreamSynchronize(c->stream);
-    return rc;
+    return fasta_ids_entry(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, probe, SpanSink{into, nullptr}, counts);
 }
 
 sgpu_status sgpu_diff_dev(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, const uint8_t *d_out, size_t n_out,
@@ -694,10 +733,10 @@ sgpu_status sgpu_diff_dev(sgpu_ctx *c, const uint8_t *d_in, size_t n_in, const u
     sgpu_idset *o_ids = nullptr;  // utils.rs:257 reads2_ids
     SGPU_TRY(idset_create(c, &o_ids));
     uint64_t n_rec = 0, n_pick = 0, err = 0;
-    sgpu_status rc = ids_locked(c, Shard{d_out, n_out, n_out, 1, 1}, 0, nullptr, 0, o_ids, &n_rec, &n_pick, &err);  // :259-267
+    sgpu_status rc = ids_locked(c, Shard{d_out, n_out, n_out, 1, 1}, 0, nullptr, 0, SpanSink{o_ids, nullptr}, &n_rec, &n_pick, &err);  // :259-267
     if (rc == SGPU_OK) {
         counts->reads_out += n_rec;
-        rc = ids_locked(c, Shard{d_in, n_in, n_in, 1, 1}, 0, o_ids, 1, *diff_ids, &n_rec, &n_pick, &err);  // :269-283
+        rc = ids_locked(c, Shard{d_in, n_in, n_in, 1, 1}, 0, o_ids, 1, SpanSink{*diff_ids, nullptr}, &n_rec, &n_pick, &err);  // :269-283
         if (rc == SGPU_OK) {
             counts->reads_in += n_rec;
             counts->difference += n_pick;
@@ -717,22 +756,8 @@ sgpu_status sgpu_fastq_ids_shard_dev(sgpu_ctx *c, const sgpu_idset *probe, const
     if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lk(c->mu);
     SGPU_CUDA(cudaSetDevice(c->device));
-    uint64_t n_rec = 0, n_pick = 0, err = 0;
-    sgpu_counts spec;
-    memset(&spec, 0, sizeof(spec));
-    sgpu_status rc = ids_locked(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, newlines_before, probe,
-                                probe != nullptr, into, &n_rec, &n_pick, &err, &spec);
-    if (rc == SGPU_OK) {
-        counts->reads_in += n_rec;
-        counts->difference += n_pick;
-        counts->speculated = spec.speculated;
-        counts->own_newlines = spec.own_newlines;
-        counts->lead_newlines = spec.lead_newlines;
-    } else {
-        counts->error_record = err;
-    }
-    cudaStreamSynchronize(c->stream);
-    return rc;
+    return fastq_ids_entry(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, newlines_before, probe,
+                           SpanSink{into, nullptr}, counts);
 }
 
 sgpu_status sgpu_diff(sgpu_ctx *c, const uint8_t *in, size_t n_in, const uint8_t *out, size_t n_out,
@@ -750,6 +775,39 @@ sgpu_status sgpu_diff(sgpu_ctx *c, const uint8_t *in, size_t n_in, const uint8_t
     }
     sgpu_status rc = sgpu_diff_dev(c, d_in.p, n_in, d_out.p, n_out, counts, diff_ids);
     cudaStreamSynchronize(c->stream);
+    return rc;
+}
+
+sgpu_status sgpu_fastq_ids_route_shard_dev(sgpu_ctx *c, const uint8_t *d_buf, size_t n_buf, size_t own_len,
+                                           uint64_t newlines_before, int is_first, int is_last, int n_parts,
+                                           uint8_t *d_lines, size_t cap, size_t *n_lines, uint64_t *part_bytes,
+                                           uint64_t *part_lines, sgpu_counts *counts) {
+    if (!c || !counts || (n_buf && !d_buf) || !fastq_shard_args_ok(n_buf, own_len, newlines_before, is_first, is_last, 0) ||
+        !route_args_ok(n_parts, d_lines, cap, n_lines, part_bytes, part_lines))
+        return SGPU_ERR_INVALID_ARG;
+    if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(c->mu);
+    SGPU_CUDA(cudaSetDevice(c->device));
+    RouteOut r{(uint32_t)n_parts, d_lines, cap, 0, part_bytes, part_lines};
+    const sgpu_status rc = fastq_ids_entry(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, newlines_before, nullptr,
+                                           SpanSink{nullptr, &r}, counts);
+    *n_lines = r.n_lines;
+    return rc;
+}
+
+sgpu_status sgpu_fasta_ids_route_shard_dev(sgpu_ctx *c, const uint8_t *d_buf, size_t n_buf, size_t own_len, int is_first,
+                                           int is_last, int n_parts, uint8_t *d_lines, size_t cap, size_t *n_lines,
+                                           uint64_t *part_bytes, uint64_t *part_lines, sgpu_counts *counts) {
+    if (!c || !counts || (n_buf && !d_buf) || !fasta_shard_args_ok(n_buf, own_len, is_last, -1, is_first) ||
+        !route_args_ok(n_parts, d_lines, cap, n_lines, part_bytes, part_lines))
+        return SGPU_ERR_INVALID_ARG;
+    if (n_buf && ((uintptr_t)d_buf & 15)) return SGPU_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(c->mu);
+    SGPU_CUDA(cudaSetDevice(c->device));
+    RouteOut r{(uint32_t)n_parts, d_lines, cap, 0, part_bytes, part_lines};
+    const sgpu_status rc = fasta_ids_entry(c, Shard{d_buf, n_buf, own_len, is_first, is_last}, nullptr,
+                                           SpanSink{nullptr, &r}, counts);
+    *n_lines = r.n_lines;
     return rc;
 }
 

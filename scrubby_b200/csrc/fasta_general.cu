@@ -334,7 +334,7 @@ sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s
 }
 
 // one loop of ReadDifference::get_difference (utils.rs:259-267 / 269-283) over the FASTA records a shard owns
-sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, sgpu_idset *into,
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, const SpanSink &sink,
                             uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record) {
     *n_records = *n_picked = 0;
     FaTables T;
@@ -354,7 +354,7 @@ sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe
     SGPU_TRY(read_u64s(c, T.scratch.p + 3, &picked, 1));
     *n_records = n_rec;
     *n_picked = picked;
-    if (into && picked) SGPU_TRY(idset_insert_spans(c, into, s.p, T.key_off.p, T.key_len.p, T.sel.p, (size_t)n_rec));
+    if (picked) SGPU_TRY(sink_spans(c, sink, s.p, T.key_off.p, T.key_len.p, T.sel.p, (size_t)n_rec));
     SGPU_CUDA(cudaStreamSynchronize(st));
     return SGPU_OK;
 }

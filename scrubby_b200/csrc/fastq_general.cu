@@ -265,7 +265,7 @@ sgpu_status clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s
 }
 
 sgpu_status fastq_ids_shard(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
-                            int want_absent, sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked,
+                            int want_absent, const SpanSink &sink, uint64_t *n_records, uint64_t *n_picked,
                             uint64_t *err_record, sgpu_counts *spec_out) {
     *n_records = *n_picked = 0;
     if (!s.is_first && (s.n == 0 || s.own_len == 0)) return SGPU_OK;
@@ -287,8 +287,9 @@ sgpu_status fastq_ids_shard(sgpu_ctx *c, const Shard &s, uint64_t newlines_befor
         if (used) {
             *n_records = ck.reads_in;
             *n_picked = ids.n_spans;
-            if (into && ids.n_spans)
-                SGPU_TRY(idset_insert_spans(c, into, s.p + ids.base, s_off.p, s_len.p, nullptr, (size_t)ids.n_spans));
+            if (ids.n_spans)  // (listed in tile completion order)
+                SGPU_TRY(sink_spans(c, sink, s.p + ids.base, s_off.p, s_len.p, nullptr, (size_t)ids.n_spans, false,
+                                    s.n - ids.base));
             return SGPU_OK;
         }
     }
@@ -318,7 +319,7 @@ sgpu_status fastq_ids_shard(sgpu_ctx *c, const Shard &s, uint64_t newlines_befor
     }
     *n_records = h[1];
     *n_picked = h[2];
-    if (into) SGPU_TRY(idset_insert_spans(c, into, s.p, key_off.p, key_len.p, sel.p, n_thr));
+    SGPU_TRY(sink_spans(c, sink, s.p, key_off.p, key_len.p, sel.p, n_thr));
     return SGPU_OK;
 }
 

@@ -139,6 +139,27 @@ static inline void clear_outputs(const Outs &out, sgpu_counts *counts) {
     if (out.n_o) *out.n_o = 0;
 }
 
+// Where an ids pass sends the id spans it selected: inserted into a set, or routed as "id\n" lines grouped by owner
+// partition (the hash-partitioned diff).
+struct RouteOut {
+    uint32_t n_parts;     // 1..64
+    uint8_t *lines;       // device
+    size_t cap;
+    size_t n_lines;       // out: bytes written (bytes needed with SGPU_ERR_CAPACITY)
+    uint64_t *part_bytes;  // out: host arrays of n_parts
+    uint64_t *part_lines;
+};
+struct SpanSink {
+    sgpu_idset *into;  // insert into this set (nullptr: count only) ...
+    RouteOut *route;   // ... unless this is set: route
+};
+
+// idset_route.cu: spans d_src[off[i] .. off[i]+len[i]) with sel[i] != 0 (sel nullptr: all) to the sink.  `in_order`:
+// the spans are listed in file order; otherwise (the single-pass kernel's list) routing sorts them by offset first,
+// so that lines keep file order inside a partition (`range`: the offsets lie in [0, range)).
+sgpu_status sink_spans(sgpu_ctx *c, const SpanSink &k, const uint8_t *d_src, const uint64_t *d_off, const uint32_t *d_len,
+                       const uint8_t *d_sel, size_t n, bool in_order = true, uint64_t range = 0);
+
 // fastq_general.cu: FastqCleaner::clean_reads and one loop of ReadDifference::get_difference over the FASTQ records a
 // shard owns (the contracts are sgpu_clean_fastq_shard_dev's and sgpu_fastq_ids_shard_dev's; a whole file is the shard
 // (n, n, newlines_before 0, first, last, crlf -1)).  The single-pass kernel runs when it takes the input, else the
@@ -149,7 +170,7 @@ static inline void clear_outputs(const Outs &out, sgpu_counts *counts) {
 sgpu_status clean_fastq_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint64_t newlines_before, int crlf,
                               int reverse, const Outs &out, sgpu_counts *counts, bool want_nl);
 sgpu_status fastq_ids_shard(sgpu_ctx *c, const Shard &s, uint64_t newlines_before, const sgpu_idset *probe,
-                            int want_absent, sgpu_idset *into, uint64_t *n_records, uint64_t *n_picked,
+                            int want_absent, const SpanSink &sink, uint64_t *n_records, uint64_t *n_picked,
                             uint64_t *err_record, sgpu_counts *spec_out);
 
 // fastq_fused.cu: the single-pass kernel over one FASTQ shard; *used = 0 when the input is not canonical (the caller
@@ -169,7 +190,7 @@ sgpu_status fused_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, uint
 // file is the shard (n, n, first, last)); the shard contract is sgpu_clean_fasta_shard_dev's
 sgpu_status clean_fasta_shard(sgpu_ctx *c, const sgpu_idset *set, const Shard &s, int le_before, int reverse,
                               const Outs &out, sgpu_counts *counts, int *le_own);
-sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, sgpu_idset *into,
+sgpu_status fasta_ids_shard(sgpu_ctx *c, const Shard &s, const sgpu_idset *probe, int want_absent, const SpanSink &sink,
                             uint64_t *n_records, uint64_t *n_picked, uint64_t *err_record);
 
 }  // namespace sgpu

@@ -161,6 +161,23 @@ __device__ __forceinline__ void key_image(const uint8_t *p, uint32_t len, uint64
     }
 }
 
+// Owner partition of a key among n_parts (1..64) in the hash-partitioned diff: route_owner(home, n_parts) with `home`
+// key_image()'s hash.  The set an owner builds from its keys takes the page from home's HIGH bits (home_page) and the
+// bucket from its low 8 bits, so the owner is drawn from a fixed bijective remix of home (xor, xorshift-multiply
+// rounds): a partition's keys still spread over every page of the owner's set.
+__device__ __forceinline__ uint64_t route_remix(uint64_t h) {
+    h ^= 0x2545F4914F6CDD1DULL;
+    h ^= h >> 30;
+    h *= 0xBF58476D1CE4E5B9ULL;
+    h ^= h >> 27;
+    h *= 0x94D049BB133111EBULL;
+    h ^= h >> 31;
+    return h;
+}
+__device__ __forceinline__ uint32_t route_owner(uint64_t home, uint32_t n_parts) {
+    return (uint32_t)__umul64hi(route_remix(home), (uint64_t)n_parts);
+}
+
 // home hash recomputed from a stored slot (rehash without touching key bytes)
 __device__ __forceinline__ uint64_t slot_home(uint64_t lo, uint64_t hi) {
     if ((lo & 0xFF) == 0x80) return mix64(lo);

@@ -112,6 +112,28 @@ class GpuOps:
     def set_ids(self, ids):
         return ids.sorted_ids()
 
+    def route_shard(self, d_buf, sh: Shard, newlines_before, n_parts):
+        """the ids of the shard's own records as "id\\n" lines grouped by owner partition -> (device uint8 tensor,
+        bytes per partition, records)"""
+        r = self.api.fastq_ids_route_shard_dev(self.ctx, d_buf, sh.buf_len, sh.own_len, newlines_before, sh.is_first,
+                                               sh.is_last, n_parts)
+        return r.lines, r.part_bytes, r.reads_in
+
+    def fasta_route_shard(self, d_buf, sh: Shard, n_parts):
+        r = self.api.fasta_ids_route_shard_dev(self.ctx, d_buf, sh.buf_len, sh.own_len, sh.is_first, sh.is_last, n_parts)
+        return r.lines, r.part_bytes, r.reads_in
+
+    def set_from_lines(self, lines):
+        """the set of the ids of "id\\n" lines (sgpu_idset_from_txt_dev: exact for read ids, see unite_sets)"""
+        return self.api.IdSet.from_txt(self.ctx, lines) if lines.numel() else self.api.IdSet.empty(self.ctx)
+
+    def probe_lines(self, probe, lines, into):
+        """-> (lines, lines absent from `probe`); the absent ids go into `into`"""
+        return self.api.idset_probe_lines_dev(self.ctx, probe, lines, lines.numel(), into)
+
+    def free_set(self, s):
+        s.free()
+
     def set_from_ids(self, id_list):
         return self.api.IdSet.from_ids(self.ctx, id_list)
 
@@ -237,27 +259,26 @@ class ShardedDiff:
     diff_ids: list      # sorted unique ids of the input records missing from their output file (every rank)
 
 
-def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo, fasta=False):
-    """one loop of ReadDifference::get_difference over one file, every rank on its own byte range; the set of the
-    rank's ids goes to `collect`; returns the (records, picked) totals of this rank.  A record longer than the halo
-    makes all ranks retry with a larger one.  FASTA shards need no newline counts."""
+def _file_sharded(ops, file_bytes, dist, halo, max_halo, fasta, run):
+    """one file, every rank on its own byte range: `run(d_buf, sh, newlines_before)` runs this rank's shard when it owns
+    bytes (newlines_before is None for FASTA: its shards need no newline counts) and its result is returned (None when
+    the rank owns nothing).  The statuses of all ranks are agreed before anyone returns: a record longer than the halo
+    makes all ranks retry with a larger one, any other failure ends every rank (_raise_collectively)."""
     world = dist.get_world_size() if dist is not None else 1
     rank = dist.get_rank() if dist is not None else 0
     n = len(file_bytes)
     while True:
         sh = plan_shards(n, world, halo)[rank]
         d_buf = ops.upload(file_bytes[sh.start : sh.start + sh.buf_len])
+        newlines_before = None
         if not fasta:
             own_nl = ops.count_newlines(d_buf, sh.own_len)
             counts = _all_gather_ints(dist, [own_nl], world)
             newlines_before = sum(c[0] for c in counts[:rank])
-        halo_short, rec, picked, failed = 0, 0, 0, None
-        scratch = ops.new_set()  # a retry must not leave ids of the failed attempt behind
+        halo_short, out, failed = 0, None, None
         try:
-            if sh.own_len and fasta:
-                rec, picked = ops.fasta_ids_shard(probe, d_buf, sh, scratch)
-            elif sh.own_len:
-                rec, picked = ops.ids_shard(probe, d_buf, sh, newlines_before, scratch)
+            if sh.own_len:
+                out = run(d_buf, sh, newlines_before)
         except Exception as e:  # SGPU_ERR_HALO == 21
             if getattr(e, "status", None) == 21:
                 halo_short = 1
@@ -270,8 +291,24 @@ def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo, 
                 raise RuntimeError("a record is longer than the maximum shard halo")
             halo = min(max_halo, halo * 8)
             continue
-        collect(scratch)
-        return rec, picked
+        return out
+
+
+def _ids_of_file_sharded(ops, file_bytes, dist, probe, collect, halo, max_halo, fasta=False):
+    """one loop of ReadDifference::get_difference over one file, every rank on its own byte range; the set of the
+    rank's ids goes to `collect`; returns the (records, picked) totals of this rank.  A record longer than the halo
+    makes all ranks retry with a larger one.  FASTA shards need no newline counts."""
+
+    def run(d_buf, sh, newlines_before):
+        scratch = ops.new_set()  # a retry must not leave ids of the failed attempt behind
+        if fasta:
+            return ops.fasta_ids_shard(probe, d_buf, sh, scratch), scratch
+        return ops.ids_shard(probe, d_buf, sh, newlines_before, scratch), scratch
+
+    out = _file_sharded(ops, file_bytes, dist, halo, max_halo, fasta, run)
+    (rec, picked), scratch = out if out is not None else ((0, 0), ops.new_set())
+    collect(scratch)
+    return rec, picked
 
 
 def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 << 30, fasta: bool = False) -> ShardedDiff:
@@ -311,6 +348,75 @@ def diff_sharded(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 <
             dist.all_gather_object(gathered, diff_local)
         ids = sorted(set(x for part in gathered for x in part))
     return ShardedDiff(sum(t[0] for t in tot), sum(t[1] for t in tot), sum(t[2] for t in tot), ids)
+
+
+def _route_file(ops, file_bytes, dist, world, halo, max_halo, fasta):
+    """this rank's byte range of one file routed: (lines grouped by owner rank, bytes per owner, records)"""
+
+    def run(d_buf, sh, newlines_before):
+        if fasta:
+            return ops.fasta_route_shard(d_buf, sh, world)
+        return ops.route_shard(d_buf, sh, newlines_before, world)
+
+    out = _file_sharded(ops, file_bytes, dist, halo, max_halo, fasta, run)
+    if out is None:  # owns nothing: sends nothing
+        import torch
+
+        return torch.empty(0, dtype=torch.uint8, device=getattr(ops, "device", "cpu")), [0] * world, 0
+    return out
+
+
+def _all_to_all_bytes(dist, buf, part_bytes):
+    """the byte exchange of the partitioned diff: `buf` holds this rank's bytes for rank 0, then for rank 1, ...
+    (part_bytes[r] each); returns the bytes every rank sent to this one, concatenated in rank order.  The sizes travel
+    first (an all-gather of the size rows), then one all_to_all_single (NCCL on device tensors, gloo on CPU tensors).
+    Without a process group it is a local copy."""
+    import torch
+
+    total = sum(part_bytes)
+    if dist is None:
+        return buf[:total].clone()
+    world, rank = dist.get_world_size(), dist.get_rank()
+    rows = _all_gather_ints(dist, list(part_bytes), world) if world > 1 else [list(part_bytes)]
+    recv = [row[rank] for row in rows]
+    out = torch.empty(sum(recv), dtype=torch.uint8, device=buf.device)
+    dist.all_to_all_single(out, buf[:total].contiguous(), recv, list(part_bytes))
+    return out
+
+
+def diff_partitioned(ops, pairs, dist=None, halo: int = 1 << 20, max_halo: int = 1 << 30,
+                     fasta: bool = False) -> ShardedDiff:
+    """ReadDifference::get_difference (utils.rs:250-285) across all ranks with the sets PARTITIONED by id instead of
+    replicated (diff_sharded's signature and result).  Every id has one owner rank, a pure function of its bytes
+    (route_owner in csrc/idset.cuh).  For each (input, output) pair: each rank routes the ids of its byte range of the
+    output file to their owners (one all_to_all of "id\\n" lines), the owner builds its part O_r of the output-id set
+    from what it received, then the input file's ids are routed the same way and the owner probes them against O_r:
+    it counts every line (a record) and every absent one, and inserts the absent ids into its part D_r of the global
+    diff set, which lives across pairs (the reference keeps one diff set; an id always lands on the same rank, so mates
+    and ranks are deduplicated there).  Per rank, set memory and set-build work are 1/world of diff_sharded's.  At the
+    end the counters are summed and the sorted dumps of the D_r (disjoint) are all-gathered and merged."""
+    import heapq
+
+    world = dist.get_world_size() if dist is not None else 1
+    reads_in = reads_out = difference = 0
+    d_set = ops.new_set()
+    for fin, fout in pairs:
+        lines, parts, rec_out = _route_file(ops, fout, dist, world, halo, max_halo, fasta)
+        o_set = ops.set_from_lines(_all_to_all_bytes(dist, lines, parts))
+        lines, parts, _ = _route_file(ops, fin, dist, world, halo, max_halo, fasta)
+        n_lines, absent = ops.probe_lines(o_set, _all_to_all_bytes(dist, lines, parts), d_set)
+        ops.free_set(o_set)
+        reads_out += rec_out
+        reads_in += n_lines
+        difference += absent
+    tot = _all_gather_ints(dist, [reads_in, reads_out, difference], world)
+    mine = ops.set_ids(d_set)
+    gathered = [mine]
+    if world > 1:
+        gathered = [None] * world
+        dist.all_gather_object(gathered, mine)
+    return ShardedDiff(sum(t[0] for t in tot), sum(t[1] for t in tot), sum(t[2] for t in tot),
+                       list(heapq.merge(*gathered)))
 
 
 class ShardError(RuntimeError):
