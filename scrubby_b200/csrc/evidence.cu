@@ -1,15 +1,18 @@
 // evidence.cu -- alignment / classifier evidence -> read-id set.
 //
-//   paf_parse_kernel + paf_segment_kernel  replace ReadAlignment::from_paf (alignment.rs:84-114),
-//       PafRecord::from_str (:244-263), query_aligned_length / query_coverage (:265-275) and the
-//       duplicate loop at cleaner.rs:669-678.  The per-read aggregation that is bit-exact with the
-//       reference is a segmented logical OR of per-record predicates over runs of adjacent equal
-//       qnames (SURVEY F9), NOT a sum of aligned lengths.
-//   txt_lines_kernel                        replaces ReadAlignment::from_txt (alignment.rs:60-82).
-//   reads_parse_kernel                      replaces get_taxid_reads_kraken / _metabuli
-//       (classifier.rs:270-290, 308-328) with KrakenReadRecord / MetabuliReadRecord::from_str
-//       (:401-419, :497-517); taxid membership is a bitmap lookup for canonical decimal taxids and
-//       a byte compare against the (normally empty) list of non-canonical taxid strings.
+// PAF, TXT id lists and Kraken2 / Metabuli per-read lines take one of two kernels with the same per-line rules:
+//   lines_tile_kernel     one CTA per 16 KiB tile, no newline index (the normal case);
+//   lines_indexed_kernel  one thread per line over a newline index: inputs with a tile too dense for the tile kernel,
+//                         and sgpu_ctx_set_mode(1).
+// Both decide a line with the same scanners; the tile kernel's ASCII fast path shares their decision helpers:
+//   paf_line_scan   replaces ReadAlignment::from_paf (alignment.rs:84-114), PafRecord::from_str (:244-263) and
+//       query_aligned_length / query_coverage (:265-275, alignment_passes).  Every passing record offers its qname and
+//       the set makes the per-read aggregation (the duplicate loop at cleaner.rs:669-678): a logical OR of per-record
+//       predicates (SURVEY F9), NOT a sum of aligned lengths.
+//   evidence_line   replaces ReadAlignment::from_txt (alignment.rs:60-82) and get_taxid_reads_kraken / _metabuli
+//       (classifier.rs:270-290, 308-328) with KrakenReadRecord / MetabuliReadRecord::from_str (:401-419, :497-517,
+//       reads_key); taxid membership is a bitmap lookup for canonical decimal taxids and a byte compare against the
+//       (normally empty) list of non-canonical taxid strings.
 // Lines follow std::io::BufRead::lines: split on '\n', one '\r' stripped before it, UTF-8 checked.
 #include <string>
 #include <vector>
@@ -41,103 +44,17 @@ __device__ __forceinline__ bool line_span(const LineParams &P, uint64_t i, uint6
     return true;
 }
 
-// BufRead::lines: validates UTF-8 (InvalidData otherwise) and strips "\n" / "\r\n"
-__device__ __forceinline__ bool line_content(const LineParams &P, uint64_t i, uint64_t s, uint64_t *e, bool *high) {
-    const uint8_t *in = P.in;
-    // any byte with its high bit set?  (bytes up to a 4-byte boundary, aligned words, tail bytes)
-    uint32_t acc = 0;
-    uint64_t k = s;
-    const uint64_t end = *e;
-    while (k < end && ((uintptr_t)(in + k) & 3)) acc |= in[k++];
-    for (; k + 4 <= end; k += 4) acc |= *reinterpret_cast<const uint32_t *>(in + k);
-    while (k < end) acc |= in[k++];
-    const bool h = (acc & 0x80808080u) != 0;
-    *high = h;
-    if (h && !utf8_valid(in + s, *e - s)) return false;
-    if (i < P.n_nl && *e > s && in[*e - 1] == '\r') (*e)--;
-    return true;
-}
-
 struct PafParams {
     uint64_t min_len;
     double min_cov;
     uint32_t min_mapq;
 };
 
-__global__ void __launch_bounds__(128)
-    paf_parse_kernel(LineParams P, PafParams F, uint64_t n_lines, uint64_t *key_off, uint32_t *key_len, uint8_t *pass,
-                     uint8_t *head, unsigned long long *err_word) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lines) return;
-    uint64_t s, e;
-    uint8_t ok = 0, hd = 1;
-    uint64_t koff = 0;
-    uint32_t klen = 0;
-    if (line_span(P, i, &s, &e)) {
-        bool high;
-        if (!line_content(P, i, s, &e, &high)) {
-            report_error(err_word, i, SGPU_ERR_IO);
-        } else {
-            const uint8_t *in = P.in;
-            int f = 0, code = 0;
-            uint64_t fs = s, qlen = 0, qstart = 0, qend = 0, mapq = 0;
-            for (uint64_t pos = s; pos <= e && f < 12; pos++) {
-                if (pos == e || in[pos] == '\t') {
-                    uint64_t v = 0;
-                    // columns 2,3,4,7,8,9,10,11 as u64/usize, 12 as u8 (alignment.rs:248-259)
-                    bool is_int = (f >= 1 && f <= 3) || (f >= 6 && f <= 11);
-                    if (is_int && !parse_uint(in + fs, pos - fs, f == 11 ? 255ull : ~0ull, &v)) {
-                        code = SGPU_ERR_PAF_INTEGER;
-                        break;
-                    }
-                    if (f == 0) {
-                        koff = fs;
-                        klen = (uint32_t)(pos - fs);
-                    } else if (f == 1) qlen = v;
-                    else if (f == 2) qstart = v;
-                    else if (f == 3) qend = v;
-                    else if (f == 11) mapq = v;
-                    f++;
-                    fs = pos + 1;
-                }
-            }
-            if (!code && f < 12) code = SGPU_ERR_WOULD_PANIC;  // fields[f] out of bounds
-            if (code) {
-                report_error(err_word, i, code);
-            } else {
-                uint64_t alen = qend - qstart;  // usize subtraction wraps in release builds
-                double cov = qlen == 0 ? 0.0 : __ull2double_rn(alen) / __ull2double_rn(qlen);
-                ok = ((alen >= F.min_len || cov >= F.min_cov) && mapq >= F.min_mapq) ? 1 : 0;
-                // run head: qname differs from the previous line's first column
-                if (i > 0) {
-                    uint64_t ps = i >= 2 ? P.nlpos[i - 2] + 1 : 0;
-                    uint64_t pe = P.nlpos[i - 1];
-                    bool same = true;
-                    uint32_t k = 0;
-                    for (; k < klen && same; k++) same = (ps + k < pe) && in[ps + k] == in[koff + k];
-                    if (same) same = (ps + klen == pe) || in[ps + klen] == '\t' ||
-                                     (ps + klen + 1 == pe && in[ps + klen] == '\r');
-                    hd = same ? 0 : 1;
-                }
-            }
-        }
-    }
-    key_off[i] = koff;
-    key_len[i] = klen;
-    pass[i] = ok;
-    head[i] = hd;
-}
-
-// segmented OR over runs of adjacent equal qnames: one candidate per run
-__global__ void paf_segment_kernel(const uint8_t *pass, const uint8_t *head, uint64_t n_lines, uint8_t *sel) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lines) return;
-    uint8_t any = 0;
-    if (head[i]) {
-        any = pass[i];
-        for (uint64_t j = i + 1; j < n_lines && !head[j] && !any; j++) any |= pass[j];
-    }
-    sel[i] = any;
+// the per-record predicate of PAF, SAM and BAM (alignment.rs:102-104, :265-275): aligned length or query coverage,
+// and mapping quality.  The u32 lengths of SAM and BAM convert to double exactly.
+__device__ __forceinline__ bool alignment_passes(const PafParams &F, uint64_t alen, uint64_t qlen, uint64_t mapq) {
+    const double cov = qlen == 0 ? 0.0 : __ull2double_rn(alen) / __ull2double_rn(qlen);
+    return (alen >= F.min_len || cov >= F.min_cov) && mapq >= F.min_mapq;
 }
 
 // ------------------------------------------------------------------ SAM (text) records
@@ -293,8 +210,7 @@ __global__ void __launch_bounds__(128)
                                                               idset_contains(refs, in + fs[2], (uint32_t)FLEN(2))));
                         const bool unmapped = (flag & 4u) || rname_star || !declared || p < 1;
                         if (!unmapped) {
-                            const double cov = qlen == 0 ? 0.0 : (double)qalen / (double)qlen;
-                            ok = (((uint64_t)qalen >= F.min_len || cov >= F.min_cov) && (uint32_t)mapq >= F.min_mapq) ? 1 : 0;
+                            ok = alignment_passes(F, qalen, qlen, (uint32_t)mapq) ? 1 : 0;
                             koff = fs[0];
                             klen = (uint32_t)FLEN(0);
                         }
@@ -397,34 +313,9 @@ __global__ void __launch_bounds__(128)
                 if ((v & 15u) <= 1u) qalen += v >> 4;  // M and I
             }
             const uint32_t qlen = (uint32_t)l_seq;
-            const double cov = qlen == 0 ? 0.0 : (double)qalen / (double)qlen;
-            ok = (((uint64_t)qalen >= F.min_len || cov >= F.min_cov) && mapq >= F.min_mapq) ? 1 : 0;
+            ok = alignment_passes(F, qalen, qlen, mapq) ? 1 : 0;
             koff = (uint64_t)(name - in);
             klen = qn;
-        }
-    }
-    key_off[i] = koff;
-    key_len[i] = klen;
-    sel[i] = ok;
-}
-
-__global__ void __launch_bounds__(128)
-    txt_lines_kernel(LineParams P, uint64_t n_lines, uint64_t *key_off, uint32_t *key_len, uint8_t *sel,
-                     unsigned long long *err_word) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lines) return;
-    uint64_t s, e;
-    uint8_t ok = 0;
-    uint64_t koff = 0;
-    uint32_t klen = 0;
-    if (line_span(P, i, &s, &e)) {
-        bool high;
-        if (!line_content(P, i, s, &e, &high)) {
-            report_error(err_word, i, SGPU_ERR_IO);
-        } else {
-            ok = 1;
-            koff = s;
-            klen = (uint32_t)(e - s);
         }
     }
     key_off[i] = koff;
@@ -457,70 +348,33 @@ __device__ __forceinline__ bool taxid_member(const TaxSet &T, const uint8_t *s, 
     return false;
 }
 
-__global__ void __launch_bounds__(128)
-    reads_parse_kernel(LineParams P, TaxSet T, int need_fields, uint64_t n_lines, uint64_t *key_off, uint32_t *key_len,
-                       uint8_t *sel, unsigned long long *err_word) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_lines) return;
-    uint64_t s, e;
-    uint8_t ok = 0;
-    uint64_t koff = 0;
-    uint32_t klen = 0;
-    if (line_span(P, i, &s, &e)) {
-        bool high;
-        if (!line_content(P, i, s, &e, &high)) {
-            report_error(err_word, i, SGPU_ERR_IO);
-        } else {
-            const uint8_t *in = P.in;
-            int f = 0;
-            uint64_t fs = s, f1s = 0, f1e = 0, f2s = 0, f2e = 0;
-            for (uint64_t pos = s; pos <= e; pos++) {
-                if (pos == e || in[pos] == '\t') {
-                    if (f == 1) { f1s = fs; f1e = pos; }
-                    if (f == 2) { f2s = fs; f2e = pos; }
-                    f++;
-                    fs = pos + 1;
-                    if (f >= need_fields) break;
-                }
-            }
-            if (f < need_fields) {
-                report_error(err_word, i, SGPU_ERR_WOULD_PANIC);  // classifier.rs:412-415 / :508-513
-            } else {
-                // str::trim (Unicode White_Space) on read id and taxid
-                if (high) {
-                    size_t b, t;
-                    utf8_trim(in + f1s, f1e - f1s, &b, &t);
-                    f1e = f1s + t;
-                    f1s += b;
-                    utf8_trim(in + f2s, f2e - f2s, &b, &t);
-                    f2e = f2s + t;
-                    f2s += b;
-                } else {
-                    while (f1s < f1e && is_ws_ascii(in[f1s])) f1s++;
-                    while (f1e > f1s && is_ws_ascii(in[f1e - 1])) f1e--;
-                    while (f2s < f2e && is_ws_ascii(in[f2s])) f2s++;
-                    while (f2e > f2s && is_ws_ascii(in[f2e - 1])) f2e--;
-                }
-                if (taxid_member(T, in + f2s, (uint32_t)(f2e - f2s))) {
-                    ok = 1;
-                    koff = f1s;
-                    klen = (uint32_t)(f1e - f1s);
-                }
-            }
-        }
+// str::trim on the read id f1 and the taxid f2 (Unicode White_Space if the line has a non-ASCII byte, ASCII otherwise),
+// then the taxid's membership: true if the line selects its read, whose id is [*k_begin, *k_begin + *k_len) of f1
+__device__ __forceinline__ bool reads_key(const uint8_t *f1, uint64_t n1, const uint8_t *f2, uint64_t n2, bool high,
+                                          const TaxSet &T, uint64_t *k_begin, uint32_t *k_len) {
+    size_t b1 = 0, e1 = n1, b2 = 0, e2 = n2;
+    if (high) {
+        utf8_trim(f1, n1, &b1, &e1);
+        utf8_trim(f2, n2, &b2, &e2);
+    } else {
+        while (b1 < e1 && is_ws_ascii(f1[b1])) b1++;
+        while (e1 > b1 && is_ws_ascii(f1[e1 - 1])) e1--;
+        while (b2 < e2 && is_ws_ascii(f2[b2])) b2++;
+        while (e2 > b2 && is_ws_ascii(f2[e2 - 1])) e2--;
     }
-    key_off[i] = koff;
-    key_len[i] = klen;
-    sel[i] = ok;
+    if (!taxid_member(T, f2 + b2, (uint32_t)(e2 - b2))) return false;
+    *k_begin = b1;
+    *k_len = (uint32_t)(e1 - b1);
+    return true;
 }
 
-// ------------------------------------------------------------------ tile kernel for order-free evidence
-// Kraken2 / Metabuli per-read lines and TXT id lists do not need a global line index: a line is decided on
-// its own and the set does not care about insertion order.  One CTA per 16 KiB tile: 16-byte loads -> '\n'
-// masks -> the tile's newline positions in shared memory -> one thread per line that STARTS in the tile
-// (it reads on past the tile's end if the line does) -> selected (offset, length) spans compacted into a
-// candidate list with one global atomic per CTA.  Replaces nl_count + scan + nl_emit + reads_parse_kernel /
-// txt_lines_kernel (same per-line semantics); PAF keeps the indexed path (its segmented OR needs line order).
+// ------------------------------------------------------------------ tile kernel
+// A PAF record, a TXT id or a Kraken2 / Metabuli line is decided on its own and the set does not care about insertion
+// order (PAF included: every passing record offers its qname and the set makes the per-read OR), so no global line
+// index is needed.  One CTA per 16 KiB tile: 16-byte loads -> '\n' masks -> the tile's newline positions in shared
+// memory -> one thread per line that STARTS in the tile (it reads on past the tile's end if the line does) -> selected
+// (offset, length) spans compacted into a candidate list with one global atomic per CTA.  A tile denser than LT_LMAX
+// lines or LT_SMAX separators sends the buffer to lines_indexed_kernel, which decides each line with the same scanners.
 constexpr int LT_NT = 256, LT_FC = 4, LT_TILE = LT_NT * LT_FC * 16, LT_LMAX = 2048, LT_HALO = 1024, LT_SMAX = 5120;
 
 struct TileOut {
@@ -538,16 +392,19 @@ struct TileOut {
     int not_last;                 // the buffer does not end at the end of the file
 };
 
-// one line [s, e_raw) of the buffer (e_raw = position of its '\n', or n for an unterminated last line):
-// returns 1 and the key span if the line offers a key, 0 if not, and reports errors.
-// One pass over the line's aligned 4-byte words finds the high-bit bytes (UTF-8 screening) and the tabs.
+// The scanners decide one line [s, e_raw) of the buffer (e_raw = position of its '\n', or n for an unterminated last
+// line) with BufRead::lines semantics (UTF-8 check, "\r\n" stripped).  They return 1 and the key span if the line offers
+// a key, 0 if not, and set *err to the line's status code (0: none); the caller reports it in its own unit.
+
+// TXT (mode 1) and Kraken2 / Metabuli (mode 0) lines.  One pass over the line's aligned 4-byte words finds the high-bit
+// bytes (UTF-8 screening) and the tabs.
 __device__ __forceinline__ int evidence_line(const uint8_t *in, uint64_t s, uint64_t e_raw, bool has_nl, int mode,
-                                             const TaxSet &T, int need_fields, uint64_t *koff, uint32_t *klen,
-                                             unsigned long long *err_word, uint64_t err_base) {
+                                             const TaxSet &T, int need_fields, uint64_t *koff, uint32_t *klen, int *err) {
     uint64_t e = e_raw;
     uint32_t acc = 0;
     int f = 0;  // fields closed so far
     uint64_t fs = s, f1s = 0, f1e = 0, f2s = 0, f2e = 0;
+    *err = 0;
     {
         const uintptr_t base = (uintptr_t)in;
         uint64_t w0 = (base + s) & ~(uintptr_t)3;         // address of the first word
@@ -576,7 +433,7 @@ __device__ __forceinline__ int evidence_line(const uint8_t *in, uint64_t s, uint
     // BufRead::lines: UTF-8 check, strip "\n" / "\r\n"
     const bool high = (acc & 0x80808080u) != 0;
     if (high && !utf8_valid(in + s, e - s)) {
-        report_error(err_word, err_base + s, SGPU_ERR_IO);
+        *err = SGPU_ERR_IO;
         return 0;
     }
     if (has_nl && e > s && in[e - 1] == '\r') e--;
@@ -591,30 +448,14 @@ __device__ __forceinline__ int evidence_line(const uint8_t *in, uint64_t s, uint
         f++;
     }
     if (f < need_fields) {
-        report_error(err_word, err_base + s, SGPU_ERR_WOULD_PANIC);  // classifier.rs:412-415 / :508-513
+        *err = SGPU_ERR_WOULD_PANIC;  // classifier.rs:412-415 / :508-513
         return 0;
     }
     // a field that ended at the raw end of a "\r\n" line: the '\r' was stripped by lines()
     if (f1e > e) f1e = e;
     if (f2e > e) f2e = e;
-    // str::trim (Unicode White_Space) on read id and taxid
-    if (high) {
-        size_t b, t;
-        utf8_trim(in + f1s, f1e - f1s, &b, &t);
-        f1e = f1s + t;
-        f1s += b;
-        utf8_trim(in + f2s, f2e - f2s, &b, &t);
-        f2e = f2s + t;
-        f2s += b;
-    } else {
-        while (f1s < f1e && is_ws_ascii(in[f1s])) f1s++;
-        while (f1e > f1s && is_ws_ascii(in[f1e - 1])) f1e--;
-        while (f2s < f2e && is_ws_ascii(in[f2s])) f2s++;
-        while (f2e > f2s && is_ws_ascii(in[f2e - 1])) f2e--;
-    }
-    if (!taxid_member(T, in + f2s, (uint32_t)(f2e - f2s))) return 0;
-    *koff = f1s;
-    *klen = (uint32_t)(f1e - f1s);
+    if (!reads_key(in + f1s, f1e - f1s, in + f2s, f2e - f2s, high, T, koff, klen)) return 0;
+    *koff += f1s;
     return 1;
 }
 
@@ -633,13 +474,19 @@ __device__ __forceinline__ bool parse_uint_short(const uint8_t *p, uint32_t n, u
     return true;
 }
 
-// one PAF line by scanning (non-ASCII tiles, lines that leave the halo, lines with fewer than 12 fields):
-// BufRead::lines semantics (UTF-8 check, "\r\n" stripped), then the fields in column order
+// PAF records (the tile kernel's fast path does not take non-ASCII tiles, lines that leave the halo, lines with fewer
+// than 12 fields): the fields in column order, the first bad integer is the error
 __device__ __noinline__ int paf_line_scan(const uint8_t *in, uint64_t s, uint64_t e_raw, bool has_nl, const PafParams &F,
-                                          uint64_t *koff, uint32_t *klen, unsigned long long *err_word) {
+                                          uint64_t *koff, uint32_t *klen, int *err) {
     uint64_t e = e_raw;
-    if (!utf8_valid(in + s, e - s)) {
-        report_error(err_word, s, SGPU_ERR_IO);
+    // only a line with a high-bit byte can fail the UTF-8 check: screen it in aligned 4-byte words first
+    uint32_t acc = 0;
+    uint64_t k = s;
+    while (k < e && ((uintptr_t)(in + k) & 3)) acc |= in[k++];
+    for (; k + 4 <= e; k += 4) acc |= *reinterpret_cast<const uint32_t *>(in + k);
+    while (k < e) acc |= in[k++];
+    if ((acc & 0x80808080u) && !utf8_valid(in + s, e - s)) {
+        *err = SGPU_ERR_IO;
         return 0;
     }
     if (has_nl && e > s && in[e - 1] == '\r') e--;
@@ -663,13 +510,9 @@ __device__ __noinline__ int paf_line_scan(const uint8_t *in, uint64_t s, uint64_
         }
     }
     if (!code && f < 12) code = SGPU_ERR_WOULD_PANIC;  // fields[f] out of bounds (alignment.rs:248-259)
-    if (code) {
-        report_error(err_word, s, code);
-        return 0;
-    }
-    const uint64_t alen = qend - qstart;
-    const double cov = qlen == 0 ? 0.0 : __ull2double_rn(alen) / __ull2double_rn(qlen);
-    if (!((alen >= F.min_len || cov >= F.min_cov) && mapq >= F.min_mapq)) return 0;
+    *err = code;
+    // usize subtraction wraps in release builds
+    if (code || !alignment_passes(F, qend - qstart, qlen, mapq)) return 0;
     *koff = s;
     *klen = (uint32_t)(k_end - s);
     return 1;
@@ -685,7 +528,7 @@ __device__ __forceinline__ void sep_masks16(uint4 v, bool want_tabs, uint32_t *m
 // The tile kernel proper.  P1 turns every 16-byte chunk of the tile (+ halo) into '\n' / '\t' masks and
 // scatters the separator positions, in order, into one list (bit 15 = newline) plus the list index of every
 // newline; a line's fields are then consecutive list entries -- no per-line scanning.  Tiles with a
-// non-ASCII byte and lines that run past the halo take the scanning routine (evidence_line) instead.
+// non-ASCII byte and lines that run past the halo take the scanners (evidence_line, paf_line_scan) instead.
 __global__ void __launch_bounds__(LT_NT)
     lines_tile_kernel(const uint8_t *in, uint64_t n, TaxSet T, int need_fields, int mode, PafParams F, TileOut O) {
     constexpr int NWARP = LT_NT / 32;
@@ -896,14 +739,10 @@ __global__ void __launch_bounds__(LT_NT)
                         }
                         if (code) {
                             report_error(O.err_word, g0 + s, code);
-                        } else {
-                            const uint64_t alen = qend - qstart;  // usize subtraction wraps in release builds
-                            const double cov = qlen == 0 ? 0.0 : __ull2double_rn(alen) / __ull2double_rn(qlen);
-                            if ((alen >= F.min_len || cov >= F.min_cov) && mapq >= F.min_mapq) {
-                                sel = 1;
-                                koff = g0 + s;
-                                klen = name_end - s;
-                            }
+                        } else if (alignment_passes(F, qend - qstart, qlen, mapq)) {  // (usize subtraction wraps)
+                            sel = 1;
+                            koff = g0 + s;
+                            klen = name_end - s;
                         }
                     }
                 } else if (fast) {
@@ -915,17 +754,11 @@ __global__ void __launch_bounds__(LT_NT)
                         if (any_nl & 0x8000u) {
                             report_error(O.err_word, g0 + s, SGPU_ERR_WOULD_PANIC);  // classifier.rs:412-415 / :508-513
                         } else {
-                            uint32_t f1s = ((uint32_t)seps[i0 + 1]) + 1u, f1e = seps[i0 + 2];
-                            uint32_t f2s = f1e + 1u, f2e = seps[i0 + 3];
-                            // str::trim on read id and taxid (ASCII tile)
-                            while (f1s < f1e && is_ws_ascii(tile[f1s])) f1s++;
-                            while (f1e > f1s && is_ws_ascii(tile[f1e - 1])) f1e--;
-                            while (f2s < f2e && is_ws_ascii(tile[f2s])) f2s++;
-                            while (f2e > f2s && is_ws_ascii(tile[f2e - 1])) f2e--;
-                            if (taxid_member(T, tile + f2s, f2e - f2s)) {
+                            const uint32_t f1s = ((uint32_t)seps[i0 + 1]) + 1u, f1e = seps[i0 + 2];
+                            const uint32_t f2s = f1e + 1u, f2e = seps[i0 + 3];
+                            if (reads_key(tile + f1s, f1e - f1s, tile + f2s, f2e - f2s, false, T, &koff, &klen)) {
                                 sel = 1;
-                                koff = g0 + f1s;
-                                klen = f1e - f1s;
+                                koff += g0 + f1s;
                             }
                         }
                     } else {
@@ -936,9 +769,11 @@ __global__ void __launch_bounds__(LT_NT)
                     // scanning routine over the buffer: non-ASCII tile, or a line that leaves the halo
                     uint64_t e = g0 + s;
                     while (e < n && in[e] != '\n') e++;
-                    if (e == n && O.not_last) report_error(O.err_word, g0 + s, SGPU_ERR_HALO);  // the halo is too short
-                    else if (mode == 2) sel = paf_line_scan(in, g0 + s, e, e < n, F, &koff, &klen, O.err_word);
-                    else sel = evidence_line(in, g0 + s, e, e < n, mode, T, need_fields, &koff, &klen, O.err_word, 0);
+                    int code = 0;
+                    if (e == n && O.not_last) code = SGPU_ERR_HALO;  // the halo is too short
+                    else if (mode == 2) sel = paf_line_scan(in, g0 + s, e, e < n, F, &koff, &klen, &code);
+                    else sel = evidence_line(in, g0 + s, e, e < n, mode, T, need_fields, &koff, &klen, &code);
+                    if (code) report_error(O.err_word, g0 + s, code);
                 }
             }
         }
@@ -973,6 +808,26 @@ __global__ void __launch_bounds__(LT_NT)
     }
 }
 
+// The same formats one thread per line over the newline index, with the tile kernel's scanners; every line writes its
+// key span and selection, and an error is reported at the line's index.
+__global__ void __launch_bounds__(128)
+    lines_indexed_kernel(LineParams P, TaxSet T, int need_fields, int mode, PafParams F, uint64_t n_lines,
+                         uint64_t *key_off, uint32_t *key_len, uint8_t *sel, unsigned long long *err_word) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lines) return;
+    uint64_t s, e, koff = 0;
+    uint32_t klen = 0;
+    int ok = 0, code = 0;
+    if (line_span(P, i, &s, &e)) {
+        if (mode == 2) ok = paf_line_scan(P.in, s, e, i < P.n_nl, F, &koff, &klen, &code);
+        else ok = evidence_line(P.in, s, e, i < P.n_nl, mode, T, need_fields, &koff, &klen, &code);
+        if (code) report_error(err_word, i, code);
+    }
+    key_off[i] = koff;
+    key_len[i] = klen;
+    sel[i] = (uint8_t)ok;
+}
+
 enum EvidenceKind { EV_PAF, EV_TXT, EV_READS, EV_SAM };
 
 static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t *d_buf, size_t n, PafParams F,
@@ -984,21 +839,26 @@ static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t
         *out = set;
         return SGPU_OK;
     }
+    if ((uintptr_t)d_buf & 15) {  // both kernels and the newline index load the buffer in aligned 16-byte words
+        sgpu_idset_free(set);
+        return SGPU_ERR_INVALID_ARG;
+    }
     sgpu_status rc = SGPU_OK;
     bool done = false;
+    const int mode = kind == EV_TXT ? 1 : kind == EV_PAF ? 2 : 0;  // (the format argument of both kernels)
+    const TaxSet none{nullptr, 0, nullptr, nullptr, 0};
     // The stream may still be busy with what produced d_buf (an NCCL all-gather of the evidence shards, an upload): wait
     // here, BEFORE the scratch and the table are taken from the stream-ordered pool.  The first host round trip of the
     // build is microseconds away anyway, and allocating while the previous set's frees are still queued behind that work
     // makes the pool grow instead of reusing them -- with peer access enabled (NCCL) growing costs milliseconds
     // (measured at 2 GPUs: set build 10.3 ms -> 5.0 ms per step).
     SGPU_CUDA(cudaStreamSynchronize(st));
-    if (c->mode == 0 && (kind == EV_TXT || kind == EV_READS || kind == EV_PAF) && ((uintptr_t)d_buf & 15) == 0) {
+    if (c->mode == 0 && kind != EV_SAM) {
         // ---- order-free evidence: the tile kernel, no newline index
         do {
             DevBuf<uint64_t> cand_off, ctr;
             DevBuf<uint32_t> cand_len;
             uint64_t cap = (kind == EV_TXT ? n / 8 : n / 32) + 4096;  // (more candidates than room: one retry with the count)
-            const TaxSet none{nullptr, 0, nullptr, nullptr, 0};
             for (int attempt = 0; attempt < 2 && rc == SGPU_OK; attempt++) {
                 if ((rc = cand_off.alloc(cap, st)) != SGPU_OK) break;
                 if ((rc = cand_len.alloc(cap, st)) != SGPU_OK) break;
@@ -1009,7 +869,7 @@ static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t
                 TileOut O{cand_off.p, cand_len.p, cap, (unsigned long long *)ctr.p, (unsigned long long *)ctr.p + 1,
                           (unsigned long long *)ctr.p + 2, (unsigned long long *)ctr.p + 3, 0ull, ~0ull, 0};
                 lines_tile_kernel<<<(unsigned)ceil_div(n, (size_t)LT_TILE), LT_NT, 0, st>>>(
-                    d_buf, (uint64_t)n, T ? *T : none, need_fields, kind == EV_TXT ? 1 : kind == EV_PAF ? 2 : 0, F, O);
+                    d_buf, (uint64_t)n, T ? *T : none, need_fields, mode, F, O);
                 SGPU_LAUNCH(c);
                 uint64_t h[6];
                 if ((rc = read_u64s(c, ctr.p, h, 6)) != SGPU_OK) break;
@@ -1043,7 +903,7 @@ static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t
     if (!done && rc == SGPU_OK) do {
         DevBuf<uint64_t> nlpos, key_off, errw;
         DevBuf<uint32_t> key_len;
-        DevBuf<uint8_t> sel, pass, head;
+        DevBuf<uint8_t> sel;
         uint64_t n_nl = 0;
         if ((rc = index_newlines(c, d_buf, n, nlpos, &n_nl)) != SGPU_OK) break;
         uint64_t n_lines = n_nl + 1;  // the last thread handles an unterminated final line (if any)
@@ -1054,15 +914,7 @@ static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t
         if ((rc = errw.alloc(1, st)) != SGPU_OK) break;
         cudaMemsetAsync(errw.p, 0xFF, 8, st);
         unsigned grid = (unsigned)ceil_div(n_lines, 128);
-        if (kind == EV_PAF) {
-            if ((rc = pass.alloc(n_lines, st)) != SGPU_OK) break;
-            if ((rc = head.alloc(n_lines, st)) != SGPU_OK) break;
-            paf_parse_kernel<<<grid, 128, 0, st>>>(P, F, n_lines, key_off.p, key_len.p, pass.p, head.p,
-                                                   (unsigned long long *)errw.p);
-            SGPU_LAUNCH(c);
-            paf_segment_kernel<<<(unsigned)ceil_div(n_lines, 256), 256, 0, st>>>(pass.p, head.p, n_lines, sel.p);
-            SGPU_LAUNCH(c);
-        } else if (kind == EV_SAM) {
+        if (kind == EV_SAM) {
             // the header's @SQ names first (a small exact set of their own), then the records
             sam_sq_kernel<<<grid, 128, 0, st>>>(P, n_lines, key_off.p, key_len.p, sel.p);
             SGPU_LAUNCH(c);
@@ -1071,13 +923,9 @@ static sgpu_status evidence_to_set(sgpu_ctx *c, EvidenceKind kind, const uint8_t
             sam_parse_kernel<<<grid, 128, 0, st>>>(P, F, view_of(sam_refs), sgpu_idset_len(sam_refs) != 0, n_lines, key_off.p,
                                                    key_len.p, sel.p, (unsigned long long *)errw.p);
             SGPU_LAUNCH(c);
-        } else if (kind == EV_TXT) {
-            txt_lines_kernel<<<grid, 128, 0, st>>>(P, n_lines, key_off.p, key_len.p, sel.p,
-                                                   (unsigned long long *)errw.p);
-            SGPU_LAUNCH(c);
         } else {
-            reads_parse_kernel<<<grid, 128, 0, st>>>(P, *T, need_fields, n_lines, key_off.p, key_len.p, sel.p,
-                                                     (unsigned long long *)errw.p);
+            lines_indexed_kernel<<<grid, 128, 0, st>>>(P, T ? *T : none, need_fields, mode, F, n_lines, key_off.p,
+                                                       key_len.p, sel.p, (unsigned long long *)errw.p);
             SGPU_LAUNCH(c);
         }
         uint64_t ew;

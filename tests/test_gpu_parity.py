@@ -32,6 +32,16 @@ def ctx_mode(request):
     c.close()
 
 
+@pytest.fixture(scope="module")
+def ctx_general():
+    """a context forced onto the general paths (sgpu_ctx_set_mode(1)): evidence takes the indexed kernel"""
+    c = api.Context(0)
+    c.set_mode(1)
+    c.mode = 1
+    yield c
+    c.close()
+
+
 def _ids(lst):
     return sorted(B(x) for x in lst)
 
@@ -70,17 +80,18 @@ def test_golden_fastq_errors(ctx_mode, golden):
         _same_clean(ctx_mode, B(c["buf"]), [])
 
 
-def test_golden_paf(ctx, golden):
-    for c in golden["paf_cases"]:
-        s = api.IdSet.from_paf(ctx, B(c["buf"]), c["min_len"], c["min_cov"], c["min_mapq"])
-        assert s.sorted_ids() == _ids(c["expect"]), c["name"]
-        assert len(s) == len(c["expect"])
-    for c in golden["paf_errors"]:
-        with pytest.raises(api.ScrubbyGpuError) as e:
-            api.IdSet.from_paf(ctx, B(c["buf"]))
-        assert e.value.status == c["error"], c["name"]
-        if "error_line" in c:
-            assert e.value.index == c["error_line"]
+def test_golden_paf(ctx, ctx_general, golden):
+    for cx in (ctx, ctx_general):  # the tile kernel, the indexed kernel
+        for c in golden["paf_cases"]:
+            s = api.IdSet.from_paf(cx, B(c["buf"]), c["min_len"], c["min_cov"], c["min_mapq"])
+            assert s.sorted_ids() == _ids(c["expect"]), c["name"]
+            assert len(s) == len(c["expect"])
+        for c in golden["paf_errors"]:
+            with pytest.raises(api.ScrubbyGpuError) as e:
+                api.IdSet.from_paf(cx, B(c["buf"]))
+            assert e.value.status == c["error"], c["name"]
+            if "error_line" in c:
+                assert e.value.index == c["error_line"]
 
 
 def test_golden_sam(ctx, golden):
@@ -107,18 +118,19 @@ def test_sam_random_matches_oracle(ctx, seed):
     assert api.IdSet.from_sam(ctx, d, 50, 0.5, 50).sorted_ids() == orc.set_from_sam(buf, 50, 0.5, 50).sorted_ids()
 
 
-def test_golden_reads_and_txt(ctx, golden):
-    for c in golden["reads_cases"]:
-        s = api.IdSet.from_reads(ctx, B(c["buf"]), c["style"], [B(t) for t in c["taxids"]])
-        assert s.sorted_ids() == _ids(c["expect"]), c["name"]
-    for c in golden["reads_errors"]:
-        with pytest.raises(api.ScrubbyGpuError) as e:
-            api.IdSet.from_reads(ctx, B(c["buf"]), c["style"], [])
-        assert e.value.status == c["error"], c["name"]
-    for c in golden["txt_cases"]:
-        s = api.IdSet.from_txt(ctx, B(c["buf"]))
-        assert s.sorted_ids() == _ids(c["expect"])
-        assert b"" in s and b"r2 " in s and b"r2" not in s
+def test_golden_reads_and_txt(ctx, ctx_general, golden):
+    for cx in (ctx, ctx_general):  # the tile kernel, the indexed kernel
+        for c in golden["reads_cases"]:
+            s = api.IdSet.from_reads(cx, B(c["buf"]), c["style"], [B(t) for t in c["taxids"]])
+            assert s.sorted_ids() == _ids(c["expect"]), c["name"]
+        for c in golden["reads_errors"]:
+            with pytest.raises(api.ScrubbyGpuError) as e:
+                api.IdSet.from_reads(cx, B(c["buf"]), c["style"], [])
+            assert e.value.status == c["error"], c["name"]
+        for c in golden["txt_cases"]:
+            s = api.IdSet.from_txt(cx, B(c["buf"]))
+            assert s.sorted_ids() == _ids(c["expect"])
+            assert b"" in s and b"r2 " in s and b"r2" not in s
 
 
 def test_golden_diff(ctx, golden):
@@ -176,14 +188,15 @@ def test_c1_alignment_config_small(ctx_mode):
                 assert g.path in (1, 2)
 
 
-def test_c2_classifier_config_small(ctx):
+def test_c2_classifier_config_small(ctx, ctx_general):
     """config 2 shape: Kraken2 reads + report, -T Chordata -D 9606 (taxids from the oracle's host stage)"""
     n = 50_000
     rep = synth.gen_kraken_report(500)
     taxids = orc.taxids_from_report(rep, ["Chordata"], ["9606"]).sorted_ids()
     kr = synth.gen_kraken_reads(n).numpy().tobytes()
-    gs = api.IdSet.from_reads(ctx, kr, 0, taxids)
     os_ = orc.set_from_reads(kr, 0, orc.OSet.from_ids(taxids))
+    assert api.IdSet.from_reads(ctx_general, kr, 0, taxids).sorted_ids() == os_.sorted_ids()  # the indexed kernel
+    gs = api.IdSet.from_reads(ctx, kr, 0, taxids)
     assert gs.sorted_ids() == os_.sorted_ids()
     fq = synth.gen_fastq(n, 1).numpy().tobytes()
     for reverse in (False, True):
@@ -694,9 +707,9 @@ def _txt_vs_oracle(ctx, buf: bytes):
 
 
 @pytest.mark.parametrize("seed", range(4))
-def test_reads_tile_kernel_edge_cases(ctx, seed):
+def test_reads_tile_kernel_edge_cases(ctx, ctx_general, seed):
     """Kraken2 / Metabuli lines across tile (16 KiB) and halo (1 KiB) edges, CRLF, whitespace to trim, non-ASCII
-    lines, very long lines, a missing final newline -- all against the oracle."""
+    lines, very long lines, a missing final newline -- all against the oracle, on the tile and the indexed kernel."""
     rng = random.Random(1000 + seed)
     taxids = ["9606", "7711", "0", "123456", "x9"]
     style = seed & 1
@@ -714,27 +727,30 @@ def test_reads_tile_kernel_edge_cases(ctx, seed):
         eol = "\r\n" if rng.random() < 0.1 else "\n"
         lines.append("\t".join(f) + eol)
     body = "".join(lines)
-    for tail in ("", "C\tlast\t9606\t1\tx" if style == 0 else "1\tlast\t9606\t1\t2\tg\tx"):
-        _reads_vs_oracle(ctx, (body + tail).encode(), style, taxids)
-    # a line longer than tile + halo, and tiles without any newline
     long_line = ("C\tlong\t9606\t1\t" if style == 0 else "1\tlong\t9606\t1\t2\tg\t") + "k" * 50000 + "\n"
-    _reads_vs_oracle(ctx, (body + long_line + body).encode(), style, taxids)
+    for cx in (ctx, ctx_general):
+        for tail in ("", "C\tlast\t9606\t1\tx" if style == 0 else "1\tlast\t9606\t1\t2\tg\tx"):
+            _reads_vs_oracle(cx, (body + tail).encode(), style, taxids)
+        # a line longer than tile + halo, and tiles without any newline
+        _reads_vs_oracle(cx, (body + long_line + body).encode(), style, taxids)
 
 
-def test_reads_tile_kernel_errors(ctx):
-    """too few fields (the reference panics) and invalid UTF-8 report the reference's error class and line"""
+def test_reads_tile_kernel_errors(ctx, ctx_general):
+    """too few fields (the reference panics) and invalid UTF-8 report the reference's error class and line, on the
+    tile and the indexed kernel"""
     good = "".join(f"C\tr{i}\t9606\t150\tk\n" for i in range(2000))
-    for bad, at in (("C\tr\t9606\t150\n", 700), ("\n", 1500), ("C\tr\n", 0), ("only one field", 2000)):
-        ls = good.splitlines(keepends=True)
-        ls.insert(at, bad)
-        _reads_vs_oracle(ctx, "".join(ls).encode(), 0, ["9606"])
-    raw = bytearray(good.encode())
-    raw[30000] = 0xFF  # invalid UTF-8 in some line
-    _reads_vs_oracle(ctx, bytes(raw), 0, ["9606"])
-    two = good.splitlines(keepends=True)
-    two.insert(100, "C\tr\n")
-    two.insert(1900, "x\n")
-    _reads_vs_oracle(ctx, "".join(two).encode(), 0, ["9606"])  # the first error wins
+    for cx in (ctx, ctx_general):
+        for bad, at in (("C\tr\t9606\t150\n", 700), ("\n", 1500), ("C\tr\n", 0), ("only one field", 2000)):
+            ls = good.splitlines(keepends=True)
+            ls.insert(at, bad)
+            _reads_vs_oracle(cx, "".join(ls).encode(), 0, ["9606"])
+        raw = bytearray(good.encode())
+        raw[30000] = 0xFF  # invalid UTF-8 in some line
+        _reads_vs_oracle(cx, bytes(raw), 0, ["9606"])
+        two = good.splitlines(keepends=True)
+        two.insert(100, "C\tr\n")
+        two.insert(1900, "x\n")
+        _reads_vs_oracle(cx, "".join(two).encode(), 0, ["9606"])  # the first error wins
 
 
 def test_fasta_input_matches_oracle(ctx_mode):
@@ -892,18 +908,100 @@ def test_paf_adversarial_fields(ctx_mode, seed):
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_txt_tile_kernel_edge_cases(ctx, seed):
+def test_txt_tile_kernel_edge_cases(ctx, ctx_general, seed):
     rng = random.Random(2000 + seed)
     lines = []
     for i in range(5000):
         lines.append(rng.choice([f"id{i}", f"id{i} ", "", f"id{i % 50}", "x" * rng.randint(1, 60), f"é{i}",
                                  "y" * rng.choice([15, 16, 17, 300, 5000])]) + rng.choice(["\n", "\n", "\r\n"]))
     body = "".join(lines)
-    _txt_vs_oracle(ctx, body.encode())
-    _txt_vs_oracle(ctx, (body + "last-without-newline").encode())
-    _txt_vs_oracle(ctx, (body + "z" * 40000 + "\n" + body).encode())
-    _txt_vs_oracle(ctx, b"\n")
-    _txt_vs_oracle(ctx, b"a")
+    for cx in (ctx, ctx_general):  # the tile kernel, the indexed kernel
+        _txt_vs_oracle(cx, body.encode())
+        _txt_vs_oracle(cx, (body + "last-without-newline").encode())
+        _txt_vs_oracle(cx, (body + "z" * 40000 + "\n" + body).encode())
+        _txt_vs_oracle(cx, b"\n")
+        _txt_vs_oracle(cx, b"a")
+
+
+def _around_dense(sparse, dense, bads):
+    """sparse lines, a dense region, sparse lines: as they are, without the final newline, and with each bad line
+    planted before the dense region, inside it, after it, and both before and after (the first error wins)"""
+    pre, post = sparse[: len(sparse) // 2], sparse[len(sparse) // 2:]
+    half = len(dense) // 2
+
+    def join(*parts):
+        return b"".join(x for p in parts for x in p)
+
+    yield join(pre, dense, post)
+    yield join(pre, dense, post).rstrip(b"\n")
+    for bad in bads:
+        yield join(pre, [bad], dense, post)
+        yield join(pre, dense[:half], [bad], dense[half:], post)
+        yield join(pre, dense, [bad], post)
+        yield join(pre, [bad], dense, [bad], post)
+
+
+def test_txt_dense_fallback(ctx):
+    """id lines of at most 7 bytes: 2341 or more lines per 16 KiB tile, more than the tile kernel's 2048, so the whole
+    list takes the indexed kernel on the default path; CRLF lines, invalid UTF-8 before / inside / after the dense
+    region, no final newline -- against the oracle"""
+    rng = random.Random(3100)
+    sparse = [b"sparse-id-%06d\n" % i for i in range(2000)]
+    dense = [b"t%d%s" % (rng.randrange(10_000), rng.choice([b"\n", b"\n", b"\r\n"])) for _ in range(20_000)]
+    assert max(map(len, dense)) <= 7
+    for buf in _around_dense(sparse, dense, [b"t\xff1\n", b"\xc3\n"]):
+        _txt_vs_oracle(ctx, buf)
+
+
+def test_reads_dense_fallback(ctx):
+    """Kraken2 lines of about 12 bytes: 5 separators each, about 6600 per 16 KiB tile, more than the tile kernel's
+    5120, so the whole file takes the indexed kernel on the default path; CRLF lines, whitespace to trim, invalid
+    UTF-8 and too few fields before / inside / after the dense region, no final newline -- against the oracle"""
+    rng = random.Random(3200)
+    sparse = [b"C\tsp%d\t1\t150\t%s\n" % (i, b" ".join(b"%d:1" % k for k in range(8))) for i in range(1000)]
+    dense = [b"C\t%s\t%s\t1\t%s" % (rng.choice([b"r%d"] * 7 + [b" r%d"]) % rng.randrange(1000),
+                                     rng.choice([b"1", b"2"] * 4 + [b"1 "]), rng.choice([b"\n"] * 3 + [b"\r\n"]))
+             for _ in range(20_000)]
+    assert sum(map(len, dense)) / len(dense) < 13
+    for buf in _around_dense(sparse, dense, [b"C\tr\xff\t1\t1\tk\n", b"C\tr1\t1\n", b"\n"]):
+        _reads_vs_oracle(ctx, buf, 0, ["1"])
+
+
+def test_paf_dense_fallback(ctx):
+    """bare 12-column PAF lines of at most 30 bytes: 12 separators each, more than 6500 per 16 KiB tile, more than the
+    tile kernel's 5120, so the whole file takes the indexed kernel on the default path; several lines per qname, CRLF
+    lines, invalid UTF-8, too few fields and a bad integer before / inside / after the dense region, no final newline
+    -- against the oracle"""
+    rng = random.Random(3300)
+    sparse = [b"s%d\t150\t%d\t%d\t+\tt\t1000\t0\t100\t90\t100\t%d\ttp:A:P\tcg:Z:150M\n" % (i, i % 50, 100 + i % 50,
+                                                                                               (i * 7) % 61)
+              for i in range(1200)]
+    dense = [b"r%d\t%d\t%d\t%d\t+\tt\t9\t0\t9\t9\t9\t%d%s" % (i // 3, rng.randrange(10), rng.randrange(5),
+                                                               rng.randrange(10), rng.randrange(100),
+                                                               rng.choice([b"\n", b"\n", b"\r\n"]))
+             for i in range(20_000)]
+    assert max(map(len, dense)) <= 30
+    bads = [b"r\xff\t9\t0\t9\t+\tt\t9\t0\t9\t9\t9\t60\n", b"r1\t9\t0\n", b"r1\t9\t0\tx\t+\tt\t9\t0\t9\t9\t9\t60\n"]
+    for buf in _around_dense(sparse, dense, bads):
+        for ml, mc, mq in [(0, 0.0, 0), (5, 0.5, 50)]:
+            _paf_vs_oracle(ctx, buf, ml, mc, mq)
+
+
+def test_misaligned_device_evidence_is_refused(ctx, ctx_general):
+    """a device view that does not start on a 16-byte boundary is SGPU_ERR_INVALID_ARG for every line format, on the
+    default and the general path"""
+    paf = b"r1\t150\t0\t150\t+\tt\t1000\t0\t150\t150\t150\t60\n" * 4
+    sam = b"@SQ\tSN:t\tLN:1000\n" + b"r1\t0\tt\t1\t60\t4M\t*\t0\t0\tACGT\tIIII\n" * 4
+    calls = [(paf, lambda cx, d: api.IdSet.from_paf(cx, d)), (b"r1\nr2\n" * 8, lambda cx, d: api.IdSet.from_txt(cx, d)),
+             (b"C\tr1\t1\t1\tk\n" * 8, lambda cx, d: api.IdSet.from_reads(cx, d, 0, ["1"])),
+             (sam, lambda cx, d: api.IdSet.from_sam(cx, d))]
+    for cx in (ctx, ctx_general):
+        for buf, call in calls:
+            d = torch.frombuffer(bytearray(b"\n" + buf), dtype=torch.uint8).cuda()
+            assert len(call(cx, d[1:].clone())) >= 1  # the same bytes, aligned, are accepted
+            with pytest.raises(api.ScrubbyGpuError) as e:
+                call(cx, d[1:])
+            assert e.value.status == 18  # SGPU_ERR_INVALID_ARG
 
 
 # ---------------------------------------------------------------------------- pipelined host-buffer path
